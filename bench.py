@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py ... --dump-outputs DIR                   (also writes the results of the last timed step, see
+                                                           dump_outputs: the inputs depend on the arguments only)
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d C2): a synthetic batch of HD-locus reads
 `(AGC)AACAGCCGCCAC(CGC)`, AGC~U{30..45}, CGC~U{7..12}, 50 % reverse strand, dwell U{5..13},
@@ -37,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 
 METRIC = 'caller_reads_per_s'
 UNIT = 'reads/s'
@@ -67,8 +70,60 @@ def parse():
     ap.add_argument('--panel-reads', type=int, default=20000, help='reads per locus of the panel leg')
     ap.add_argument('--c3-reads', type=int, default=33334, help='reads per locus of the c3 leg')
     ap.add_argument('--leg-base', type=int, default=2000, help='noiseless base reads per locus of a leg')
-    ap.add_argument('--leg-steps', type=int, default=3)
-    return ap.parse_args()
+    ap.add_argument('--leg-steps', type=int, default=None, help='timed steps of each leg (default: --steps)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="after the timed steps, write the per-read results of the last device-resident step as "
+                         "DIR/<name>.npy (rank 0's batch), to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.leg_steps is None:
+        args.leg_steps = args.steps
+    return args
+
+
+DUMP_MAX_READS = 1 << 18        # per-read arrays: every read up to this many, else a seeded sample of them
+DUMP_SEQ_READS = 4096           # reads whose called sequences are written
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, o, n_reads):
+    """The results one call_packed returned, as float64 / float32 .npy files under ``path``.
+
+    read_index            the reads written (all of them, or a sorted sample drawn with a fixed seed)
+    len1, len2, cost1, cost2, status, ttest_ties
+                          per read of read_index; a read with status != 0 has no device result (NaN)
+    seq_read_index        a fixed sample of read_index whose sequences are written
+    seq1, seq2            those reads' called sequences (first / rescaled pass), ASCII codes, concatenated
+                          in seq_read_index order; their lengths are len1 / len2 of the same reads
+    """
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(0)
+    idx = np.arange(n_reads) if n_reads <= DUMP_MAX_READS else np.sort(rng.choice(n_reads, DUMP_MAX_READS, replace=False))
+    status = o['status'].cpu().numpy()[idx]
+    failed = status != 0
+    out = {'read_index': idx.astype(np.float64), 'status': status.astype(np.float64),
+           'ttest_ties': o['ties'].cpu().numpy()[idx].astype(np.float64)}
+    for k in ('len1', 'len2', 'cost1', 'cost2'):
+        v = o[k].cpu().numpy()[idx].astype(np.float64)
+        v[failed] = np.nan
+        out[k] = v
+    # the sequences of a sample of the written reads, halved until everything fits the budget
+    seq_idx = np.sort(rng.choice(len(idx), min(DUMP_SEQ_READS, len(idx)), replace=False))
+    seq_idx = seq_idx[~failed[seq_idx]]
+    soff = np.asarray(o['seq_off'])[idx]
+    seq1, seq2 = o['seq1'].cpu().numpy(), o['seq2'].cpu().numpy()
+    while True:
+        for k, s in (('seq1', seq1), ('seq2', seq2)):
+            n = out['len' + k[-1]][seq_idx].astype(np.int64)
+            out[k] = np.concatenate([s[a:a + m] for a, m in zip(soff[seq_idx], n)] or [np.zeros(0, np.uint8)]
+                                    ).astype(np.float32)
+        if sum(v.nbytes for v in out.values()) + 8 * len(seq_idx) <= DUMP_MAX_BYTES or len(seq_idx) <= 1:
+            break
+        seq_idx = seq_idx[::2]
+    out['seq_read_index'] = idx[seq_idx].astype(np.float64)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + '.npy'), v)
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -497,13 +552,17 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_resident()
+        last = None                 # each step's results are freed before the next, as when nobody keeps them
+        last = step_resident()
     e1.record()
     barrier()
     clocks = sampler.stop()
     ms_total = e0.elapsed_time(e1)
     prof = _lib.profile_read()
     _lib.profile_enable(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, args.reads)
+    del last
 
     # ---- end-to-end timing (host buffers in, host arrays out) --------------------------------------
     for _ in range(args.warmup):

@@ -1,7 +1,10 @@
 """CPU: locus front-end (FASTA slices without pysam, motif -> regex)."""
+import json
+import os
+
+import numpy as np
 import pytest
 
-from oracle import refshim
 from warpstr_b200 import locus as lc
 
 
@@ -55,19 +58,11 @@ def test_motif_to_regex(fasta):
         lc.prepare_sequence('A', 'AGC')
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not refshim.available(), reason='reference tree not present')
-def test_motif_walk_equals_reference(fasta):
-    """Locus.prepare_sequence of the reference, fed through a stubbed pysam.faidx."""
-    import sys
-    ref = refshim.load()
-    from src.schemas import locus as rl
-    cases = [('AGC' * 19 + 'AACAGCCGCCAC' + 'CGC' * 7, 'AGC,CGC'), ('AAATAAATAAATGAAAT', 'AAAT'),
-             ('CAGCAGCAACAGCAGCCGCCG', 'CAG,CCG'), ('GGCCGGCCTTGGCC', 'GGCC'), ('CACACATCA', 'CA')]
-    for seq, motif in cases:
-        sys.modules['pysam'].faidx = lambda path, coord, s=seq: '>x\n' + s + '\n'
-        rl.pysam = sys.modules['pysam']
-        obj = rl.Locus.__new__(rl.Locus)
-        obj.name, obj.coord, obj.motif = 'n', 'c', motif
-        want = obj.prepare_sequence('ref.fa')
-        assert lc.prepare_sequence(seq, motif) == want, (seq, motif)
+def test_motif_walk_equals_reference():
+    """What Locus.prepare_sequence of the reference returned for these sequences and motifs (stored in
+    golden/reference_pin.npz, see tests/test_reference_pin.py)."""
+    z = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'reference_pin.npz'))
+    cases = json.loads(str(z['cases']))['motif_walk']
+    assert len(cases) == 5
+    for seq, motif, want in cases:
+        assert list(lc.prepare_sequence(seq, motif)) == want, (seq, motif)

@@ -1,11 +1,11 @@
 """CPU: the caller step's file contract (overview.csv columns, FASTA, complex-unit CSV)."""
+import json
 import os
 
 import numpy as np
 import pandas as pd
 import pytest
 
-from oracle import refshim
 from warpstr_b200 import overview as ov
 
 
@@ -53,20 +53,15 @@ def test_missing_overview(tmp_path):
         ov.load_overview(str(tmp_path))
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not refshim.available(), reason='reference tree not present')
 def test_files_identical_to_the_reference(tmp_path):
-    ref = refshim.load()
-    import importlib
-    rov = importlib.import_module('src.caller.overview')
-    a = _make_locus_dir(tmp_path / 'a') if (tmp_path / 'a').mkdir() is None else None
-    b = _make_locus_dir(tmp_path / 'b') if (tmp_path / 'b').mkdir() is None else None
-    for p in (a, b):
-        os.makedirs(os.path.join(p, 'predictions', 'sequences'))
+    """The files the reference's store_results wrote for the same inputs (stored in
+    golden/reference_pin.npz, see tests/test_reference_pin.py)."""
+    z = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'reference_pin.npz'))
+    want = json.loads(str(z['cases']))['overview_files']
+    a = _make_locus_dir(tmp_path)
+    os.makedirs(os.path.join(a, 'predictions', 'sequences'))
     ovp, df = ov.load_overview(a)
     ov.store_results(ovp, df, SEQS, COSTS, a)
-    rvp, rdf = rov.load_overview(b)
-    rov.store_results(rvp, rdf, SEQS, COSTS, b)
-    for rel in ('overview.csv', 'predictions/sequences/all.fasta', 'predictions/sequences/sequences_template.fasta',
-                'predictions/sequences/sequences_reverse.fasta'):
-        assert open(os.path.join(a, rel)).read() == open(os.path.join(b, rel)).read(), rel
+    assert len(want) == 4
+    for rel, text in want.items():
+        assert open(os.path.join(a, rel)).read() == text, rel

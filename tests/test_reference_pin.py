@@ -1,88 +1,91 @@
-"""Build container only (needs /root/reference): the oracle and the product's host code
-against the UNMODIFIED reference functions on fresh inputs.  Skipped on the GPU box, where
-the committed goldens (made by oracle/make_golden.py from the same functions) stand in."""
+"""CPU: the oracle and the product's host code against what the UNMODIFIED reference returned on
+the same inputs.  The reference's answers are stored in golden/reference_pin.npz: they were recorded
+from this code at the commit where every one of these comparisons last passed against the live
+reference (af33a0e), so that the pins hold on any machine, without the reference."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
-from oracle import refshim
-
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not refshim.available(), reason='reference tree not present')]
+GOLD = os.path.join(os.path.dirname(__file__), 'golden')
 
 
 @pytest.fixture(scope='module')
-def ref():
-    return refshim.load()
+def pin():
+    z = np.load(os.path.join(GOLD, 'reference_pin.npz'))
+    return json.loads(str(z['cases'])), z
 
 
-def test_automaton_builder_against_reference(ref):
+def test_automaton_builder_against_reference(pin):
     from warpstr_b200.automata import StateAutomata
-    from warpstr_b200 import synth
-    rng = np.random.default_rng(11)
-    pats = ['(AAAT)', '((CGG){AGG})', '(CAN)', '(AC{GT}(TA))', 'AC{G}{T}CA(GA)', '(RY)N(A)']
-    for pat in pats:
-        seq = synth.random_flank(rng, 40) + pat + synth.random_flank(rng, 40)
-        a, b = ref.StateAutomata(seq), StateAutomata(seq)
-        assert [s.kmer for s in a.states] == b.kmers
-        assert [s.value for s in a.states] == list(b.values)
-        assert [[p.idx for p in s.incoming] for s in a.states] == [list(b.incoming_of(i)) for i in range(b.n_states)]
-        assert a.mask == b.mask and a.endstate == b.endstate
+    cases, _ = pin
+    assert len(cases['automata']) == 6
+    for want in cases['automata']:
+        b = StateAutomata(want['seq'])
+        assert want['kmers'] == b.kmers
+        assert want['values'] == list(b.values)
+        assert want['incoming'] == [list(b.incoming_of(i)) for i in range(b.n_states)]
+        assert want['mask'] == b.mask and want['endstate'] == b.endstate
 
 
-def test_oracle_against_reference_run(ref):
+def test_oracle_against_reference_run(pin):
     from oracle import caller_oracle as co
-    from warpstr_b200 import synth
-    locus = synth.make_locus('FMR1', seed=77, flank_length=40)
-    rd = synth.make_reads(locus, 1, seed=78)[0]
-    sta = ref.StateAutomata(locus.reverse_regex if rd.reverse else locus.template_regex)
-    w = ref.WarpSTR(40, sta.states, sta.endstate, sta.mask, None, rd.reverse, rd.name)
-    want = w.run(rd.signal)
-    got = co.run_read(rd.signal, co.tables_from(sta), 40, rd.reverse, impl='c')
-    assert (got.seq, got.resc_seq, got.cost, got.resc_cost) == (want.seq, want.resc_seq, want.cost, want.resc_cost)
-    m0 = np.full(len(rd.signal), False)
-    D = w._calc_dtw_astates(rd.signal, sta.states, m0)
-    assert np.array_equal(D, co.fill_scalar(rd.signal, co.tables_from(sta), m0, 4, 40))
+    from warpstr_b200.automata import StateAutomata
+    cases, z = pin
+    want = cases['run']
+    x = z['run_signal']
+    tb = co.tables_from(StateAutomata(want['regex']))
+    got = co.run_read(x, tb, want['flank'], want['reverse'], impl='c')
+    assert (got.seq, got.resc_seq, got.cost, got.resc_cost) == (want['seq'], want['resc_seq'], want['cost'], want['resc_cost'])
+    D = co.fill_scalar(x, tb, np.full(len(x), False), 4, want['flank'])
+    assert list(D.shape) == want['fill_shape']
+    assert hashlib.sha256(np.ascontiguousarray(D, dtype=np.float64).tobytes()).hexdigest() == want['fill_sha256']
 
 
-def test_wrapper_helpers_against_reference(ref):
+def test_wrapper_helpers_against_reference(pin):
     from warpstr_b200.wrapper import CallerWrapper
+    want = pin[0]['wrapper']
     mine = CallerWrapper.__new__(CallerWrapper)
-    theirs = ref.wrapper.CallerWrapper.__new__(ref.wrapper.CallerWrapper)
-    for pat in ('((CAGG){CAGM})(CAGA)(CA)', '(AGC)AACAGCCGCCAC(CGC)', '(MGG)', 'AC(A{CN}T)G(CA)'):
-        assert mine.break_into_units(pat) == theirs.break_into_units(pat)
-        assert mine.reverse_uniq_sequence(pat) == theirs.reverse_uniq_sequence(pat)
+    for pat, w in want['units'].items():
+        assert json.loads(json.dumps(mine.break_into_units(pat))) == w['break_into_units']
+        assert mine.reverse_uniq_sequence(pat) == w['reverse_uniq_sequence']
     mine.units, mine.repeat_units, mine.offsets = mine.break_into_units('((CAGG){CAGM})(CAGA)(CA)')
-    theirs.units, theirs.repeat_units, theirs.offsets = mine.units, mine.repeat_units, mine.offsets
-    for seq in ('CAGGCAGGCAGACAGACA', 'CAGGCAGGCAGCCAGACACACA', 'TTT', ''):
-        assert mine.collapse_repeats(seq) == theirs.collapse_repeats(seq)
+    assert len(want['collapse']) == 4
+    for seq, w in want['collapse'].items():
+        assert json.loads(json.dumps(mine.collapse_repeats(seq))) == w
 
 
-def test_normalize_oracle_against_reference(ref):
+def test_normalize_oracle_against_reference(pin):
     from oracle import normalize_oracle as no
-    rng = np.random.default_rng(5)
-    raw = rng.integers(200, 1100, size=5001).astype(np.int16)
-    assert np.array_equal(no.brute_remove(raw), ref.Fast5.brute_remove(raw))
-    assert np.array_equal(no.normalize_signal_mad(raw), ref.normalize_signal_mad(raw))
+    z = pin[1]
+    raw = z['norm_raw']
+    assert np.array_equal(raw, np.random.default_rng(5).integers(200, 1100, size=5001).astype(np.int16))
+    assert np.array_equal(no.brute_remove(raw), z['norm_brute_remove'])
+    assert np.array_equal(no.normalize_signal_mad(raw), z['norm_mad'])
 
 
-def test_bundled_reads_against_reference_run(ref):
+def test_bundled_reads_against_reference_run():
     """Two of the reference's own bundled test reads (real nanopore signal, golden/c1_bundled.npz):
-    the unmodified reference's normalisation and WarpSTR.run against what the fixture holds from
-    the oracle -- which is what the GPU path is compared with in tests/test_gpu_c1.py."""
-    import os
+    the oracle's normalisation and call against what the fixture holds -- the answers the unmodified
+    reference's normalisation and WarpSTR.run gave for these reads, and what the GPU path is compared
+    with in tests/test_gpu_c1.py."""
+    from oracle import caller_oracle as co
+    from oracle import normalize_oracle as no
     from warpstr_b200 import templates as tmpl
-    z = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'c1_bundled.npz'))
+    from warpstr_b200.automata import StateAutomata
+    z = np.load(os.path.join(GOLD, 'c1_bundled.npz'))
     left, right, seq, F = str(z['left']), str(z['right']), str(z['sequence']), int(z['flank_length'])
     regex = {False: left + seq + right,
              True: tmpl.reverse_complement(right) + tmpl.reverse_uniq_sequence(seq) + tmpl.reverse_complement(left)}
     order = np.argsort(z['r_end_raw'] - z['l_start_raw'])[:2]            # the two shortest windows
     for i in order:
         raw = np.cumsum(z[f'raw_delta{i}'].astype(np.int64)).astype(np.int16)
-        norm = ref.normalize_signal_mad(ref.Fast5.brute_remove(raw))       # Fast5.get_data_processed, fast5.py:45-57
+        norm = no.normalize_signal_mad(no.brute_remove(raw))              # Fast5.get_data_processed, fast5.py:45-57
         x = np.ascontiguousarray(norm[int(z['l_start_raw'][i]):int(z['r_end_raw'][i]) + 1])
         rev = bool(z['reverse'][i])
-        sta = ref.StateAutomata(regex[rev])
-        got = ref.WarpSTR(F, sta.states, sta.endstate, sta.mask, None, rev, str(z['names'][i])).run(x)
+        got = co.run_read(x, co.tables_from(StateAutomata(regex[rev])), F, rev, impl='c')
         assert got.seq == str(z['seq'][i]) and got.resc_seq == str(z['resc_seq'][i])
         assert got.cost == z['cost1'][i] and got.resc_cost == z['cost2'][i]
         assert len(got.resc_seq) in (40, 44)
