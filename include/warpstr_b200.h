@@ -88,6 +88,36 @@ int wstr_dequantize_batch(const int16_t *d_raw, const int64_t *raw_off, const in
                           const double *d_shift_scale, int32_t n_reads, double *d_out,
                           const int64_t *out_off, void *d_workspace, int64_t workspace_bytes, void *stream);
 
+/* ---- (2c) VBZ-compressed raw signal --------------------------------------------------------------
+ * Replaces the StreamVByte + zig-zag delta half of the VBZ HDF5 filter (nanoporetech/vbz_compression)
+ * that h5py runs when the reference reads Raw/.../Signal (src/schemas/fast5.py:50-52); zstd stays on the
+ * host.  Chunk c's body after zstd is d_payload[in_off[c] .. in_off[c] + in_bytes[c]); kind[c]:
+ *   WSTR_VBZ_KIND_V0   VBZ version 0: ceil(n/4) bytes of 2-bit codes (c + 1 data bytes), then the data;
+ *   WSTR_VBZ_KIND_V1   VBZ version 1 (16-bit integers): ceil(n/8) bytes of 1-bit keys, then the data;
+ *   WSTR_VBZ_KIND_RAW  verbatim little-endian int16 (a chunk the host decoded itself).
+ * n_samples[c] is the count the body codes (the VBZ header's size / 2); the first n_out[c] <= n_samples[c]
+ * samples are written to d_raw + out_off[c] (HDF5's last chunk of a dataset codes a whole chunk).
+ * zigzag[c] != 0: the values are zig-zag deltas, summed from 0 in every chunk.  Bit-exact with
+ * warpstr_b200/fast5.py:vbz_decompress including its wrap-around to 16 bits; its format errors become
+ * d_status[c] (WSTR_VBZ_*), and a bad chunk leaves its own output range undefined and nothing else.
+ * The payload is fetched in whole 16-byte words: d_payload and every in_off must be 16-byte aligned, and
+ * the bytes up to in_off + in_bytes rounded up to 16 readable (the Python layer pads each chunk with
+ * zeros); no byte outside that padded span is read.  Output ranges of the chunks must not overlap.
+ * d_workspace: wstr_vbz_workspace_bytes(n_chunks) bytes; the chunk table travels through the staging
+ * slot like every other call's host arrays. */
+#define WSTR_VBZ_KIND_V0 0
+#define WSTR_VBZ_KIND_V1 1
+#define WSTR_VBZ_KIND_RAW 2
+#define WSTR_VBZ_OK 0
+#define WSTR_VBZ_TRUNCATED_CONTROL 1      /* fewer payload bytes than the control (v0) or key (v1) block */
+#define WSTR_VBZ_SHORT_DATA 2             /* v0: the data block is shorter than the codes need (extra bytes are fine) */
+#define WSTR_VBZ_LENGTH_MISMATCH 3        /* v1: the data block is not exactly as long as the keys say */
+int64_t wstr_vbz_workspace_bytes(int32_t n_chunks);
+int wstr_vbz_decode_batch(const uint8_t *d_payload, const int64_t *in_off, const int64_t *in_bytes,
+                          const int32_t *n_samples, const int32_t *n_out, const int32_t *kind,
+                          const int32_t *zigzag, const int64_t *out_off, int32_t n_chunks, int16_t *d_raw,
+                          int32_t *d_status, void *d_workspace, int64_t workspace_bytes, void *stream);
+
 /* ---- (3) DTW state automaton ----------------------------------------------------------------
  * wstr_automaton_create uploads one strand's automaton: the flat form of StateAutomata
  * (src/caller/automata.py:36-48).  All arrays are host pointers.

@@ -52,6 +52,9 @@ _SIGNATURES = {
     'wstr_dequantize_workspace_bytes': (ctypes.c_int64, [ctypes.c_int32]),
     'wstr_dequantize_batch': (ctypes.c_int, [c_vp, c_i64p, c_i32p, c_vp, ctypes.c_int32, c_vp, c_i64p, c_vp,
                                              ctypes.c_int64, c_vp]),
+    'wstr_vbz_workspace_bytes': (ctypes.c_int64, [ctypes.c_int32]),
+    'wstr_vbz_decode_batch': (ctypes.c_int, [c_vp, c_i64p, c_i64p, c_i32p, c_i32p, c_i32p, c_i32p, c_i64p,
+                                             ctypes.c_int32, c_vp, c_vp, c_vp, ctypes.c_int64, c_vp]),
     'wstr_automaton_create': (ctypes.c_int, [c_f64p, c_i32p, c_i32p, c_i32p, c_u8p, c_u8p, ctypes.c_int32,
                                              ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                              ctypes.POINTER(c_vp)]),
@@ -264,6 +267,38 @@ def dequantize_batch(d_raw, raw_off, lengths, d_shift_scale, d_out, out_off, d_w
                                      int(ln.shape[0]), _dptr(d_out), _ptr(oo, c_i64p), _dptr(d_workspace),
                                      int(d_workspace.numel() * d_workspace.element_size()), _stream_ptr(stream))
     check(rc, 'wstr_dequantize_batch')
+
+
+VBZ_KIND_V0, VBZ_KIND_V1, VBZ_KIND_RAW = 0, 1, 2
+# d_status of wstr_vbz_decode_batch -> the message fast5.vbz_decompress raises for the same chunk
+VBZ_STATUS_MESSAGES = {
+    1: 'VBZ: truncated StreamVByte control block',
+    2: 'VBZ: truncated StreamVByte data block',
+    3: 'VBZ v1: data block length does not match the keys',
+}
+
+
+def vbz_workspace_bytes(n_chunks: int) -> int:
+    n = lib().wstr_vbz_workspace_bytes(int(n_chunks))
+    if n < 0:
+        check(int(n), 'wstr_vbz_workspace_bytes')
+    return int(n)
+
+
+def vbz_decode_batch(d_payload, in_off, in_bytes, n_samples, n_out, kind, zigzag, out_off, d_raw, d_status,
+                     d_workspace, stream=None) -> None:
+    io = _np(in_off, np.int64)
+    ib = _np(in_bytes, np.int64)
+    ns = _np(n_samples, np.int32)
+    no = _np(n_out, np.int32)
+    kd = _np(kind, np.int32)
+    zz = _np(zigzag, np.int32)
+    oo = _np(out_off, np.int64)
+    rc = lib().wstr_vbz_decode_batch(
+        _dptr(d_payload), _ptr(io, c_i64p), _ptr(ib, c_i64p), _ptr(ns, c_i32p), _ptr(no, c_i32p), _ptr(kd, c_i32p),
+        _ptr(zz, c_i32p), _ptr(oo, c_i64p), int(io.shape[0]), _dptr(d_raw), _dptr(d_status), _dptr(d_workspace),
+        int(d_workspace.numel() * d_workspace.element_size()), _stream_ptr(stream))
+    check(rc, 'wstr_vbz_decode_batch')
 
 
 def measure_fp64_add_rate(stream=None) -> float:

@@ -195,6 +195,83 @@ class _IngestRaw:
         res['lengths'] = self.lengths
 
 
+def pack_vbz(reads):
+    """Chunks of compressed reads (fast5.CompressedRead) -> what ``call_arrays_vbz`` takes: the pinned payload
+    buffer (every chunk's body at a 16-byte aligned offset, zero padded: the decoder reads whole 16-byte
+    words), the chunk table, the first chunk of every read (int64[n + 1]) and the read offsets in the
+    decoded int16 buffer (int64[n + 1])."""
+    import torch
+    chunks = [c for r in reads for c in r.chunks]
+    m = len(chunks)
+    n_chunks = np.fromiter((len(r.chunks) for r in reads), dtype=np.int64, count=len(reads))
+    read_chunk = np.zeros(len(reads) + 1, dtype=np.int64)
+    read_chunk[1:] = np.cumsum(n_chunks)
+    raw_off = np.zeros(len(reads) + 1, dtype=np.int64)
+    raw_off[1:] = np.cumsum(np.fromiter((r.n_samples for r in reads), dtype=np.int64, count=len(reads)))
+    in_bytes = np.fromiter((len(c.payload) for c in chunks), dtype=np.int64, count=m)
+    in_off = np.zeros(m + 1, dtype=np.int64)
+    in_off[1:] = np.cumsum((in_bytes + 15) & ~15)
+    chunk_read = np.repeat(np.arange(len(reads)), n_chunks)
+    table = dict(in_off=in_off[:-1], in_bytes=in_bytes,
+                 n_samples=np.fromiter((c.coded if c.kind != 2 else c.count for c in chunks), dtype=np.int32, count=m),
+                 n_out=np.fromiter((c.count for c in chunks), dtype=np.int32, count=m),
+                 kind=np.fromiter((c.kind for c in chunks), dtype=np.int32, count=m),
+                 zigzag=np.fromiter((c.zigzag for c in chunks), dtype=np.int32, count=m),
+                 out_off=raw_off[chunk_read] + np.fromiter((c.start for c in chunks), dtype=np.int64, count=m))
+    host = torch.zeros(max(int(in_off[-1]), 16), dtype=torch.uint8, pin_memory=torch.cuda.is_available())
+    hb = host.numpy()
+    for c, o in zip(chunks, in_off[:-1]):
+        hb[o:o + len(c.payload)] = np.frombuffer(c.payload, dtype=np.uint8)
+    return host, table, read_chunk, raw_off
+
+
+class _IngestVBZ(_IngestRaw):
+    """VBZ chunk bodies (after zstd) of whole reads + windows: the StreamVByte / delta decode
+    (wstr_vbz_decode_batch) writes the int16 reads on the device, which then go on as in _IngestRaw."""
+
+    def __init__(self, eng, host_payload, table, read_chunk, raw_off, lo, hi, lengths, spike_mode):
+        super().__init__(eng, None, raw_off, lo, hi, lengths, spike_mode)
+        self.payload, self.table, self.read_chunk = host_payload, table, read_chunk
+        m = len(table['in_off'])
+        self.pay_off = np.append(table['in_off'], int(table['in_off'][-1] + ((table['in_bytes'][-1] + 15) & ~15))
+                                 if m else 0)[read_chunk]                     # payload bytes of reads [a, b)
+        self.h2d_bytes = int(self.pay_off[-1]) if len(self.pay_off) else 0
+
+    def allocate(self):
+        import torch
+        super().allocate()
+        e = self.eng
+        m = len(self.table['in_off'])
+        self.d_payload = e._device_buffer('vbz_payload', max(self.h2d_bytes, 16), torch.uint8)
+        self.d_status = e._device_buffer('vbz_status', m, torch.int32)
+        cur = e._host_vbz_status
+        if cur is None or cur.numel() < m:
+            e._host_vbz_status = torch.empty(max(m, 1), dtype=torch.int32, pin_memory=torch.cuda.is_available())
+
+    def send(self, a, b):
+        lo, hi = int(self.pay_off[a]), int(self.pay_off[b])
+        self.d_payload[lo:hi].copy_(self.payload[lo:hi], non_blocking=True)
+
+    def prepare(self, a, b, lane):
+        import torch
+        c0, c1 = int(self.read_chunk[a]), int(self.read_chunk[b])
+        if c1 > c0:
+            t = {k: v[c0:c1] for k, v in self.table.items()}
+            ws = self.eng._device_buffer(f'vbz_ws{lane}', _lib.vbz_workspace_bytes(c1 - c0), torch.uint8)
+            _lib.vbz_decode_batch(self.d_payload, t['in_off'], t['in_bytes'], t['n_samples'], t['n_out'], t['kind'],
+                                  t['zigzag'], t['out_off'], self.d_raw, self.d_status[c0:c1], ws)
+        super().prepare(a, b, lane)
+
+    def fetch(self, a, b, out):
+        super().fetch(a, b, out)
+        c0, c1 = int(self.read_chunk[a]), int(self.read_chunk[b])
+        self.eng._host_vbz_status[c0:c1].copy_(self.d_status[c0:c1], non_blocking=True)
+
+    def finish(self, res, out, n):
+        super().finish(res, out, n)
+        res['chunk_status'] = self.eng._host_vbz_status[:len(self.table['in_off'])].numpy().copy()
+
+
 class CallerEngine:
     """Batched two-pass WarpSTR caller on one GPU."""
 
@@ -220,6 +297,7 @@ class CallerEngine:
         self.timeline = None      # set to a list to collect (label, CUDA event) pairs from call_arrays
         self._host_out = None
         self._host_ss = None
+        self._host_vbz_status = None
         self._dev_cache = {}
         self._h2d_probe = None
         self.split_small = (4096, 40000)   # batch sizes a resident call runs as two concurrent halves (None: never)
@@ -499,6 +577,23 @@ class CallerEngine:
         return self._pipeline(_IngestRaw(self, host_raw, raw_off, lo, hi, lengths, SPIKE_MODES[spike_removal]),
                               lengths, aut, rev, want_seq, chunk_reads, lanes)
 
+    def call_arrays_vbz(self, host_payload, table, read_chunk, raw_off, win_lo, win_hi, aut, rev,
+                        spike_removal: str = 'Brute', want_seq: bool = True, chunk_reads: int = 25000,
+                        lanes: int = 2) -> Dict[str, np.ndarray]:
+        """``call_arrays_raw`` for reads still VBZ-compressed as their fast5 file stores them (``pack_vbz`` makes
+        the arguments): only the chunk bodies (after zstd, ~1.25 B per sample instead of 2) cross PCIe, and the
+        StreamVByte / zig-zag delta decode (wstr_vbz_decode_batch) writes the int16 reads on the device.  Same
+        result dict, plus ``chunk_status`` (WSTR_VBZ_* per chunk; a read with a bad chunk has undefined results)."""
+        from .normalize import SPIKE_MODES
+        raw_off = np.asarray(raw_off, dtype=np.int64)
+        lo = np.asarray(win_lo, dtype=np.int32)
+        hi = np.asarray(win_hi, dtype=np.int32)
+        lens = np.diff(raw_off)
+        lengths = np.maximum(np.minimum(hi.astype(np.int64), lens - 1) - lo + 1, 0).astype(np.int32)
+        ingest = _IngestVBZ(self, host_payload, table, np.asarray(read_chunk, dtype=np.int64), raw_off, lo, hi,
+                            lengths, SPIKE_MODES[spike_removal])
+        return self._pipeline(ingest, lengths, aut, rev, want_seq, chunk_reads, lanes)
+
     def _pipeline(self, ingest, lengths, aut, rev, want_seq, chunk_reads, lanes) -> Dict[str, np.ndarray]:
         import torch
         n = len(lengths)
@@ -708,12 +803,46 @@ class CallerEngine:
         aut = np.asarray(aut_ids, dtype=np.int32)
         rev = np.asarray(reverse, dtype=np.uint8)
         res = self.call_arrays_raw(host, raw_off, lo, hi, aut, rev, spike_removal)
+        return self._raw_results(res, lambda idx: [raws[r] for r in idx], windows, aut_ids, reverse, spike_removal)
+
+    def call_vbz_batch(self, reads, windows, aut_ids, reverse, spike_removal: str = 'Brute') -> List[CallerResult]:
+        """``call_raw_batch`` for reads as their fast5 files store them (fast5.CompressedRead, from
+        ``fast5.raw_chunks``): the chunk bodies go to the device, are decoded there (wstr_vbz_decode_batch) and
+        called as ``call_raw_batch`` calls raw reads.  A chunk the host decoder would refuse raises that
+        Fast5FormatError, naming the file and the read, before any result is returned."""
+        from .fast5 import Fast5FormatError
+        n = len(reads)
+        if n == 0:
+            return []
+        if any(r.n_samples <= 0 for r in reads):
+            raise ValueError('empty raw read')
+        lo = np.array([w[0] for w in windows], dtype=np.int32)
+        hi = np.array([w[1] for w in windows], dtype=np.int32)
+        if (lo < 0).any():
+            raise ValueError('negative window start')
+        host, table, read_chunk, raw_off = pack_vbz(reads)
+        res = self.call_arrays_vbz(host, table, read_chunk, raw_off, lo, hi, np.asarray(aut_ids, dtype=np.int32),
+                                   np.asarray(reverse, dtype=np.uint8), spike_removal)
+        bad = np.flatnonzero(res['chunk_status'])
+        if len(bad):
+            c = int(bad[0])
+            r = int(np.searchsorted(read_chunk, c, side='right')) - 1
+            msg = _lib.VBZ_STATUS_MESSAGES.get(int(res['chunk_status'][c]), 'VBZ: corrupt chunk')
+            raise Fast5FormatError(f'{reads[r].path}: read {reads[r].read_name}: {msg} '
+                                   f'(chunk at sample {reads[r].chunks[c - int(read_chunk[r])].start})')
+        return self._raw_results(res, lambda idx: [reads[r].decode() for r in idx], windows, aut_ids, reverse,
+                                 spike_removal)
+
+    def _raw_results(self, res, raws_of, windows, aut_ids, reverse, spike_removal) -> List[CallerResult]:
+        """CallerResults of a ``call_arrays_raw``-style result dict.  Reads the device did not finish, or whose
+        t-test decision was within rounding of flipping, are redone as in results_from (the reference's
+        exception, or the host's libm for a t-test tie) from their host int16 samples, ``raws_of(indices)``."""
         status, ties = res['status'], res['ttest_ties']
         self.last_ttest_ties = int((ties > 0).sum())
         out: List[Optional[CallerResult]] = []
         redo = []
         so = res['seq_off']
-        for r in range(n):
+        for r in range(len(status)):
             if status[r] == 0 and ties[r] == 0:
                 a = int(so[r])
                 out.append(CallerResult(seq=res['seq1'][a:a + res['len1'][r]].tobytes().decode('ascii'),
@@ -723,9 +852,9 @@ class CallerEngine:
             else:
                 out.append(None)
                 redo.append(r)
-        if redo:        # as in results_from: the reference's exception, or the host's libm for a t-test tie
+        if redo:
             from .normalize import normalize_windows
-            sigs = normalize_windows([raws[r] for r in redo], [windows[r] for r in redo], spike_removal,
+            sigs = normalize_windows(raws_of(redo), [windows[r] for r in redo], spike_removal,
                                      device=str(self.device))
             fixed = self._call_batch_host(sigs, [aut_ids[r] for r in redo], [reverse[r] for r in redo])
             for r, f in zip(redo, fixed):

@@ -25,7 +25,8 @@ import ctypes.util
 import mmap
 import struct
 import zlib
-from typing import Dict, List, Optional, Tuple
+from dataclasses import dataclass
+from typing import Dict, Iterator, List, NamedTuple, Optional, Tuple
 
 import numpy as np
 
@@ -114,21 +115,29 @@ def _svb_decode_u16(buf: np.ndarray, n: int) -> np.ndarray:
     return (padded[starts] | np.where(lens > 1, padded[starts + 1] << np.uint16(8), np.uint16(0))).astype(np.uint16)
 
 
-def vbz_decompress(chunk: bytes, cd_values: Tuple[int, ...]) -> bytes:
-    """One HDF5 chunk written by the VBZ filter -> raw little-endian integers."""
+def _vbz_params(cd_values: Tuple[int, ...]):
+    """(version, integer size, zig-zag flag, zstd level) of the VBZ filter's cd_values."""
     version = cd_values[0] if len(cd_values) > 0 else 0
     int_size = cd_values[1] if len(cd_values) > 1 else 0
     zigzag = cd_values[2] if len(cd_values) > 2 else 0
     zstd_level = cd_values[3] if len(cd_values) > 3 else 1
+    return version, int_size, zigzag, zstd_level
+
+
+def _vbz_body(chunk: bytes, int_size: int, zstd_level: int):
+    """A VBZ chunk's sample count and its StreamVByte body (zstd undone)."""
     if len(chunk) < 4:
         raise Fast5FormatError('VBZ: chunk shorter than its size header')
     (orig_size,) = struct.unpack_from('<I', chunk, 0)
-    body = chunk[4:]
-    if int_size == 0:                                   # bytes passed through zstd only
-        return zstd_decompress(body, orig_size) if zstd_level else bytes(body[:orig_size])
     n = orig_size // int_size
+    body = chunk[4:]
     if zstd_level:
         body = zstd_decompress(body, n * 5 + 16)
+    return n, body
+
+
+def vbz_decode_body(body: bytes, n: int, version: int, int_size: int, zigzag: int) -> bytes:
+    """StreamVByte body of ``n`` integers (after zstd) -> raw little-endian integers."""
     buf = np.frombuffer(body, dtype=np.uint8)
     if int_size in (1,):
         raise Fast5FormatError('VBZ: 1-byte integers are not used by fast5 signals')
@@ -150,6 +159,58 @@ def vbz_decompress(chunk: bytes, cd_values: Tuple[int, ...]) -> bytes:
         raise Fast5FormatError(f'VBZ: unsupported version {version} / integer size {int_size}')
     dt = {2: '<i2', 4: '<i4'}[int_size] if zigzag else {2: '<u2', 4: '<u4'}[int_size]
     return vals.astype(dt).tobytes()
+
+
+def vbz_decompress(chunk: bytes, cd_values: Tuple[int, ...]) -> bytes:
+    """One HDF5 chunk written by the VBZ filter -> raw little-endian integers."""
+    version, int_size, zigzag, zstd_level = _vbz_params(cd_values)
+    if int_size == 0:                                   # bytes passed through zstd only
+        if len(chunk) < 4:
+            raise Fast5FormatError('VBZ: chunk shorter than its size header')
+        (orig_size,) = struct.unpack_from('<I', chunk, 0)
+        body = chunk[4:]
+        return zstd_decompress(body, orig_size) if zstd_level else bytes(body[:orig_size])
+    n, body = _vbz_body(chunk, int_size, zstd_level)
+    return vbz_decode_body(body, n, version, int_size, zigzag)
+
+
+# chunk kinds of raw_chunks (the numbering of wstr_vbz_decode_batch)
+KIND_VBZ0, KIND_VBZ1, KIND_RAW = 0, 1, 2
+
+
+class RawChunk(NamedTuple):
+    """One chunk of a read's signal as the device decoder takes it: samples [start, start + count) of the
+    read come from ``payload`` -- a VBZ StreamVByte body after zstd (kind KIND_VBZ0 / KIND_VBZ1, coding
+    ``coded`` >= count samples, zig-zag deltas if ``zigzag``) or ``count`` little-endian int16 (KIND_RAW)."""
+    start: int
+    count: int
+    kind: int
+    payload: bytes
+    zigzag: bool = False
+    coded: int = 0
+
+    def decode(self) -> np.ndarray:
+        """The chunk's int16 samples, decoded on the host (fast5.vbz_decompress)."""
+        if self.kind == KIND_RAW:
+            return np.frombuffer(self.payload, dtype='<i2', count=self.count)
+        raw = vbz_decode_body(self.payload, self.coded, self.kind, 2, int(self.zigzag))
+        return np.frombuffer(raw, dtype='<i2', count=self.count)
+
+
+@dataclass
+class CompressedRead:
+    """A read's raw signal as its file stores it (see ``raw_chunks``)."""
+    path: str
+    read_name: Optional[str]
+    n_samples: int
+    chunks: List[RawChunk]
+
+    def decode(self) -> np.ndarray:
+        """The read's int16 samples decoded on the host: what ``raw_signal`` returns."""
+        out = np.zeros(self.n_samples, dtype=np.int16)
+        for c in self.chunks:
+            out[c.start:c.start + c.count] = c.decode()
+        return out
 
 
 def _unshuffle(data: bytes, elem: int) -> bytes:
@@ -425,11 +486,12 @@ class H5File:
         arr = np.frombuffer(raw, dtype=obj.dtype, count=count)
         return arr.reshape(shape).astype(obj.dtype.newbyteorder('='), copy=True)
 
-    def _read_chunks(self, obj: _Obj, n: int, elem: int) -> bytes:
+    def _chunk_entries(self, obj: _Obj) -> Iterator[Tuple[int, int, int, int]]:
+        """(first element, stored bytes, filter mask, address) of every chunk in the v1 chunk B-tree."""
         _, bt, dims = obj.layout
-        chunk_elems = int(dims[0])
-        out = bytearray(n * elem)
         b = self.buf
+        nd = len(dims)
+        key_size = 8 + 8 * nd
 
         def walk(node):
             p = node + self.base
@@ -438,42 +500,99 @@ class H5File:
             ntype, level, used = struct.unpack_from('<BBH', b, p + 4)
             if ntype != 1:
                 raise Fast5FormatError(f'{self.path}: chunk B-tree expected')
-            nd = len(dims)
-            key_size = 8 + 8 * nd
             q = p + 24
             for _ in range(used):
                 csize, fmask = struct.unpack_from('<II', b, q)
                 offs = struct.unpack_from('<%dQ' % nd, b, q + 8)
                 (child,) = struct.unpack_from('<Q', b, q + key_size)
                 if level > 0:
-                    walk(child)
+                    yield from walk(child)
                 else:
-                    data = bytes(b[child + self.base:child + self.base + csize])
-                    for idx in range(len(obj.filters) - 1, -1, -1):
-                        if fmask & (1 << idx):
-                            continue
-                        fid, cd = obj.filters[idx]
-                        if fid == VBZ_FILTER_ID:
-                            data = vbz_decompress(data, cd)
-                        elif fid == 1:
-                            data = zlib.decompress(data)
-                        elif fid == 2:
-                            data = _unshuffle(data, elem)
-                        elif fid == 3:
-                            data = data[:-4]              # fletcher32 checksum, not verified
-                        else:
-                            raise Fast5FormatError(f'{self.path}: HDF5 filter {fid} is not supported')
-                    start = int(offs[0])
-                    take = min(chunk_elems, n - start) * elem
-                    if take > 0:
-                        if len(data) < take:
-                            raise Fast5FormatError(f'{self.path}: chunk shorter than its extent')
-                        out[start * elem:start * elem + take] = data[:take]
+                    yield int(offs[0]), csize, fmask, child
                 q += key_size + 8
 
         if bt != UNDEF:
-            walk(bt)
+            yield from walk(bt)
+
+    def _chunk_bytes(self, addr: int, csize: int) -> bytes:
+        return bytes(self.buf[addr + self.base:addr + self.base + csize])
+
+    def _unfilter(self, obj: _Obj, data: bytes, fmask: int, elem: int) -> bytes:
+        for idx in range(len(obj.filters) - 1, -1, -1):
+            if fmask & (1 << idx):
+                continue
+            fid, cd = obj.filters[idx]
+            if fid == VBZ_FILTER_ID:
+                data = vbz_decompress(data, cd)
+            elif fid == 1:
+                data = zlib.decompress(data)
+            elif fid == 2:
+                data = _unshuffle(data, elem)
+            elif fid == 3:
+                data = data[:-4]              # fletcher32 checksum, not verified
+            else:
+                raise Fast5FormatError(f'{self.path}: HDF5 filter {fid} is not supported')
+        return data
+
+    def _read_chunks(self, obj: _Obj, n: int, elem: int) -> bytes:
+        chunk_elems = int(obj.layout[2][0])
+        out = bytearray(n * elem)
+        for start, csize, fmask, addr in self._chunk_entries(obj):
+            data = self._unfilter(obj, self._chunk_bytes(addr, csize), fmask, elem)
+            take = min(chunk_elems, n - start) * elem
+            if take > 0:
+                if len(data) < take:
+                    raise Fast5FormatError(f'{self.path}: chunk shorter than its extent')
+                out[start * elem:start * elem + take] = data[:take]
         return bytes(out)
+
+    def raw_chunks(self, path: str) -> Tuple[int, List[RawChunk]]:
+        """An int16 signal dataset as (sample count, chunks covering [0, count) in order) without the
+        StreamVByte decode: a VBZ chunk of 2-byte integers comes back as its body after zstd (kind KIND_VBZ0
+        or KIND_VBZ1); every other chunk -- other filters, other VBZ integer sizes, contiguous and compact
+        layouts -- is decoded here, as ``dataset`` decodes it, and comes back verbatim (KIND_RAW), and so
+        do unallocated chunks (zeros, as ``dataset`` leaves them)."""
+        obj = self._object(self._resolve(path))
+        vbz = None
+        if (obj.layout is not None and obj.layout[0] == 'chunked' and obj.shape is not None and len(obj.shape) == 1
+                and obj.dtype == np.dtype('<i2') and len(obj.filters) == 1 and obj.filters[0][0] == VBZ_FILTER_ID):
+            version, int_size, zigzag, zstd_level = _vbz_params(obj.filters[0][1])
+            if int_size == 2 and version in (0, 1):
+                vbz = version, zigzag, zstd_level
+        if vbz is None:
+            x = np.ascontiguousarray(self.dataset(path), dtype=np.int16).reshape(-1)
+            return len(x), [RawChunk(0, len(x), KIND_RAW, x.tobytes())]
+        version, zigzag, zstd_level = vbz
+        n = int(obj.shape[0])
+        chunk_elems = int(obj.layout[2][0])
+        found = []
+        for start, csize, fmask, addr in self._chunk_entries(obj):
+            take = min(chunk_elems, n - start)
+            if take <= 0:
+                continue
+            data = self._chunk_bytes(addr, csize)
+            if fmask & 1:                                       # stored without the filter
+                data = self._unfilter(obj, data, fmask, 2)
+                if len(data) < 2 * take:
+                    raise Fast5FormatError(f'{self.path}: chunk shorter than its extent')
+                found.append(RawChunk(start, take, KIND_RAW, data[:2 * take]))
+                continue
+            coded, body = _vbz_body(data, 2, zstd_level)
+            if coded < take:
+                raise Fast5FormatError(f'{self.path}: chunk shorter than its extent')
+            found.append(RawChunk(start, take, KIND_VBZ0 if version == 0 else KIND_VBZ1, body, bool(zigzag), coded))
+        found.sort(key=lambda c: c.start)
+        chunks, at = [], 0
+        for c in found:
+            if c.start < at:
+                raise Fast5FormatError(f'{self.path}: overlapping chunks')
+            if c.start > at:
+                chunks.append(RawChunk(at, c.start - at, KIND_RAW, bytes(2 * (c.start - at))))
+            chunks.append(c)
+            at = c.start + c.count
+        if at < n:
+            chunks.append(RawChunk(at, n - at, KIND_RAW, bytes(2 * (n - at))))
+        return n, chunks
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -493,19 +612,36 @@ def raw_signal(path: str, read_name: Optional[str] = None) -> np.ndarray:
 
 
 def _raw_signal(h5: H5File, read_name: Optional[str]) -> np.ndarray:
+    return h5.dataset(_signal_path(h5, read_name))
+
+
+def _signal_path(h5: H5File, read_name: Optional[str]) -> str:
+    """The dataset holding a read's signal: ``read_<name>/Raw/Signal`` (the ``read_`` prefix optional),
+    else the first read of a single-read file, else the only read of a multi-read file."""
     if read_name is not None:
         name = read_name if read_name.startswith('read_') else 'read_' + read_name
         if name in h5:
-            return h5.dataset(f'{name}/Raw/Signal')
+            return f'{name}/Raw/Signal'
     if 'Raw/Reads' in h5:
         reads = h5.keys('Raw/Reads')
         if reads:
-            return h5.dataset(f'Raw/Reads/{reads[0]}/Signal')     # fast5.py:50-52: the first read
+            return f'Raw/Reads/{reads[0]}/Signal'         # fast5.py:50-52: the first read
     if read_name is None:
         members = [k for k in h5.keys('/') if k.startswith('read_')]
         if len(members) == 1:
-            return h5.dataset(f'{members[0]}/Raw/Signal')
+            return f'{members[0]}/Raw/Signal'
     raise KeyError(f'read {read_name} not found in {h5.path}')
+
+
+def raw_chunks(path: str, read_name: Optional[str] = None, h5: Optional[H5File] = None) -> CompressedRead:
+    """One read's signal as its file stores it, for the device decoder (CallerEngine.call_vbz_batch):
+    the read is chosen exactly as ``raw_signal`` chooses it, zstd is undone here and the StreamVByte
+    decode is left to the GPU (see H5File.raw_chunks).  ``h5``: the file, already open."""
+    if h5 is None:
+        with H5File(path) as f:
+            return raw_chunks(path, read_name, f)
+    n, chunks = h5.raw_chunks(_signal_path(h5, read_name))
+    return CompressedRead(path, read_name, n, chunks)
 
 
 class Fast5:

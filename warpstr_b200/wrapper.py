@@ -128,6 +128,15 @@ class CallerWrapper:
         return self.engine.call_raw_batch(raws, windows, aut, reverse,
                                           spike_removal or self.caller_config.spike_removal)
 
+    def run_compressed(self, reads, windows, reverse: Sequence[bool],
+                       spike_removal: Optional[str] = None) -> List[CallerResult]:
+        """``run_raw`` for reads as their fast5 files store them (fast5.CompressedRead, see
+        ``get_compressed_workload``): the VBZ decode happens on the device too, order preserved."""
+        reverse = [bool(r) for r in reverse]
+        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
+        return self.engine.call_vbz_batch(reads, windows, aut, reverse,
+                                          spike_removal or self.caller_config.spike_removal)
+
     # -- state similarity report (wrapper.py:122-160) ------------------------------------------------
     def check_high_similarity(self, sequence: str):
         diffs = {'template': self.pore_model.get_diffs_for_all(sequence),
@@ -229,24 +238,53 @@ def get_raw_workload(df_overview, path: str):
     has_src = 'fast5_path' in df_overview.columns
     for row in df_overview.itertuples():
         if row.saved:
-            fpath = os.path.join(path, tmpl.FAST5_SUBDIR, str(row.run_id), tmpl.ANNOT_SUBDIR, row.Index + '.fast5')
-            if os.path.exists(fpath):
-                raws.append(raw_signal(fpath))
-            elif has_src and isinstance(row.fast5_path, str) and os.path.exists(row.fast5_path):
-                raws.append(raw_signal(row.fast5_path, row.Index))
-            else:
-                raise FileNotFoundError(f'no fast5 for read {row.Index}: {fpath}')
+            raws.append(raw_signal(*_read_source(row, path, has_src)))
             names.append(row.Index)
             revs.append(bool(row.reverse))
             wins.append((int(row.l_start_raw), int(row.r_end_raw)))
     return names, revs, raws, wins
 
 
+def _read_source(row, path: str, has_src: bool):
+    """(file, read name or None) a saved overview row's signal comes from: its annotated single-read fast5,
+    else the multi-read file of the row's ``fast5_path``."""
+    fpath = os.path.join(path, tmpl.FAST5_SUBDIR, str(row.run_id), tmpl.ANNOT_SUBDIR, row.Index + '.fast5')
+    if os.path.exists(fpath):
+        return fpath, None
+    if has_src and isinstance(row.fast5_path, str) and os.path.exists(row.fast5_path):
+        return row.fast5_path, row.Index
+    raise FileNotFoundError(f'no fast5 for read {row.Index}: {fpath}')
+
+
+def get_compressed_workload(df_overview, path: str):
+    """``get_raw_workload`` without the host's StreamVByte decode: (names, reverse flags, reads as their
+    files store them (fast5.CompressedRead: zstd undone, the rest left to the GPU), windows).  Files are
+    found as ``get_raw_workload`` finds them, and each is opened and parsed once for all its rows."""
+    from .fast5 import H5File, raw_chunks
+    names, revs, reads, wins = [], [], [], []
+    has_src = 'fast5_path' in df_overview.columns
+    rows = [row for row in df_overview.itertuples() if row.saved]
+    sources = [_read_source(row, path, has_src) for row in rows]
+    by_file = {}
+    for k, (fpath, _) in enumerate(sources):
+        by_file.setdefault(fpath, []).append(k)
+    reads = [None] * len(rows)
+    for fpath, ks in by_file.items():
+        with H5File(fpath) as h5:
+            for k in ks:
+                reads[k] = raw_chunks(fpath, sources[k][1], h5)
+    for row in rows:
+        names.append(row.Index)
+        revs.append(bool(row.reverse))
+        wins.append((int(row.l_start_raw), int(row.r_end_raw)))
+    return names, revs, reads, wins
+
+
 def get_workload(df_overview, path: str, spike_removal: str = 'Brute') -> List[ReadSignal]:
     """Reads of the locus with their normalised STR windows (reference: wrapper.py:44-54): all reads are
     spike-filtered, MAD normalised and sliced in one GPU launch and returned as host float64 arrays, which
     is what the reference's ``ReadSignal`` holds.  ``main_wrapper`` does not take this detour: it hands the
-    raw reads to ``CallerWrapper.run_raw``, which keeps the windows on the device."""
+    compressed reads to ``CallerWrapper.run_compressed``, which decodes them and keeps the windows on the device."""
     from .normalize import normalize_windows
     names, revs, raws, wins = get_raw_workload(df_overview, path)
     sigs = normalize_windows(raws, wins, spike_removal)
@@ -264,9 +302,10 @@ def main_wrapper(locus: Locus, threads: int = 1, config: Optional[Config] = None
     cc = config.caller_config if config is not None else CallerConfig()
     call_wrapper = CallerWrapper(locus, threads, flanks=flanks, config=config, engine=engine)
     if workload is None:
-        # raw int16 reads -> normalisation kernel -> caller, all on the device
-        names, revs, raws, wins = get_raw_workload(df_overview, locus.path)
-        results = call_wrapper.run_raw(raws, wins, revs, cc.spike_removal)
+        # the reads' VBZ chunk bodies (zstd undone on the host) -> StreamVByte decode -> normalisation kernel
+        # -> caller, all on the device
+        names, revs, reads, wins = get_compressed_workload(df_overview, locus.path)
+        results = call_wrapper.run_compressed(reads, wins, revs, cc.spike_removal)
         workload = [ReadSignal(n, r, None) for n, r in zip(names, revs)]
     else:
         results = call_wrapper.run(workload)
