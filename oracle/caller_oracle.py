@@ -389,14 +389,15 @@ def create_alignment_bulk(trace: np.ndarray, x: np.ndarray, tb: Tables, kn: Knob
     return [RunStat(x[a:b], tb.values[trace[a]], _collapse(kn, x[a:b])) for a, b in zip(starts, ends)]
 
 
-def _tstats_bulk(data: np.ndarray, win: int) -> List[float]:
-    """t statistic at every centre of `data` (caller.py:347-354, 358): np.mean / np.std of 3 samples are
-    sequential sums; the squares are libm pow(x, 2.0) -- what `np.float64 ** 2` evaluates to."""
+def _tstat_terms(data: np.ndarray, win: int):
+    """Numerator and denominator of the t statistic at every centre of `data` (caller.py:347-354, 358),
+    the denominator before a zero is replaced: np.mean / np.std of 3 samples are sequential sums; the
+    squares are libm pow(x, 2.0) -- what `np.float64 ** 2` evaluates to."""
     from math import pow as libm_pow
     assert win == 3
     n = len(data) - 2 * win + 1
     if n <= 0:
-        return []
+        return np.zeros(0), np.zeros(0)
     w = np.lib.stride_tricks.sliding_window_view(data, win)          # w[c] = data[c:c+3]
 
     mean = ((w[:, 0] + w[:, 1]) + w[:, 2]) / 3
@@ -404,8 +405,20 @@ def _tstats_bulk(data: np.ndarray, win: int) -> List[float]:
     sd = np.sqrt(((d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]) + d[:, 2] * d[:, 2]) / 3)
     sq = np.fromiter((libm_pow(v, 2.0) for v in sd.tolist()), dtype=np.float64, count=len(sd))
     den = np.sqrt((sq[:n] + sq[win:win + n]) / win)
+    return mean[:n] - mean[win:win + n], den
+
+
+def _tstats_bulk(data: np.ndarray, win: int) -> List[float]:
+    num, den = _tstat_terms(data, win)
     den = np.where(den == 0, den + 0.0000001, den)
-    return ((mean[:n] - mean[win:win + n]) / den).tolist()
+    return (num / den).tolist()
+
+
+def zero_sd_windows(x: np.ndarray, rep_mask, trace: np.ndarray, kn: Knobs) -> int:
+    """How many t statistics of the bad-repeat mask of ``x`` along ``trace`` have two windows of zero
+    deviation, i.e. divide by the 1e-7 of caller.py:352-353 (for reads the mask does not raise on)."""
+    _, _, _, _, bounds = find_event_borders(rep_mask, trace, state_transitions(trace), kn)
+    return sum(int((_tstat_terms(x[bounds[n] - 3:b + 3], 3)[1] == 0).sum()) for n, b in enumerate(bounds[1:]))
 
 
 def segment_count_bulk(data: np.ndarray, win: int) -> int:
@@ -466,23 +479,62 @@ class OracleResult:
     badmask: np.ndarray
 
 
+@dataclass
+class FirstPass:
+    """What the reference derives from the first pass's trace (caller.py:123-126, 138)."""
+    alignment: List[RunStat]
+    rescaled: np.ndarray
+    badmask: np.ndarray
+    start: int
+    end: int
+    cost: float
+
+
+@dataclass
+class SecondPass:
+    """What the reference derives from the second pass's trace (caller.py:132-135, 139)."""
+    start: int
+    end: int
+    cost: float
+
+
+def _state_cost(runs: List[RunStat], start: int, end: int) -> float:
+    # caller.py:138-139
+    return np.mean([abs(r.state_value - r.expected) for r in runs[start:end]])
+
+
+def after_first_pass(x: np.ndarray, t1: np.ndarray, tb: Tables, kn: Knobs, bulk: bool = False) -> FirstPass:
+    """The mid-stage between the passes: alignment of ``x`` along ``t1``, rescaled signal, bad-repeat mask,
+    repeat region and state-wise cost.  Raises what the reference raises for the read."""
+    align = create_alignment_bulk if bulk else create_alignment
+    mask_of = mask_bad_repeats_bulk if bulk else mask_bad_repeats
+    runs = align(t1, x, tb, kn)
+    resc = rescale_signal(x, runs, kn)
+    start, end, bad = mask_of(x, tb.rep_mask, t1, state_transitions(t1), kn)
+    return FirstPass(alignment=runs, rescaled=np.asarray(resc), badmask=np.asarray(bad, dtype=bool),
+                     start=start, end=end, cost=_state_cost(runs, start, end))
+
+
+def after_second_pass(resc: np.ndarray, t2: np.ndarray, tb: Tables, kn: Knobs, bulk: bool = False) -> SecondPass:
+    """The stage after the second pass: the rescaled signal is rescaled again only to find the repeat region
+    (its mask is not used); returns that region and the state-wise cost."""
+    align = create_alignment_bulk if bulk else create_alignment
+    mask_of = mask_bad_repeats_bulk if bulk else mask_bad_repeats
+    runs = align(t2, resc, tb, kn)
+    resc2 = rescale_signal(resc, runs, kn)
+    start, end, _ = mask_of(resc2, tb.rep_mask, t2, state_transitions(t2), kn)
+    return SecondPass(start=start, end=end, cost=_state_cost(runs, start, end))
+
+
 def run_read(x: np.ndarray, tb: Tables, flank_length: int, reverse: bool,
              kn: Optional[Knobs] = None, impl: str = 'rows', bulk: bool = False) -> OracleResult:
     """``bulk``: the array-slice variants of the mid-stage (same arithmetic, ~3x faster)."""
     kn = kn or Knobs()
     x = np.asarray(x, dtype=np.float64)
-    align = create_alignment_bulk if bulk else create_alignment
-    mask_of = mask_bad_repeats_bulk if bulk else mask_bad_repeats
     t1 = warp(x, tb, None, kn, flank_length, impl)
-    runs1 = align(t1, x, tb, kn)
-    resc = rescale_signal(x, runs1, kn)
-    start, end, bad = mask_of(x, tb.rep_mask, t1, state_transitions(t1), kn)
-    t2 = warp(resc, tb, bad, kn, flank_length, impl)
-    runs2 = align(t2, resc, tb, kn)
-    resc2 = rescale_signal(resc, runs2, kn)
-    start2, end2, _ = mask_of(resc2, tb.rep_mask, t2, state_transitions(t2), kn)
-    cost = np.mean([abs(r.state_value - r.expected) for r in runs1[start:end]])
-    cost2 = np.mean([abs(r.state_value - r.expected) for r in runs2[start2:end2]])
-    return OracleResult(seq=decode_sequence(t1, tb, flank_length, reverse), cost=cost,
-                        resc_seq=decode_sequence(t2, tb, flank_length, reverse), resc_cost=cost2,
-                        trace1=t1, trace2=t2, rescaled=np.asarray(resc), badmask=np.asarray(bad, dtype=bool))
+    p1 = after_first_pass(x, t1, tb, kn, bulk)
+    t2 = warp(p1.rescaled, tb, p1.badmask, kn, flank_length, impl)
+    p2 = after_second_pass(p1.rescaled, t2, tb, kn, bulk)
+    return OracleResult(seq=decode_sequence(t1, tb, flank_length, reverse), cost=p1.cost,
+                        resc_seq=decode_sequence(t2, tb, flank_length, reverse), resc_cost=p2.cost,
+                        trace1=t1, trace2=t2, rescaled=p1.rescaled, badmask=p1.badmask)

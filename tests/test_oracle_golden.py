@@ -55,6 +55,33 @@ def test_bulk_oracle_equals_the_plain_one(caller_gold, oracle_c):
         assert got.cost == case['cost'] and got.resc_cost == case['resc_cost'], k
 
 
+@pytest.mark.parametrize('bulk', [False, True])
+def test_midstage_functions_on_the_reference_traces(caller_gold, oracle_c, bulk):
+    """after_first_pass / after_second_pass, fed with the reference's own traces and no DP, give the
+    reference's rescaled signal, bad-repeat mask and costs; the pooled driver over them gives the same and
+    the sequences (what tests/test_gpu_midstage.py holds the device's mid-stage to)."""
+    from oracle import bulk as ob
+    z, cases = caller_gold
+    kn = co.Knobs()
+    for case in cases:
+        k = case['key']
+        tb = _tables(case)
+        x, t1, t2 = z[f'{k}_signal'], z[f'{k}_ref_trace1'], z[f'{k}_ref_trace2']
+        p1 = co.after_first_pass(x, t1, tb, kn, bulk)
+        assert np.array_equal(p1.rescaled, z[f'{k}_ref_rescaled']), k
+        assert np.array_equal(p1.badmask, np.unpackbits(z[f'{k}_ref_badmask'])[:len(x)].astype(bool)), k
+        assert p1.cost == case['cost'], k
+        assert co.after_second_pass(p1.rescaled, t2, tb, kn, bulk).cost == case['resc_cost'], k
+        if bulk:
+            rx = case['reverse_regex'] if case['reverse'] else case['template_regex']
+            g = ob.run_midstage([rx], case['flank'], [x], [t1], [t2], [0], [case['reverse']], workers=1)[0]
+            assert g['status'] == 0, k
+            assert np.array_equal(g['rescaled'], p1.rescaled) and np.array_equal(g['mask'], p1.badmask), k
+            assert (g['seq1'], g['seq2']) == (case['seq'], case['resc_seq']), k
+            assert (g['cost1'], g['cost2']) == (case['cost'], case['resc_cost']), k
+            assert g['m'] > 3 and g['run_hist'].sum() == len(co.state_transitions(t1)), k
+
+
 def test_fill_matrices_bit_identical(caller_gold, oracle_c):
     z, cases = caller_gold
     for case in cases[:6]:

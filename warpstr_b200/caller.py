@@ -460,9 +460,11 @@ class CallerEngine:
                     o['seq2'] = torch.empty(total, dtype=torch.uint8, device=self.device)
                 o['seq_off'] = seq_off
             if want_debug:   # intermediate products, for the parity tests
-                o['trace1'] = torch.empty(d_sig.numel(), dtype=torch.int32, device=self.device)
-                o['trace2'] = torch.empty(d_sig.numel(), dtype=torch.int32, device=self.device)
-                o['rescaled'] = torch.empty(d_sig.numel(), dtype=torch.float64, device=self.device)
+                # (zeroed: the padding between reads is never written, and the tests compare whole buffers; left
+                # uninitialised it holds whatever an earlier call freed)
+                o['trace1'] = torch.zeros(d_sig.numel(), dtype=torch.int32, device=self.device)
+                o['trace2'] = torch.zeros(d_sig.numel(), dtype=torch.int32, device=self.device)
+                o['rescaled'] = torch.zeros(d_sig.numel(), dtype=torch.float64, device=self.device)
             params = _lib.CallParams(self.cc.min_values_per_state, self.cc.states_in_segment,
                                      float(self.rc.threshold), float(self.rc.max_std),
                                      1 if self.rc.method == 'median' else 0, 1 if self.rc.reps_as_one else 0,
