@@ -184,6 +184,30 @@ int wstr_warp_batch(wstr_automaton *const *automata, int32_t n_automata,
                     int32_t n_reads, void *d_workspace, int64_t workspace_bytes,
                     int32_t *d_trace, double *d_end_cost, int32_t *d_status, void *stream);
 
+/* ---- (3b) STR window search in whole reads --------------------------------------------------------
+ * Replaces the two steps of the reference that give a read its window [l_start_raw, r_end_raw] (Guppy's
+ * re-basecall with a move table, and the flank alignment mapped through it): the strand's automaton is
+ * searched against the whole normalised read (wstr_normalize_batch with window [0, N-1]) by the caller's
+ * DP with the cost |x_t - v_j| - offset, a free start in state 0 and a free end (DESIGN.md section 4.5):
+ * no mask (back = min_values_per_state on every row), no end band.  Per read:
+ *   d_lo / d_hi  int32: the best window, inclusive, in the read's sample indices (-1 when there is no path);
+ *   d_score      float64: its score, the least L[i][endstate] (+inf when there is no path);
+ *   d_status     int32, WSTR_LOCATE_*: found iff the score is below zero.
+ * Bit-exact with oracle/locate_oracle.c:wso_locate.  d_signal / sig_off / lengths as for wstr_warp_batch;
+ * lengths up to WSTR_LOCATE_MAX_SAMPLES.  All automata of a call have the same min_values_per_state; any
+ * automaton wstr_automaton_create accepts is covered (rings beyond shared memory go to the workspace).
+ * d_workspace: wstr_locate_workspace_bytes(...) bytes, 16-byte aligned; the plan travels through the
+ * staging slot, nothing is copied by the DMA engines and the call does not block. */
+#define WSTR_LOCATE_FOUND 0
+#define WSTR_LOCATE_NOT_FOUND 1           /* the best window's score is >= 0: nothing in the read matches */
+#define WSTR_LOCATE_NO_PATH 2             /* the read is shorter than the automaton's shortest path */
+#define WSTR_LOCATE_MAX_SAMPLES 2147479552 /* 2^31 - 4096 */
+int64_t wstr_locate_workspace_bytes(wstr_automaton *const *automata, int32_t n_automata, int32_t n_reads);
+int wstr_locate_batch(wstr_automaton *const *automata, int32_t n_automata, const int32_t *read_automaton,
+                      const double *d_signal, const int64_t *sig_off, const int32_t *lengths, int32_t n_reads,
+                      double offset, int32_t *d_lo, int32_t *d_hi, double *d_score, int32_t *d_status,
+                      void *d_workspace, int64_t workspace_bytes, void *stream);
+
 /* ---- whole per-read call --------------------------------------------------------------------------
  * Replaces WarpSTR.run (src/caller/caller.py:117-149) for a batch: first pass, per-run statistics
  * and spline rescale, bad-repeat mask, second pass on the rescaled signal, state-wise costs and

@@ -77,6 +77,10 @@ _SIGNATURES = {
     'wstr_call_batch': (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int32, c_i32p, c_u8p, c_vp, c_i64p, c_i32p,
                                        ctypes.c_int32, ctypes.POINTER(CallParams), c_vp, ctypes.c_int64,
                                        ctypes.POINTER(CallOutputs), c_vp]),
+    'wstr_locate_workspace_bytes': (ctypes.c_int64, [ctypes.POINTER(c_vp), ctypes.c_int32, ctypes.c_int32]),
+    'wstr_locate_batch': (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int32, c_i32p, c_vp, c_i64p, c_i32p,
+                                         ctypes.c_int32, ctypes.c_double, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int64,
+                                         c_vp]),
     'wstr_profile_enable': (ctypes.c_int, [ctypes.c_int32]),
     'wstr_profile_read': (ctypes.c_int, [c_f64p, c_i32p, ctypes.c_int32]),
 }
@@ -346,7 +350,30 @@ def call_batch(automata: Sequence[DeviceAutomaton], read_automaton, read_reverse
     check(rc, 'wstr_call_batch')
 
 
-PROFILE_CATEGORIES = ('dp_fill_traceback', 'midstage', 'normalize', 'pore_lookup', 'plan_upload')
+LOCATE_FOUND, LOCATE_NOT_FOUND, LOCATE_NO_PATH = 0, 1, 2     # d_status of wstr_locate_batch
+LOCATE_MAX_SAMPLES = 2**31 - 4096
+
+
+def locate_workspace_bytes(automata: Sequence[DeviceAutomaton], n_reads: int) -> int:
+    n = lib().wstr_locate_workspace_bytes(_handles(automata), len(automata), int(n_reads))
+    if n < 0:
+        check(int(n), 'wstr_locate_workspace_bytes')
+    return int(n)
+
+
+def locate_batch(automata: Sequence[DeviceAutomaton], read_automaton, d_signal, sig_off, lengths, offset: float,
+                 d_lo, d_hi, d_score, d_status, d_workspace, stream=None) -> None:
+    ra = _np(read_automaton, np.int32)
+    so = _np(sig_off, np.int64)
+    ln = _np(lengths, np.int32)
+    rc = lib().wstr_locate_batch(
+        _handles(automata), len(automata), _ptr(ra, c_i32p), _dptr(d_signal), _ptr(so, c_i64p), _ptr(ln, c_i32p),
+        int(ln.shape[0]), float(offset), _dptr(d_lo), _dptr(d_hi), _dptr(d_score), _dptr(d_status),
+        _dptr(d_workspace), int(d_workspace.numel() * d_workspace.element_size()), _stream_ptr(stream))
+    check(rc, 'wstr_locate_batch')
+
+
+PROFILE_CATEGORIES =('dp_fill_traceback', 'midstage', 'normalize', 'pore_lookup', 'plan_upload')
 
 
 def profile_enable(on: bool = True) -> None:

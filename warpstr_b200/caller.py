@@ -35,6 +35,15 @@ class WarpResult:
         return self.trace[keep]
 
 
+@dataclass
+class NotLocated:
+    """In place of a CallerResult: the read's STR window was not found in the whole read (DESIGN.md section
+    4.5), so the read was not called.  ``status`` is _lib.LOCATE_NOT_FOUND (the best window scores >= 0) or
+    _lib.LOCATE_NO_PATH (the read is shorter than the automaton's shortest path)."""
+    status: int
+    score: float
+
+
 _SCALARS = ('len1', 'len2', 'cost1', 'cost2', 'status', 'ties')      # per-read results of a call
 
 # exception types the reference raises for a read, by d_status code
@@ -164,12 +173,14 @@ class _IngestRaw:
         self.lengths, self.spike_mode = lengths, spike_mode
         self.sig_off, self.total = even_offsets(lengths)
         self.h2d_bytes = int(raw_off[-1]) * 2 if len(raw_off) else 0
+        self.d_raw = None
 
     def allocate(self):
         import torch
         e = self.eng
         self.d_sig = e._device_buffer('sig', self.total, torch.float64)
-        self.d_raw = e._device_buffer('raw16', int(self.raw_off[-1]), torch.int16)
+        if self.d_raw is None:
+            self.d_raw = e._device_buffer('raw16', int(self.raw_off[-1]), torch.int16)
         self.d_ss = e._device_buffer('shift_scale', 2 * len(self.lengths), torch.float64)
         pin = torch.cuda.is_available()
         cur = e._host_ss
@@ -193,6 +204,35 @@ class _IngestRaw:
     def finish(self, res, out, n):
         res['shift_scale'] = self.eng._host_ss[:2 * n].numpy().reshape(n, 2).copy()
         res['lengths'] = self.lengths
+
+
+class _IngestDeviceRaw(_IngestRaw):
+    """Whole int16 reads that are already on the device (the located-then-called chain): nothing crosses
+    PCIe, the windows are normalised and called as in _IngestRaw."""
+
+    def __init__(self, eng, d_raw, raw_off, lo, hi, lengths, spike_mode):
+        super().__init__(eng, None, raw_off, lo, hi, lengths, spike_mode)
+        self.d_raw = d_raw
+        self.h2d_bytes = 0
+
+    def send(self, a, b):
+        pass
+
+
+def pack_raw(raws):
+    """Whole int16 reads -> one pinned host buffer and the read offsets (int64[n + 1])."""
+    import torch
+    n = len(raws)
+    lens = np.fromiter((len(r) for r in raws), dtype=np.int64, count=n)
+    if (lens <= 0).any():
+        raise ValueError('empty raw read')
+    raw_off = np.zeros(n + 1, dtype=np.int64)
+    raw_off[1:] = np.cumsum(lens)
+    host = torch.empty(int(raw_off[-1]), dtype=torch.int16, pin_memory=torch.cuda.is_available())
+    hb = host.numpy()
+    for r, o in zip(raws, raw_off[:-1]):
+        hb[o:o + len(r)] = np.asarray(r, dtype=np.int16)
+    return host, raw_off
 
 
 def pack_vbz(reads):
@@ -303,6 +343,7 @@ class CallerEngine:
         self.split_small = (4096, 40000)   # batch sizes a resident call runs as two concurrent halves (None: never)
         self.ttest_guard_ulps = 0    # 0 = the library's default (16 ulp), see wstr_call_outputs.d_ttest_ties
         self.last_ttest_ties = 0     # reads of the last results_from() that were re-evaluated for a t-test tie
+        self.last_located = None     # windows of the last call_*_batch(windows=None): dict as from locate_packed
 
     # -- automata ------------------------------------------------------------------------
     def add_automaton(self, sta, flank_length: int) -> int:
@@ -652,7 +693,8 @@ class CallerEngine:
             sent = [send(a, b) for a, b in chunks]
             h2d_end = torch.cuda.Event(enable_timing=True)
             h2d_end.record(cs_in)
-            self._h2d_probe = (h2d_begin, h2d_end, int(ingest.h2d_bytes))
+            if ingest.h2d_bytes:        # (reads already on the device say nothing about the host link)
+                self._h2d_probe = (h2d_begin, h2d_end, int(ingest.h2d_bytes))
             # chunks alternate between `lanes` compute streams (each with its own workspace): the
             # kernels of consecutive chunks are independent, so one chunk's kernel tails and
             # latency-bound mid-stage overlap the next chunk's DP
@@ -781,59 +823,166 @@ class CallerEngine:
         return cur
 
     def call_raw_batch(self, raws: Sequence[np.ndarray], windows, aut_ids, reverse,
-                       spike_removal: str = 'Brute') -> List[CallerResult]:
+                       spike_removal: str = 'Brute', offset: float = 0.35) -> list:
         """Raw int16 reads and their STR windows in, CallerResults out: the reference's
         ``get_workload`` + ``CallerWrapper.run`` (wrapper.py:44-54, 104-120) as one device-resident chain
-        (``call_arrays_raw``: normalisation kernel -> caller, the float64 windows never leave the GPU)."""
-        import torch
+        (``call_arrays_raw``: normalisation kernel -> caller, the float64 windows never leave the GPU).
+
+        ``windows=None``: the windows are found first, in the whole reads, by ``locate_arrays_raw`` (score offset
+        ``offset``); the int16 reads stay on the device for the call.  A read whose window is not found is
+        not called: its entry is a ``NotLocated``.  The located windows are in ``last_located``."""
         n = len(raws)
         if n == 0:
             return []
-        lens = np.fromiter((len(r) for r in raws), dtype=np.int64, count=n)
-        if (lens <= 0).any():
-            raise ValueError('empty raw read')
-        raw_off = np.zeros(n + 1, dtype=np.int64)
-        raw_off[1:] = np.cumsum(lens)
-        host = torch.empty(int(raw_off[-1]), dtype=torch.int16, pin_memory=True)
-        hb = host.numpy()
-        for r, o in zip(raws, raw_off[:-1]):
-            hb[o:o + len(r)] = np.asarray(r, dtype=np.int16)
+        host, raw_off = pack_raw(raws)
+        aut = np.asarray(aut_ids, dtype=np.int32)
+        rev = np.asarray(reverse, dtype=np.uint8)
+        if windows is None:
+            d_raw = self._upload_raw(host)
+            return self._call_located(d_raw, raw_off, aut, rev, spike_removal, offset, lambda idx: [raws[r] for r in idx])
         lo = np.array([w[0] for w in windows], dtype=np.int32)
         hi = np.array([w[1] for w in windows], dtype=np.int32)
         if (lo < 0).any():
             raise ValueError('negative window start')
-        aut = np.asarray(aut_ids, dtype=np.int32)
-        rev = np.asarray(reverse, dtype=np.uint8)
         res = self.call_arrays_raw(host, raw_off, lo, hi, aut, rev, spike_removal)
         return self._raw_results(res, lambda idx: [raws[r] for r in idx], windows, aut_ids, reverse, spike_removal)
 
-    def call_vbz_batch(self, reads, windows, aut_ids, reverse, spike_removal: str = 'Brute') -> List[CallerResult]:
+    def call_vbz_batch(self, reads, windows, aut_ids, reverse, spike_removal: str = 'Brute',
+                       offset: float = 0.35) -> list:
         """``call_raw_batch`` for reads as their fast5 files store them (fast5.CompressedRead, from
         ``fast5.raw_chunks``): the chunk bodies go to the device, are decoded there (wstr_vbz_decode_batch) and
         called as ``call_raw_batch`` calls raw reads.  A chunk the host decoder would refuse raises that
-        Fast5FormatError, naming the file and the read, before any result is returned."""
-        from .fast5 import Fast5FormatError
+        Fast5FormatError, naming the file and the read, before any result is returned.  ``windows=None``
+        locates the windows first (``locate_arrays_vbz``): the payload crosses PCIe once and the decoded reads
+        stay on the device for the call; reads not found come back as ``NotLocated``."""
         n = len(reads)
         if n == 0:
             return []
         if any(r.n_samples <= 0 for r in reads):
             raise ValueError('empty raw read')
+        aut = np.asarray(aut_ids, dtype=np.int32)
+        rev = np.asarray(reverse, dtype=np.uint8)
+        host, table, read_chunk, raw_off = pack_vbz(reads)
+        if windows is None:
+            d_raw, chunk_status = self._decode_vbz(host, table, raw_off)
+            _raise_bad_chunk(reads, read_chunk, chunk_status.cpu().numpy())
+            return self._call_located(d_raw, raw_off, aut, rev, spike_removal, offset,
+                                      lambda idx: [reads[r].decode() for r in idx])
         lo = np.array([w[0] for w in windows], dtype=np.int32)
         hi = np.array([w[1] for w in windows], dtype=np.int32)
         if (lo < 0).any():
             raise ValueError('negative window start')
-        host, table, read_chunk, raw_off = pack_vbz(reads)
-        res = self.call_arrays_vbz(host, table, read_chunk, raw_off, lo, hi, np.asarray(aut_ids, dtype=np.int32),
-                                   np.asarray(reverse, dtype=np.uint8), spike_removal)
-        bad = np.flatnonzero(res['chunk_status'])
-        if len(bad):
-            c = int(bad[0])
-            r = int(np.searchsorted(read_chunk, c, side='right')) - 1
-            msg = _lib.VBZ_STATUS_MESSAGES.get(int(res['chunk_status'][c]), 'VBZ: corrupt chunk')
-            raise Fast5FormatError(f'{reads[r].path}: read {reads[r].read_name}: {msg} '
-                                   f'(chunk at sample {reads[r].chunks[c - int(read_chunk[r])].start})')
+        res = self.call_arrays_vbz(host, table, read_chunk, raw_off, lo, hi, aut, rev, spike_removal)
+        _raise_bad_chunk(reads, read_chunk, res['chunk_status'])
         return self._raw_results(res, lambda idx: [reads[r].decode() for r in idx], windows, aut_ids, reverse,
                                  spike_removal)
+
+    # -- STR window search in whole reads (DESIGN.md section 4.5) ----------------------------------------------
+    def locate_packed(self, d_sig, off, lengths, aut, offset: float = 0.35) -> Dict[str, np.ndarray]:
+        """wstr_locate_batch on device-resident whole normalised reads (float64, even starts ``off``).  Returns
+        host arrays: ``lo``, ``hi`` (the window, inclusive, in the read's samples), ``score`` and ``status``
+        (_lib.LOCATE_*: found iff the score is below zero)."""
+        import torch
+        n = len(lengths)
+        lengths = np.asarray(lengths, dtype=np.int32)
+        aut = np.asarray(aut, dtype=np.int32)
+        with torch.cuda.device(self.device):
+            ws = self._device_buffer('loc_ws', _lib.locate_workspace_bytes(self.automata, n), torch.uint8)
+            d_i = torch.empty((3, max(n, 1)), dtype=torch.int32, device=self.device)
+            d_score = torch.empty(max(n, 1), dtype=torch.float64, device=self.device)
+            _lib.locate_batch(self.automata, aut, d_sig, off, lengths, offset, d_i[0], d_i[1], d_score, d_i[2], ws)
+            h_i = d_i.cpu().numpy()
+            score = d_score.cpu().numpy()
+        return dict(lo=h_i[0, :n].copy(), hi=h_i[1, :n].copy(), score=score[:n].copy(), status=h_i[2, :n].copy())
+
+    def locate_arrays_raw(self, host_raw, raw_off, aut, spike_removal: str = 'Brute',
+                          offset: float = 0.35) -> Dict[str, np.ndarray]:
+        """Whole int16 reads ``host_raw[raw_off[r] : raw_off[r+1]]`` (``pack_raw``) in, their STR windows out:
+        whole-read normalisation (wstr_normalize_batch, window [0, N-1]) and the window search on the device.
+        Same dict as ``locate_packed``."""
+        raw_off = np.asarray(raw_off, dtype=np.int64)
+        return self._locate_device(self._upload_raw(host_raw), raw_off, np.asarray(aut, dtype=np.int32),
+                                   spike_removal, offset)
+
+    def locate_arrays_vbz(self, host_payload, table, read_chunk, raw_off, aut, spike_removal: str = 'Brute',
+                          offset: float = 0.35) -> Dict[str, np.ndarray]:
+        """``locate_arrays_raw`` for VBZ-compressed reads (``pack_vbz``): decoded on the device first.  The dict
+        also carries ``chunk_status`` (WSTR_VBZ_* per chunk; a read with a bad chunk has undefined results)."""
+        raw_off = np.asarray(raw_off, dtype=np.int64)
+        d_raw, chunk_status = self._decode_vbz(host_payload, table, raw_off)
+        res = self._locate_device(d_raw, raw_off, np.asarray(aut, dtype=np.int32), spike_removal, offset)
+        res['chunk_status'] = chunk_status.cpu().numpy()
+        return res
+
+    def _upload_raw(self, host_raw):
+        import torch
+        with torch.cuda.device(self.device):
+            d_raw = self._device_buffer('loc_raw16', int(host_raw.numel()), torch.int16)
+            d_raw.copy_(host_raw, non_blocking=True)
+        return d_raw
+
+    def _decode_vbz(self, host_payload, table, raw_off):
+        """Payload -> device -> decoded whole int16 reads (device) and the per-chunk status (device)."""
+        import torch
+        m = len(table['in_off'])
+        with torch.cuda.device(self.device):
+            d_pay = self._device_buffer('vbz_payload', int(host_payload.numel()), torch.uint8)
+            d_pay.copy_(host_payload, non_blocking=True)
+            d_raw = self._device_buffer('loc_raw16', int(raw_off[-1]), torch.int16)
+            d_st = torch.zeros(max(m, 1), dtype=torch.int32, device=self.device)
+            if m:
+                ws = self._device_buffer('vbz_ws0', _lib.vbz_workspace_bytes(m), torch.uint8)
+                _lib.vbz_decode_batch(d_pay, table['in_off'], table['in_bytes'], table['n_samples'], table['n_out'],
+                                      table['kind'], table['zigzag'], table['out_off'], d_raw, d_st, ws)
+        return d_raw, d_st[:m]
+
+    def _locate_device(self, d_raw, raw_off, aut, spike_removal, offset) -> Dict[str, np.ndarray]:
+        """Whole-read normalisation of int16 reads on the device, then the window search."""
+        import torch
+        from .normalize import SPIKE_MODES
+        lens = np.diff(raw_off)
+        if (lens > _lib.LOCATE_MAX_SAMPLES).any():
+            raise ValueError(f'a read longer than {_lib.LOCATE_MAX_SAMPLES} samples cannot be located')
+        lengths = lens.astype(np.int32)
+        n = len(lengths)
+        sig_off, total = even_offsets(lengths)
+        with torch.cuda.device(self.device):
+            d_sig = torch.empty(total, dtype=torch.float64, device=self.device)
+            ws = self._device_buffer('norm_ws0', _lib.normalize_workspace_bytes(n), torch.uint8)
+            _lib.normalize_batch(d_raw, raw_off, np.zeros(n, dtype=np.int32), lengths - 1, SPIKE_MODES[spike_removal],
+                                 d_sig, sig_off, None, ws)
+            res = self.locate_packed(d_sig, sig_off, lengths, aut, offset)
+            del d_sig
+        return res
+
+    def _call_located(self, d_raw, raw_off, aut, rev, spike_removal, offset, raws_of) -> list:
+        """The located-then-called chain on whole int16 reads already on the device: locate, bring the windows
+        to the host, normalise the found windows and call them from the same device buffer."""
+        import torch
+        from .normalize import SPIKE_MODES
+        loc = self._locate_device(d_raw, raw_off, aut, spike_removal, offset)
+        self.last_located = loc
+        out: list = [NotLocated(int(st), float(sc)) for st, sc in zip(loc['status'], loc['score'])]
+        found = np.flatnonzero(loc['status'] == _lib.LOCATE_FOUND)
+        if not len(found):
+            return out
+        if len(found) < len(out):         # the found reads, packed
+            with torch.cuda.device(self.device):
+                d_raw = torch.cat([d_raw[int(raw_off[r]):int(raw_off[r + 1])] for r in found])
+            sub_off = np.zeros(len(found) + 1, dtype=np.int64)
+            sub_off[1:] = np.cumsum(np.diff(raw_off)[found])
+        else:
+            sub_off = raw_off
+        lo, hi = loc['lo'][found], loc['hi'][found]
+        lengths = (hi - lo + 1).astype(np.int32)
+        ingest = _IngestDeviceRaw(self, d_raw, sub_off, lo, hi, lengths, SPIKE_MODES[spike_removal])
+        res = self._pipeline(ingest, lengths, aut[found], rev[found], True, 25000, 2)
+        windows = list(zip(lo.tolist(), hi.tolist()))
+        calls = self._raw_results(res, lambda idx: raws_of([int(found[k]) for k in idx]), windows,
+                                  aut[found].tolist(), [bool(x) for x in rev[found]], spike_removal)
+        for k, r in enumerate(found):
+            out[r] = calls[k]
+        return out
 
     def _raw_results(self, res, raws_of, windows, aut_ids, reverse, spike_removal) -> List[CallerResult]:
         """CallerResults of a ``call_arrays_raw``-style result dict.  Reads the device did not finish, or whose
@@ -922,6 +1071,18 @@ class CallerEngine:
             return midstage.after_pass(trace, x, tb['values'], tb['rep_mask'], self.cc, self.rc, second)
         except midstage.ReadError as e:
             raise e.kind(str(e))
+
+
+def _raise_bad_chunk(reads, read_chunk, chunk_status) -> None:
+    """The Fast5FormatError of the first chunk the device decoder refused, naming the file and the read."""
+    from .fast5 import Fast5FormatError
+    bad = np.flatnonzero(chunk_status)
+    if len(bad):
+        c = int(bad[0])
+        r = int(np.searchsorted(read_chunk, c, side='right')) - 1
+        msg = _lib.VBZ_STATUS_MESSAGES.get(int(chunk_status[c]), 'VBZ: corrupt chunk')
+        raise Fast5FormatError(f'{reads[r].path}: read {reads[r].read_name}: {msg} '
+                               f'(chunk at sample {reads[r].chunks[c - int(read_chunk[r])].start})')
 
 
 _default_engine: Optional[CallerEngine] = None

@@ -7,6 +7,11 @@ single-read file under ``<output>/<locus>/fast5/<run_id>/annot/`` (h5py) and wri
 overview keeps the ``fast5_path`` column (the reference keeps it too) and
 ``wrapper.get_workload`` reads the signal straight from the multi-read file.
 
+The STR window columns ``l_start_raw, r_end_raw`` may be left out, or left empty in some rows: the
+caller then finds those reads' windows itself in the whole read (``wrapper.main_wrapper``, DESIGN.md
+section 4.5), so the reads of a locus (their names and strands, e.g. from a BAM) and the run's fast5
+files are enough.
+
     python -m warpstr_b200.caller_only --config cfg.yaml --file reads.csv
 """
 import argparse
@@ -18,7 +23,8 @@ import yaml
 
 from . import fast5
 
-REQUIRED = ['fast5_path', 'locus', 'read_name', 'reverse', 'l_start_raw', 'r_end_raw']
+REQUIRED = ['fast5_path', 'locus', 'read_name', 'reverse']
+WINDOW = ['l_start_raw', 'r_end_raw']       # optional; an overview always gets them, empty where not given
 
 
 def prepare(output: str, csv_path: str, check_reads: bool = True) -> Dict[str, str]:
@@ -29,8 +35,10 @@ def prepare(output: str, csv_path: str, check_reads: bool = True) -> Dict[str, s
     with open(csv_path, 'r') as fh:
         reader = csv.reader(fh)
         header = next(reader)
-        if any(col not in REQUIRED + ['run_id'] for col in header) or any(col not in header for col in REQUIRED):
-            raise ValueError(f'Not all required columns present in input CSV file. Required fields are: {REQUIRED}')
+        if any(col not in REQUIRED + WINDOW + ['run_id'] for col in header) or any(col not in header for col in REQUIRED):
+            raise ValueError(f'Not all required columns present in input CSV file. Required fields are: {REQUIRED}, '
+                             f'optional: {WINDOW + ["run_id"]}')
+        add_win = [c for c in WINDOW if c not in header]
         add_run_id = 'run_id' not in header
         rows: Dict[str, List[List[str]]] = {}
         known: Dict[str, set] = {}
@@ -44,8 +52,9 @@ def prepare(output: str, csv_path: str, check_reads: bool = True) -> Dict[str, s
                     known[src] = set(fast5.read_names(src))
                 if rec['read_name'] not in known[src]:
                     raise ValueError(f"Read {rec['read_name']} not found in fast5 file {src}")
-            rows.setdefault(rec['locus'], []).append(row + (['run_0'] if add_run_id else []) + ['1'])
-    out_header = header + (['run_id'] if add_run_id else []) + ['saved']
+            rows.setdefault(rec['locus'], []).append(row + [''] * len(add_win) + (['run_0'] if add_run_id else []) +
+                                                     ['1'])
+    out_header = header + add_win + (['run_id'] if add_run_id else []) + ['saved']
     written = {}
     for locus, lines in rows.items():
         dest = os.path.join(output, locus)

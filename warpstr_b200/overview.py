@@ -26,11 +26,16 @@ def load_overview(locus_path: str):
 
 
 def append_results(seq_results: Sequence[Tuple[str, str]], cost_results: Sequence[Tuple[float, float]], df):
-    """One entry per overview row; rows that were not extracted (``saved`` false) get -1."""
+    """One entry per overview row; rows that were not extracted (``saved`` false) get -1, saved rows without a
+    result (``None`` in ``seq_results``: the STR window was not found) get None."""
     fasta, results, orig, c1, c2 = [], [], [], [], []
     k = 0
     for row in df.itertuples():
-        if row.saved:
+        if row.saved and seq_results[k] is None:
+            for col in (results, orig, c1, c2):
+                col.append(None)
+            k += 1
+        elif row.saved:
             seq, resc = seq_results[k]
             results.append(len(resc))
             orig.append(len(seq))
@@ -64,6 +69,9 @@ def write_results_to_fasta(fasta: List[Tuple[str, str, bool]], locus_path: str) 
 def save_overview(overview_path: str, df, results, orig, c1, c2):
     old = [c for c in df.columns if c.startswith('result')]
     df.drop(columns=old, inplace=True)
+    if any(r is None for r in results):    # rows without a result: empty cells, the other lengths still integers
+        results, orig = pd.array(results, dtype='Int64'), pd.array(orig, dtype='Int64')
+        c1, c2 = pd.array(c1, dtype='Float64'), pd.array(c2, dtype='Float64')
     df['results'] = results
     df['orig'] = orig
     df['dtw_cost1'] = c1

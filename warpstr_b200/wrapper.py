@@ -12,6 +12,7 @@ from dataclasses import dataclass
 from typing import List, Optional, Sequence
 
 import numpy as np
+import pandas as pd
 
 from . import templates as tmpl
 from .automata import StateAutomata
@@ -120,22 +121,54 @@ class CallerWrapper:
         return self.engine.call_batch(signals, aut, reverse)
 
     def run_raw(self, raws: Sequence[np.ndarray], windows, reverse: Sequence[bool],
-                spike_removal: Optional[str] = None) -> List[CallerResult]:
+                spike_removal: Optional[str] = None, offset: float = 0.35) -> list:
         """``get_workload`` + ``run`` for reads still in DAC counts (wrapper.py:44-54, 104-120): normalised
-        and called on the device in one chain, order preserved."""
+        and called on the device in one chain, order preserved.  ``windows=None``: each read's STR window is
+        first found in the whole read (``locate_raw``); a read whose window is not found comes back as a
+        ``caller.NotLocated`` instead of a CallerResult, and the windows are in ``engine.last_located``."""
         reverse = [bool(r) for r in reverse]
         aut = [self._rev_id if rv else self._temp_id for rv in reverse]
         return self.engine.call_raw_batch(raws, windows, aut, reverse,
-                                          spike_removal or self.caller_config.spike_removal)
+                                          spike_removal or self.caller_config.spike_removal, offset)
 
     def run_compressed(self, reads, windows, reverse: Sequence[bool],
-                       spike_removal: Optional[str] = None) -> List[CallerResult]:
+                       spike_removal: Optional[str] = None, offset: float = 0.35) -> list:
         """``run_raw`` for reads as their fast5 files store them (fast5.CompressedRead, see
         ``get_compressed_workload``): the VBZ decode happens on the device too, order preserved."""
         reverse = [bool(r) for r in reverse]
         aut = [self._rev_id if rv else self._temp_id for rv in reverse]
         return self.engine.call_vbz_batch(reads, windows, aut, reverse,
-                                          spike_removal or self.caller_config.spike_removal)
+                                          spike_removal or self.caller_config.spike_removal, offset)
+
+    # -- STR windows without a basecall (DESIGN.md section 4.5) ----------------------------------------------
+    def locate_raw(self, raws: Sequence[np.ndarray], reverse: Sequence[bool], spike_removal: Optional[str] = None,
+                   offset: float = 0.35) -> dict:
+        """The STR window ``[lo, hi]`` of every whole raw read, found by searching the strand's automaton
+        (flank - repeat - flank) in the whole normalised read: host arrays ``lo``, ``hi``, ``score`` and
+        ``status`` (0 found, 1 nothing scores below zero, 2 the read is too short).  The strand is an input."""
+        from .caller import pack_raw
+        reverse = [bool(r) for r in reverse]
+        if not raws:
+            return dict(lo=np.zeros(0, np.int32), hi=np.zeros(0, np.int32), score=np.zeros(0), status=np.zeros(0, np.int32))
+        host, raw_off = pack_raw(raws)
+        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
+        return self.engine.locate_arrays_raw(host, raw_off, aut, spike_removal or self.caller_config.spike_removal,
+                                             offset)
+
+    def locate_compressed(self, reads, reverse: Sequence[bool], spike_removal: Optional[str] = None,
+                          offset: float = 0.35) -> dict:
+        """``locate_raw`` for reads as their fast5 files store them (fast5.CompressedRead): decoded on the device.
+        A chunk the host decoder would refuse raises that Fast5FormatError."""
+        from .caller import _raise_bad_chunk, pack_vbz
+        reverse = [bool(r) for r in reverse]
+        if not reads:
+            return dict(lo=np.zeros(0, np.int32), hi=np.zeros(0, np.int32), score=np.zeros(0), status=np.zeros(0, np.int32))
+        host, table, read_chunk, raw_off = pack_vbz(reads)
+        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
+        res = self.engine.locate_arrays_vbz(host, table, read_chunk, raw_off, aut,
+                                            spike_removal or self.caller_config.spike_removal, offset)
+        _raise_bad_chunk(reads, read_chunk, res.pop('chunk_status'))
+        return res
 
     # -- state similarity report (wrapper.py:122-160) ------------------------------------------------
     def check_high_similarity(self, sequence: str):
@@ -228,7 +261,8 @@ class CallerWrapper:
 
 
 def get_raw_workload(df_overview, path: str):
-    """The saved reads of a locus as they are on disk: (names, reverse flags, raw int16 signals, windows).
+    """The saved reads of a locus as they are on disk: (names, reverse flags, raw int16 signals, windows; a
+    window is None where the row leaves it empty).
     The raw signal of every saved read comes from its annotated single-read fast5
     (``<locus>/fast5/<run_id>/annot/<read>.fast5``, what the reference's extraction step
     writes) or, for a caller-only run prepared straight from a sequencing run's multi-read
@@ -241,8 +275,15 @@ def get_raw_workload(df_overview, path: str):
             raws.append(raw_signal(*_read_source(row, path, has_src)))
             names.append(row.Index)
             revs.append(bool(row.reverse))
-            wins.append((int(row.l_start_raw), int(row.r_end_raw)))
+            wins.append(_window(row))
     return names, revs, raws, wins
+
+
+def _window(row):
+    """(l_start_raw, r_end_raw) of an overview row, or None where the row leaves them empty (caller_only.py)."""
+    if pd.isna(row.l_start_raw) or pd.isna(row.r_end_raw):
+        return None
+    return int(row.l_start_raw), int(row.r_end_raw)
 
 
 def _read_source(row, path: str, has_src: bool):
@@ -276,7 +317,7 @@ def get_compressed_workload(df_overview, path: str):
     for row in rows:
         names.append(row.Index)
         revs.append(bool(row.reverse))
-        wins.append((int(row.l_start_raw), int(row.r_end_raw)))
+        wins.append(_window(row))
     return names, revs, reads, wins
 
 
@@ -291,12 +332,48 @@ def get_workload(df_overview, path: str, spike_removal: str = 'Brute') -> List[R
     return [ReadSignal(n, r, s) for n, r, s in zip(names, revs, sigs)]
 
 
+def _run_locating(call_wrapper, df_overview, names, revs, reads, wins, spike_removal, offset):
+    """main_wrapper's call of a locus where some rows leave their window empty: those reads are located in
+    the whole read first and their windows are written into the overview's two columns; a read whose window
+    is not found gets no result (a caller.NotLocated), and all such reads are named in one warning."""
+    import warnings
+    results = [None] * len(reads)
+    given = [k for k, w in enumerate(wins) if w is not None]
+    missing = [k for k, w in enumerate(wins) if w is None]
+    if given:
+        for k, r in zip(given, call_wrapper.run_compressed([reads[k] for k in given], [wins[k] for k in given],
+                                                           [revs[k] for k in given], spike_removal)):
+            results[k] = r
+    located = call_wrapper.run_compressed([reads[k] for k in missing], None, [revs[k] for k in missing],
+                                          spike_removal, offset)
+    loc = call_wrapper.engine.last_located
+    lo = df_overview['l_start_raw'].astype('Int64')
+    hi = df_overview['r_end_raw'].astype('Int64')
+    lost = []
+    for i, (k, r) in enumerate(zip(missing, located)):
+        results[k] = r
+        if loc['status'][i] == 0:
+            lo[names[k]] = int(loc['lo'][i])
+            hi[names[k]] = int(loc['hi'][i])
+        else:
+            lost.append(names[k])
+    df_overview['l_start_raw'] = lo
+    df_overview['r_end_raw'] = hi
+    if lost:
+        warnings.warn(f'{len(lost)} read(s) without a window in the overview: the STR window was not found in the '
+                      f'whole read, so they have no result: {", ".join(map(str, lost))}', RuntimeWarning, stacklevel=3)
+    return results
+
+
 def main_wrapper(locus: Locus, threads: int = 1, config: Optional[Config] = None,
                  workload: Optional[Sequence[ReadSignal]] = None, flanks: Optional[Flanks] = None,
-                 engine: Optional[CallerEngine] = None):
+                 engine: Optional[CallerEngine] = None, offset: float = 0.35):
     """The caller step of one locus (reference: wrapper.py:17-41): overview.csv in, calls on the
     GPU, overview.csv / FASTA / complex-unit CSV out.  Plots are not produced.  ``workload``
-    (one ReadSignal per saved overview row, in row order) bypasses the fast5 reading."""
+    (one ReadSignal per saved overview row, in row order) bypasses the fast5 reading.  Rows whose
+    ``l_start_raw`` / ``r_end_raw`` are empty are located in the whole read first (DESIGN.md section 4.5,
+    score offset ``offset``) and get the located window written into those columns; rows whose window is not
+    found keep empty result columns."""
     from .overview import load_overview, store_collapsed, store_results
     overview_path, df_overview = load_overview(locus.path)
     cc = config.caller_config if config is not None else CallerConfig()
@@ -305,17 +382,22 @@ def main_wrapper(locus: Locus, threads: int = 1, config: Optional[Config] = None
         # the reads' VBZ chunk bodies (zstd undone on the host) -> StreamVByte decode -> normalisation kernel
         # -> caller, all on the device
         names, revs, reads, wins = get_compressed_workload(df_overview, locus.path)
-        results = call_wrapper.run_compressed(reads, wins, revs, cc.spike_removal)
+        if all(w is not None for w in wins):
+            results = call_wrapper.run_compressed(reads, wins, revs, cc.spike_removal)
+        else:
+            results = _run_locating(call_wrapper, df_overview, names, revs, reads, wins, cc.spike_removal, offset)
         workload = [ReadSignal(n, r, None) for n, r in zip(names, revs)]
     else:
         results = call_wrapper.run(workload)
-    seq_results = [(r.seq, r.resc_seq) for r in results]
-    cost_results = [(r.cost, r.resc_cost) for r in results]
+    seq_results = [(r.seq, r.resc_seq) if isinstance(r, CallerResult) else None for r in results]
+    cost_results = [(r.cost, r.resc_cost) if isinstance(r, CallerResult) else None for r in results]
     df_overview = store_results(overview_path, df_overview, seq_results, cost_results, locus.path)
     df_collapsed = None
     if len(call_wrapper.units) > 1:
         print(f'Running complex genotyping as complex repeat units present: {call_wrapper.units}')
-        collapsed = [call_wrapper.collapse_repeats(s[1]) for s in seq_results]
+        called = [k for k, sr in enumerate(seq_results) if sr is not None]
+        workload = [workload[k] for k in called]
+        collapsed = [call_wrapper.collapse_repeats(seq_results[k][1]) for k in called]
         df_collapsed = store_collapsed(collapsed, call_wrapper.units, call_wrapper.repeat_units,
                                        [bool(r.reverse) for r in workload], locus.path)
     return df_overview, df_collapsed
