@@ -5,8 +5,11 @@
 1. Locate rate (reads/s, DP cells/s with cells = N x S per read) of CallerEngine.locate_packed on device-resident
    whole normalised reads of ~150 000 samples (HD locus), for 10 and 2 000 reads, against the FP64 add rate
    measured in the same run (wstr_measure_fp64_add_rate).  A cell costs at least mv + 1 + in-degree FP64 adds.
-2. Files to overview.csv: main_wrapper on multi-read VBZ fast5 files of a caller-only overview, once with every
-   window given and once with the window columns left empty (located first), on the same files.
+   Strand mode, on the same reads: the single-strand search with the true strands against the both-strand search
+   (every read a (template, reverse) pair, two entries per read; its cells count both strands), alternated.
+2. Files to overview.csv: main_wrapper on multi-read VBZ fast5 files of a caller-only overview, with every
+   window given, with the window columns left empty (located first) and with the window and ``reverse``
+   columns left empty (located on both strands), on the same files.
 Card name and power limit are read in the same run and written beside the numbers.
 """
 import argparse
@@ -63,28 +66,40 @@ def bench_locate(n, samples, reps):
     host, off, lengths = pack_signals(sigs)
     d_sig = host.to(eng.device)
     aut = [ids[int(r)] for r in rev]
+    pairs = [tuple(ids)] * n
     res = eng.locate_packed(d_sig, off, lengths, aut)          # warm-up, also the accuracy figure below
+    both = eng.locate_packed(d_sig, off, lengths, pairs)
     torch.cuda.synchronize()
-    t = []
-    for _ in range(reps):
+    t, t2 = [], []
+    for _ in range(reps):                                      # single and both strands alternated
         t0 = time.perf_counter()
         eng.locate_packed(d_sig, off, lengths, aut)            # ends in a device-to-host copy: synchronised
         t.append(time.perf_counter() - t0)
-    sec = float(np.median(t))
+        t0 = time.perf_counter()
+        eng.locate_packed(d_sig, off, lengths, pairs)
+        t2.append(time.perf_counter() - t0)
+    sec, sec2 = float(np.median(t)), float(np.median(t2))
     S = np.array([stas[int(r)].n_states for r in rev], dtype=np.float64)
     cells = float((lengths.astype(np.float64) * S).sum())
+    cells2 = float(lengths.astype(np.float64).sum()) * float(stas[0].n_states + stas[1].n_states)
     deg = stas[0].n_edges / stas[0].n_states
     w = np.array(wins)
     err = np.maximum(np.abs(res['lo'] - w[:, 0]), np.abs(res['hi'] - w[:, 1]))
+    truth = np.array(rev, dtype=np.int8)
+    gap = np.abs(both['strand_score'][:, 0] - both['strand_score'][:, 1])
     return dict(reads=n, samples_per_read=int(np.mean(lengths)), states=int(S.mean()), seconds_median=sec,
                 seconds_all=t, reads_per_s=n / sec, cells_per_s=cells / sec,
                 fp64_adds_per_cell_min=float(eng.cc.min_values_per_state + 1 + deg),
                 found=int((res['status'] == 0).sum()), end_error_max=int(err.max()),
-                end_error_p99=float(np.percentile(err, 99)))
+                end_error_p99=float(np.percentile(err, 99)),
+                both_strands=dict(seconds_median=sec2, seconds_all=t2, reads_per_s=n / sec2, cells_per_s=cells2 / sec2,
+                                  time_over_single_strand=sec2 / sec, right_strand=int((both['strand'] == truth).sum()),
+                                  same_window_as_single=int(((both['lo'] == res['lo']) & (both['hi'] == res['hi'])).sum()),
+                                  score_gap_min=float(gap.min())))
 
 
 def bench_files(n_reads, samples, reps):
-    """files -> overview.csv with windows given vs located, same fast5 files."""
+    """files -> overview.csv with windows given vs located vs located on both strands, same fast5 files."""
     import warnings
     import _h5write as hw
     from warpstr_b200 import caller_only, synth
@@ -105,12 +120,13 @@ def bench_files(n_reads, samples, reps):
             hw.write_multi(p, d, 'vbz0', chunk=4000)
             paths.append(p)
         out = {}
-        for mode in ('given', 'located'):
+        for mode in ('given', 'located', 'detected'):
             csv_path = os.path.join(tmp, f'{mode}.csv')
             with open(csv_path, 'w') as fh:
                 fh.write('fast5_path,locus,read_name,reverse,l_start_raw,r_end_raw\n')
                 for k, rid, rv, a, b in rows:
-                    fh.write(f'{paths[k]},LOC,{rid},{rv},{a if mode == "given" else ""},{b if mode == "given" else ""}\n')
+                    win = f'{a},{b}' if mode == 'given' else ','
+                    fh.write(f'{paths[k]},LOC,{rid},{rv if mode != "detected" else ""},{win}\n')
             times = []
             for rep in range(reps + 1):
                 o = os.path.join(tmp, f'out_{mode}')
@@ -126,6 +142,7 @@ def bench_files(n_reads, samples, reps):
                     times.append(time.perf_counter() - t0)
             out[mode] = dict(seconds_median=float(np.median(times)), seconds_all=times)
         out['located_over_given'] = out['located']['seconds_median'] / out['given']['seconds_median']
+        out['detected_over_given'] = out['detected']['seconds_median'] / out['given']['seconds_median']
         out['reads'] = n_reads
         out['samples_per_read'] = samples
         return out

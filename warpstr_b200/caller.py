@@ -44,6 +44,55 @@ class NotLocated:
     score: float
 
 
+def choose_strand(status, score):
+    """The strand of reads searched on both strands (DESIGN.md section 4.5).  ``status`` / ``score``: (n, 2), column
+    0 the template automaton's search, column 1 the reverse automaton's.  The rule:
+
+    * found (_lib.LOCATE_FOUND) on one strand only: that strand;
+    * found on both: the lower score; an exact tie goes to the template (no margin);
+    * found on neither: no strand (-1), status LOCATE_NOT_FOUND if either search had it, else LOCATE_NO_PATH,
+      and the lower score.
+
+    Returns (strand int8[n]: 0 template, 1 reverse, -1 neither; col int64[n]: the column the window and score
+    come from, the lower score's (template on a tie) where neither is found; status int32[n]; score float64[n])."""
+    status = np.asarray(status).reshape(-1, 2)
+    score = np.asarray(score, dtype=np.float64).reshape(-1, 2)
+    found = status == _lib.LOCATE_FOUND
+    lower_rev = score[:, 1] < score[:, 0]
+    both, neither = found.all(axis=1), ~found.any(axis=1)
+    col = np.where(both | neither, lower_rev, found[:, 1]).astype(np.int64)
+    strand = np.where(neither, -1, col).astype(np.int8)
+    st = np.where(neither, np.where((status == _lib.LOCATE_NOT_FOUND).any(axis=1), _lib.LOCATE_NOT_FOUND,
+                                    _lib.LOCATE_NO_PATH), _lib.LOCATE_FOUND).astype(np.int32)
+    return strand, col, st, score[np.arange(len(col)), col]
+
+
+def split_pairs(aut):
+    """Per read one automaton id or a (template id, reverse id) pair -> (pair bool[n], ids int32[n, 2]); a read
+    given one id has it in both columns."""
+    if isinstance(aut, np.ndarray) and aut.ndim == 1:
+        ids = aut.astype(np.int32)
+        return np.zeros(len(ids), dtype=bool), np.stack((ids, ids), axis=1)
+    n = len(aut)
+    ids = np.empty((n, 2), dtype=np.int32)
+    pair = np.zeros(n, dtype=bool)
+    for r, a in enumerate(aut):
+        if np.ndim(a) == 0:
+            ids[r] = int(a)
+        else:
+            ids[r] = [int(x) for x in a]
+            pair[r] = True
+    return pair, ids
+
+
+def fill_given_strands(loc, reverse) -> None:
+    """Completes ``loc['strand']`` of a locate dict: a read with a given strand (``reverse[r]`` a bool; None for a
+    read searched on both strands) gets that strand, found or not."""
+    given = np.array([r is not None for r in reverse], dtype=bool)
+    rv = np.array([bool(r) if r is not None else False for r in reverse], dtype=np.int8)
+    loc['strand'] = np.where(given, rv, loc['strand']).astype(np.int8)
+
+
 _SCALARS = ('len1', 'len2', 'cost1', 'cost2', 'status', 'ties')      # per-read results of a call
 
 # exception types the reference raises for a read, by d_status code
@@ -830,16 +879,20 @@ class CallerEngine:
 
         ``windows=None``: the windows are found first, in the whole reads, by ``locate_arrays_raw`` (score offset
         ``offset``); the int16 reads stay on the device for the call.  A read whose window is not found is
-        not called: its entry is a ``NotLocated``.  The located windows are in ``last_located``."""
+        not called: its entry is a ``NotLocated``.  The located windows are in ``last_located``.  Here an entry
+        of ``aut_ids`` may be a (template id, reverse id) pair (its ``reverse`` entry is ignored, e.g. None): the
+        read is searched on both strands and called with the strand ``choose_strand`` picks, whose id and
+        orientation are then used; ``last_located['strand']`` has every read's strand, given or detected."""
         n = len(raws)
         if n == 0:
             return []
         host, raw_off = pack_raw(raws)
-        aut = np.asarray(aut_ids, dtype=np.int32)
-        rev = np.asarray(reverse, dtype=np.uint8)
         if windows is None:
             d_raw = self._upload_raw(host)
-            return self._call_located(d_raw, raw_off, aut, rev, spike_removal, offset, lambda idx: [raws[r] for r in idx])
+            return self._call_located(d_raw, raw_off, aut_ids, reverse, spike_removal, offset,
+                                      lambda idx: [raws[r] for r in idx])
+        aut = _single_ids(aut_ids)
+        rev = np.asarray(reverse, dtype=np.uint8)
         lo = np.array([w[0] for w in windows], dtype=np.int32)
         hi = np.array([w[1] for w in windows], dtype=np.int32)
         if (lo < 0).any():
@@ -854,20 +907,21 @@ class CallerEngine:
         called as ``call_raw_batch`` calls raw reads.  A chunk the host decoder would refuse raises that
         Fast5FormatError, naming the file and the read, before any result is returned.  ``windows=None``
         locates the windows first (``locate_arrays_vbz``): the payload crosses PCIe once and the decoded reads
-        stay on the device for the call; reads not found come back as ``NotLocated``."""
+        stay on the device for the call; reads not found come back as ``NotLocated``.  Strand pairs in ``aut_ids``
+        as in ``call_raw_batch``."""
         n = len(reads)
         if n == 0:
             return []
         if any(r.n_samples <= 0 for r in reads):
             raise ValueError('empty raw read')
-        aut = np.asarray(aut_ids, dtype=np.int32)
-        rev = np.asarray(reverse, dtype=np.uint8)
         host, table, read_chunk, raw_off = pack_vbz(reads)
         if windows is None:
             d_raw, chunk_status = self._decode_vbz(host, table, raw_off)
             _raise_bad_chunk(reads, read_chunk, chunk_status.cpu().numpy())
-            return self._call_located(d_raw, raw_off, aut, rev, spike_removal, offset,
+            return self._call_located(d_raw, raw_off, aut_ids, reverse, spike_removal, offset,
                                       lambda idx: [reads[r].decode() for r in idx])
+        aut = _single_ids(aut_ids)
+        rev = np.asarray(reverse, dtype=np.uint8)
         lo = np.array([w[0] for w in windows], dtype=np.int32)
         hi = np.array([w[1] for w in windows], dtype=np.int32)
         if (lo < 0).any():
@@ -881,28 +935,55 @@ class CallerEngine:
     def locate_packed(self, d_sig, off, lengths, aut, offset: float = 0.35) -> Dict[str, np.ndarray]:
         """wstr_locate_batch on device-resident whole normalised reads (float64, even starts ``off``).  Returns
         host arrays: ``lo``, ``hi`` (the window, inclusive, in the read's samples), ``score`` and ``status``
-        (_lib.LOCATE_*: found iff the score is below zero)."""
+        (_lib.LOCATE_*: found iff the score is below zero).
+
+        ``aut[r]`` is one automaton id, or a (template id, reverse id) pair for a read whose strand is not known.
+        Such a read enters the launch twice, both entries on the same samples, one after the other (the plan's
+        stable longest-first order keeps them adjacent, so both CTAs read the read while it is in L2), and
+        ``choose_strand`` decides: ``lo``, ``hi``, ``score``, ``status`` are the chosen strand's, ``strand`` is
+        0 (template), 1 (reverse) or -1 (found on neither), and ``strand_score`` (float64[n, 2]),
+        ``strand_status``, ``strand_lo``, ``strand_hi`` (int32[n, 2]) hold both searches.  A read given one id
+        has NaN / -1 there and ``strand`` -1: which strand its automaton is is the caller's to say
+        (``fill_given_strands``)."""
         import torch
         n = len(lengths)
         lengths = np.asarray(lengths, dtype=np.int32)
-        aut = np.asarray(aut, dtype=np.int32)
+        off = np.asarray(off, dtype=np.int64)
+        pair, ids = split_pairs(aut)
+        reps = 1 + pair.astype(np.int64)
+        first = np.cumsum(reps) - reps                       # each read's first entry
+        entry_read = np.repeat(np.arange(n), reps)
+        entry_aut = ids[entry_read, np.arange(len(entry_read)) - first[entry_read]]
+        m = len(entry_read)
         with torch.cuda.device(self.device):
-            ws = self._device_buffer('loc_ws', _lib.locate_workspace_bytes(self.automata, n), torch.uint8)
-            d_i = torch.empty((3, max(n, 1)), dtype=torch.int32, device=self.device)
-            d_score = torch.empty(max(n, 1), dtype=torch.float64, device=self.device)
-            _lib.locate_batch(self.automata, aut, d_sig, off, lengths, offset, d_i[0], d_i[1], d_score, d_i[2], ws)
+            ws = self._device_buffer('loc_ws', _lib.locate_workspace_bytes(self.automata, m), torch.uint8)
+            d_i = torch.empty((3, max(m, 1)), dtype=torch.int32, device=self.device)
+            d_score = torch.empty(max(m, 1), dtype=torch.float64, device=self.device)
+            _lib.locate_batch(self.automata, entry_aut, d_sig, off[entry_read], lengths[entry_read], offset,
+                              d_i[0], d_i[1], d_score, d_i[2], ws)
             h_i = d_i.cpu().numpy()
-            score = d_score.cpu().numpy()
-        return dict(lo=h_i[0, :n].copy(), hi=h_i[1, :n].copy(), score=score[:n].copy(), status=h_i[2, :n].copy())
+            e_score = d_score.cpu().numpy()
+        second = first + pair
+        st2 = np.stack((h_i[2, first], h_i[2, second]), axis=1)
+        sc2 = np.stack((e_score[first], e_score[second]), axis=1)
+        strand, col, status, score = choose_strand(st2, sc2)     # a single entry is its own "pair": unchanged
+        pick = np.where(col == 1, second, first)
+        lo2 = np.stack((h_i[0, first], h_i[0, second]), axis=1)
+        hi2 = np.stack((h_i[1, first], h_i[1, second]), axis=1)
+        strand[~pair] = -1
+        for a in (st2, lo2, hi2):
+            a[~pair] = -1
+        sc2[~pair] = np.nan
+        return dict(lo=h_i[0, pick], hi=h_i[1, pick], score=score, status=status, strand=strand,
+                    strand_score=sc2, strand_status=st2, strand_lo=lo2, strand_hi=hi2)
 
     def locate_arrays_raw(self, host_raw, raw_off, aut, spike_removal: str = 'Brute',
                           offset: float = 0.35) -> Dict[str, np.ndarray]:
         """Whole int16 reads ``host_raw[raw_off[r] : raw_off[r+1]]`` (``pack_raw``) in, their STR windows out:
         whole-read normalisation (wstr_normalize_batch, window [0, N-1]) and the window search on the device.
-        Same dict as ``locate_packed``."""
+        ``aut`` and the dict as in ``locate_packed``."""
         raw_off = np.asarray(raw_off, dtype=np.int64)
-        return self._locate_device(self._upload_raw(host_raw), raw_off, np.asarray(aut, dtype=np.int32),
-                                   spike_removal, offset)
+        return self._locate_device(self._upload_raw(host_raw), raw_off, aut, spike_removal, offset)
 
     def locate_arrays_vbz(self, host_payload, table, read_chunk, raw_off, aut, spike_removal: str = 'Brute',
                           offset: float = 0.35) -> Dict[str, np.ndarray]:
@@ -910,7 +991,7 @@ class CallerEngine:
         also carries ``chunk_status`` (WSTR_VBZ_* per chunk; a read with a bad chunk has undefined results)."""
         raw_off = np.asarray(raw_off, dtype=np.int64)
         d_raw, chunk_status = self._decode_vbz(host_payload, table, raw_off)
-        res = self._locate_device(d_raw, raw_off, np.asarray(aut, dtype=np.int32), spike_removal, offset)
+        res = self._locate_device(d_raw, raw_off, aut, spike_removal, offset)
         res['chunk_status'] = chunk_status.cpu().numpy()
         return res
 
@@ -955,13 +1036,18 @@ class CallerEngine:
             del d_sig
         return res
 
-    def _call_located(self, d_raw, raw_off, aut, rev, spike_removal, offset, raws_of) -> list:
+    def _call_located(self, d_raw, raw_off, aut_ids, reverse, spike_removal, offset, raws_of) -> list:
         """The located-then-called chain on whole int16 reads already on the device: locate, bring the windows
-        to the host, normalise the found windows and call them from the same device buffer."""
+        to the host, normalise the found windows and call them from the same device buffer, each with the
+        automaton and orientation of its strand (given, or chosen by the both-strand search)."""
         import torch
         from .normalize import SPIKE_MODES
-        loc = self._locate_device(d_raw, raw_off, aut, spike_removal, offset)
+        loc = self._locate_device(d_raw, raw_off, aut_ids, spike_removal, offset)
+        pair, ids = split_pairs(aut_ids)
+        fill_given_strands(loc, [None if p else r for p, r in zip(pair, reverse)])
         self.last_located = loc
+        rev = loc['strand'].clip(0, 1).astype(np.uint8)
+        aut = ids[np.arange(len(rev)), rev]
         out: list = [NotLocated(int(st), float(sc)) for st, sc in zip(loc['status'], loc['score'])]
         found = np.flatnonzero(loc['status'] == _lib.LOCATE_FOUND)
         if not len(found):
@@ -1071,6 +1157,16 @@ class CallerEngine:
             return midstage.after_pass(trace, x, tb['values'], tb['rep_mask'], self.cc, self.rc, second)
         except midstage.ReadError as e:
             raise e.kind(str(e))
+
+
+def _single_ids(aut_ids) -> np.ndarray:
+    """Automaton ids of reads called on given windows: one per read, a strand pair is refused (the strand is not
+    searched inside a given window)."""
+    pair, ids = split_pairs(aut_ids)
+    if pair.any():
+        raise ValueError(f'read {int(np.flatnonzero(pair)[0])} of the batch: a given window needs a given strand '
+                         '(one automaton id, not a pair)')
+    return ids[:, 0].copy()
 
 
 def _raise_bad_chunk(reads, read_chunk, chunk_status) -> None:

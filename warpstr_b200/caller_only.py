@@ -9,8 +9,10 @@ overview keeps the ``fast5_path`` column (the reference keeps it too) and
 
 The STR window columns ``l_start_raw, r_end_raw`` may be left out, or left empty in some rows: the
 caller then finds those reads' windows itself in the whole read (``wrapper.main_wrapper``, DESIGN.md
-section 4.5), so the reads of a locus (their names and strands, e.g. from a BAM) and the run's fast5
-files are enough.
+section 4.5).  The ``reverse`` column is required but its cells may be empty too: such a read is searched
+on both strands and the strand found is written into the overview.  So the run's fast5 files and the
+names of a locus's reads are enough, e.g. read IDs of targeted or adaptive sampling, which come without
+strands.  A window is only taken with its strand: a row with a window and an empty ``reverse`` is refused.
 
     python -m warpstr_b200.caller_only --config cfg.yaml --file reads.csv
 """
@@ -46,6 +48,9 @@ def prepare(output: str, csv_path: str, check_reads: bool = True) -> Dict[str, s
             if not row:
                 continue
             rec = dict(zip(header, row))
+            if not rec.get('reverse', '').strip() and any(rec.get(c, '').strip() for c in WINDOW):
+                raise ValueError(f"Read {rec['read_name']}: a window (l_start_raw, r_end_raw) is given without "
+                                 f"its strand (reverse is empty)")
             if check_reads:
                 src = rec['fast5_path']
                 if src not in known:

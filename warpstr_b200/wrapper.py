@@ -16,7 +16,7 @@ import pandas as pd
 
 from . import templates as tmpl
 from .automata import StateAutomata
-from .caller import CallerEngine, CallerResult
+from .caller import CallerEngine, CallerResult, fill_given_strands
 from .config import CallerConfig, Config, RescalerConfig
 from .pore_model import PoreModel, get_pore_model
 
@@ -115,59 +115,77 @@ class CallerWrapper:
 
     # -- the call (wrapper.py:104-120) ---------------------------------------------------------------
     def run(self, workload: Sequence[ReadSignal]) -> List[CallerResult]:
+        """The reference's call: float64 STR windows, each with its strand (a None strand raises ValueError)."""
         signals = [np.ascontiguousarray(r.signal, dtype=np.float64) for r in workload]
-        reverse = [bool(r.reverse) for r in workload]
-        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
+        reverse = _strands([r.reverse for r in workload])
+        _need_strands(reverse, [r.name for r in workload], 'a ReadSignal')
+        aut = self._aut(reverse)
         return self.engine.call_batch(signals, aut, reverse)
 
-    def run_raw(self, raws: Sequence[np.ndarray], windows, reverse: Sequence[bool],
+    def run_raw(self, raws: Sequence[np.ndarray], windows, reverse: Sequence[Optional[bool]],
                 spike_removal: Optional[str] = None, offset: float = 0.35) -> list:
         """``get_workload`` + ``run`` for reads still in DAC counts (wrapper.py:44-54, 104-120): normalised
         and called on the device in one chain, order preserved.  ``windows=None``: each read's STR window is
         first found in the whole read (``locate_raw``); a read whose window is not found comes back as a
-        ``caller.NotLocated`` instead of a CallerResult, and the windows are in ``engine.last_located``."""
-        reverse = [bool(r) for r in reverse]
-        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
-        return self.engine.call_raw_batch(raws, windows, aut, reverse,
+        ``caller.NotLocated`` instead of a CallerResult, and the windows are in ``engine.last_located``.  There
+        a strand may be None: the read is searched on both strands and called on the one found
+        (``caller.choose_strand``); ``engine.last_located['strand']`` has every read's strand (0 template,
+        1 reverse, -1 found on neither).  Given windows need given strands (ValueError naming the read)."""
+        reverse = _strands(reverse)
+        if windows is not None:
+            _need_strands(reverse, [f'#{k}' for k in range(len(reverse))], 'a given window')
+        return self.engine.call_raw_batch(raws, windows, self._aut(reverse), reverse,
                                           spike_removal or self.caller_config.spike_removal, offset)
 
-    def run_compressed(self, reads, windows, reverse: Sequence[bool],
+    def run_compressed(self, reads, windows, reverse: Sequence[Optional[bool]],
                        spike_removal: Optional[str] = None, offset: float = 0.35) -> list:
         """``run_raw`` for reads as their fast5 files store them (fast5.CompressedRead, see
-        ``get_compressed_workload``): the VBZ decode happens on the device too, order preserved."""
-        reverse = [bool(r) for r in reverse]
-        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
-        return self.engine.call_vbz_batch(reads, windows, aut, reverse,
+        ``get_compressed_workload``): the VBZ decode happens on the device too, order preserved.  None strands
+        as in ``run_raw``."""
+        reverse = _strands(reverse)
+        if windows is not None:
+            _need_strands(reverse, [r.read_name for r in reads], 'a given window')
+        return self.engine.call_vbz_batch(reads, windows, self._aut(reverse), reverse,
                                           spike_removal or self.caller_config.spike_removal, offset)
 
+    def _aut(self, reverse):
+        """Per read the automaton of its strand, or the (template, reverse) pair where the strand is None."""
+        return [(self._temp_id, self._rev_id) if rv is None else self._rev_id if rv else self._temp_id
+                for rv in reverse]
+
     # -- STR windows without a basecall (DESIGN.md section 4.5) ----------------------------------------------
-    def locate_raw(self, raws: Sequence[np.ndarray], reverse: Sequence[bool], spike_removal: Optional[str] = None,
-                   offset: float = 0.35) -> dict:
+    def locate_raw(self, raws: Sequence[np.ndarray], reverse: Sequence[Optional[bool]],
+                   spike_removal: Optional[str] = None, offset: float = 0.35) -> dict:
         """The STR window ``[lo, hi]`` of every whole raw read, found by searching the strand's automaton
         (flank - repeat - flank) in the whole normalised read: host arrays ``lo``, ``hi``, ``score`` and
-        ``status`` (0 found, 1 nothing scores below zero, 2 the read is too short).  The strand is an input."""
+        ``status`` (0 found, 1 nothing scores below zero, 2 the read is too short).  A read whose strand is None
+        is searched on both strands and ``caller.choose_strand`` picks one; ``strand`` holds every read's strand
+        (0 template, 1 reverse, given or detected; -1 found on neither), ``strand_score`` / ``strand_status`` /
+        ``strand_lo`` / ``strand_hi`` (n, 2) both searches of those reads (NaN / -1 for a read with a given
+        strand)."""
         from .caller import pack_raw
-        reverse = [bool(r) for r in reverse]
+        reverse = _strands(reverse)
         if not raws:
-            return dict(lo=np.zeros(0, np.int32), hi=np.zeros(0, np.int32), score=np.zeros(0), status=np.zeros(0, np.int32))
+            return _no_reads()
         host, raw_off = pack_raw(raws)
-        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
-        return self.engine.locate_arrays_raw(host, raw_off, aut, spike_removal or self.caller_config.spike_removal,
-                                             offset)
+        res = self.engine.locate_arrays_raw(host, raw_off, self._aut(reverse),
+                                            spike_removal or self.caller_config.spike_removal, offset)
+        fill_given_strands(res, reverse)
+        return res
 
-    def locate_compressed(self, reads, reverse: Sequence[bool], spike_removal: Optional[str] = None,
+    def locate_compressed(self, reads, reverse: Sequence[Optional[bool]], spike_removal: Optional[str] = None,
                           offset: float = 0.35) -> dict:
         """``locate_raw`` for reads as their fast5 files store them (fast5.CompressedRead): decoded on the device.
         A chunk the host decoder would refuse raises that Fast5FormatError."""
         from .caller import _raise_bad_chunk, pack_vbz
-        reverse = [bool(r) for r in reverse]
+        reverse = _strands(reverse)
         if not reads:
-            return dict(lo=np.zeros(0, np.int32), hi=np.zeros(0, np.int32), score=np.zeros(0), status=np.zeros(0, np.int32))
+            return _no_reads()
         host, table, read_chunk, raw_off = pack_vbz(reads)
-        aut = [self._rev_id if rv else self._temp_id for rv in reverse]
-        res = self.engine.locate_arrays_vbz(host, table, read_chunk, raw_off, aut,
+        res = self.engine.locate_arrays_vbz(host, table, read_chunk, raw_off, self._aut(reverse),
                                             spike_removal or self.caller_config.spike_removal, offset)
         _raise_bad_chunk(reads, read_chunk, res.pop('chunk_status'))
+        fill_given_strands(res, reverse)
         return res
 
     # -- state similarity report (wrapper.py:122-160) ------------------------------------------------
@@ -274,9 +292,42 @@ def get_raw_workload(df_overview, path: str):
         if row.saved:
             raws.append(raw_signal(*_read_source(row, path, has_src)))
             names.append(row.Index)
-            revs.append(bool(row.reverse))
+            revs.append(_strand(row))
             wins.append(_window(row))
     return names, revs, raws, wins
+
+
+def _strands(reverse) -> list:
+    """Strand flags as bools, None kept (a strand to be found)."""
+    return [None if r is None else bool(r) for r in reverse]
+
+
+def _need_strands(reverse, names, what: str) -> None:
+    missing = [str(n) for n, r in zip(names, reverse) if r is None]
+    if missing:
+        raise ValueError(f'read {missing[0]}: {what} needs a strand (reverse), and none is given'
+                         + (f' (nor for {len(missing) - 1} more)' if len(missing) > 1 else ''))
+
+
+def _no_reads() -> dict:
+    return dict(lo=np.zeros(0, np.int32), hi=np.zeros(0, np.int32), score=np.zeros(0), status=np.zeros(0, np.int32),
+                strand=np.zeros(0, np.int8), strand_score=np.zeros((0, 2)), strand_status=np.zeros((0, 2), np.int32),
+                strand_lo=np.zeros((0, 2), np.int32), strand_hi=np.zeros((0, 2), np.int32))
+
+
+def _strand(row) -> Optional[bool]:
+    """``reverse`` of an overview row, or None where the row leaves it empty (caller_only.py): the strand is
+    then found in the whole read.  pandas reads a column of True, False and empty cells as bools and NaN; a cell
+    read as text (a column with other values) is parsed, never passed to bool(), for which 'False' is true."""
+    v = row.reverse
+    if isinstance(v, str):
+        t = v.strip().lower()
+        if t in ('true', 'false', ''):
+            return None if t == '' else t == 'true'
+        raise ValueError(f'read {row.Index}: reverse must be True, False or empty, not {v!r}')
+    if pd.isna(v):
+        return None
+    return bool(v)
 
 
 def _window(row):
@@ -316,7 +367,7 @@ def get_compressed_workload(df_overview, path: str):
                 reads[k] = raw_chunks(fpath, sources[k][1], h5)
     for row in rows:
         names.append(row.Index)
-        revs.append(bool(row.reverse))
+        revs.append(_strand(row))
         wins.append(_window(row))
     return names, revs, reads, wins
 
@@ -334,10 +385,13 @@ def get_workload(df_overview, path: str, spike_removal: str = 'Brute') -> List[R
 
 def _run_locating(call_wrapper, df_overview, names, revs, reads, wins, spike_removal, offset):
     """main_wrapper's call of a locus where some rows leave their window empty: those reads are located in
-    the whole read first and their windows are written into the overview's two columns; a read whose window
-    is not found gets no result (a caller.NotLocated), and all such reads are named in one warning."""
+    the whole read first (on both strands where ``reverse`` is empty too) and their windows, and detected
+    strands, are written into the overview's columns; a read whose window is not found gets no result (a
+    caller.NotLocated) and keeps its empty cells, and all such reads are named in one warning.  Returns the
+    results and the strands (detected ones filled in; None for a read found on neither)."""
     import warnings
     results = [None] * len(reads)
+    revs = list(revs)
     given = [k for k, w in enumerate(wins) if w is not None]
     missing = [k for k, w in enumerate(wins) if w is None]
     if given:
@@ -349,20 +403,27 @@ def _run_locating(call_wrapper, df_overview, names, revs, reads, wins, spike_rem
     loc = call_wrapper.engine.last_located
     lo = df_overview['l_start_raw'].astype('Int64')
     hi = df_overview['r_end_raw'].astype('Int64')
+    detect = any(revs[k] is None for k in missing)
+    strand = df_overview['reverse'].astype(object) if detect else None
     lost = []
     for i, (k, r) in enumerate(zip(missing, located)):
         results[k] = r
         if loc['status'][i] == 0:
             lo[names[k]] = int(loc['lo'][i])
             hi[names[k]] = int(loc['hi'][i])
+            if revs[k] is None:
+                revs[k] = bool(loc['strand'][i] == 1)
+                strand[names[k]] = revs[k]
         else:
             lost.append(names[k])
     df_overview['l_start_raw'] = lo
     df_overview['r_end_raw'] = hi
+    if detect:
+        df_overview['reverse'] = strand
     if lost:
         warnings.warn(f'{len(lost)} read(s) without a window in the overview: the STR window was not found in the '
                       f'whole read, so they have no result: {", ".join(map(str, lost))}', RuntimeWarning, stacklevel=3)
-    return results
+    return results, revs
 
 
 def main_wrapper(locus: Locus, threads: int = 1, config: Optional[Config] = None,
@@ -372,8 +433,10 @@ def main_wrapper(locus: Locus, threads: int = 1, config: Optional[Config] = None
     GPU, overview.csv / FASTA / complex-unit CSV out.  Plots are not produced.  ``workload``
     (one ReadSignal per saved overview row, in row order) bypasses the fast5 reading.  Rows whose
     ``l_start_raw`` / ``r_end_raw`` are empty are located in the whole read first (DESIGN.md section 4.5,
-    score offset ``offset``) and get the located window written into those columns; rows whose window is not
-    found keep empty result columns."""
+    score offset ``offset``) and get the located window written into those columns; rows whose ``reverse`` is
+    empty as well are searched on both strands and get the detected strand written into ``reverse`` (so the
+    FASTA files and the complex-unit CSV split on it); rows whose window is not found keep empty result columns.
+    A row with a window but no strand raises ValueError."""
     from .overview import load_overview, store_collapsed, store_results
     overview_path, df_overview = load_overview(locus.path)
     cc = config.caller_config if config is not None else CallerConfig()
@@ -385,7 +448,8 @@ def main_wrapper(locus: Locus, threads: int = 1, config: Optional[Config] = None
         if all(w is not None for w in wins):
             results = call_wrapper.run_compressed(reads, wins, revs, cc.spike_removal)
         else:
-            results = _run_locating(call_wrapper, df_overview, names, revs, reads, wins, cc.spike_removal, offset)
+            results, revs = _run_locating(call_wrapper, df_overview, names, revs, reads, wins, cc.spike_removal,
+                                          offset)
         workload = [ReadSignal(n, r, None) for n, r in zip(names, revs)]
     else:
         results = call_wrapper.run(workload)
