@@ -150,7 +150,9 @@ int wstr_automaton_plan(const int32_t *in_ptr, const int32_t *in_idx, int32_t n_
 /* info[0]=states per lane (K), info[1]=direction-code bits per lane per row (32/info[1] rows
  * share a 32-bit word), info[2]=chain slots (KC), info[3]=generic slots (KG), info[4]=n_states,
  * info[5]=n_edges, info[6]=states placed in generic slots, info[7]=1 if no edge leads from a
- * state kept by the end band into a skipped one (the band test then stops mv rows into it) */
+ * state kept by the end band into a skipped one (the band test then stops mv rows into it),
+ * info[8]=candidate encoding of the generic slots (DEG: 2 or 4 per slot, 100 + d "low", 200 + 10a + b
+ * "graded"; 0 for the catch-all kernel).  Copies min(n_info, 9) values. */
 int wstr_automaton_info(const wstr_automaton *a, int32_t *info, int32_t n_info);
 /* state index stored at each of the 32*K kernel positions (-1 = padding); for tests */
 int wstr_automaton_layout(const wstr_automaton *a, int32_t *state_of_pos, int32_t n_pos);

@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 
+import _layouts as lay
 from warpstr_b200 import config as cfg
 from warpstr_b200 import midstage, synth
 from warpstr_b200.automata import StateAutomata
@@ -92,45 +93,7 @@ def test_kernel_layout_plan_invariants(built_lib):
         for rx in (locus.template_regex, locus.reverse_regex):
             sta = StateAutomata(rx)
             info, sop = _lib.automaton_plan(sta.in_ptr, sta.in_idx, sta.n_states)
-            KC, KG = info['chain_slots'], info['generic_slots']
-            K = KC + KG
-            assert sorted(int(s) for s in sop if s >= 0) == list(range(sta.n_states))
-            pos = {int(s): p for p, s in enumerate(sop) if s >= 0}
-            deg = np.diff(sta.in_ptr)
-            code = info['unrolled_in_degree']   # 2 / 4; 100 + d: "low" layout; 200 + 10a + b: "graded" layout
-            KGn = KG
-
-            def slot_deg(g):                    # candidates generic slot g is built with (dtw.cu: slot_deg)
-                if code >= 200:
-                    return (code - 200) // 10 if g == KGn - 1 else ((code - 200) % 10 if g == KGn - 2 else 1)
-                if code >= 100:
-                    return code - 100 if g == KGn - 1 else 1
-                return code
-            for s_, p_ in pos.items():
-                u_ = p_ % K
-                if u_ >= KC:
-                    assert deg[s_] <= slot_deg(u_ - KC), (name, s_, u_, code)
-            outdeg = np.bincount(sta.in_idx, minlength=sta.n_states)
-            for s, p in pos.items():
-                lane, u = divmod(p, K)
-                if u >= KC:
-                    continue
-                # a chain slot holds a state with at most one incoming edge ...
-                assert deg[s] <= 1
-                if u > 0:
-                    # ... which comes from the slot before it, and that state feeds nothing else
-                    pred = int(sta.incoming_of(s)[0])
-                    assert pos[pred] == p - 1 and outdeg[pred] == 1
-                elif deg[s] == 1:
-                    # slot 0 reads a published value: a generic state or another lane's tail
-                    pp = pos[int(sta.incoming_of(s)[0])]
-                    assert pp % K >= KC or pp % K == KC - 1
-            # every predecessor of a generic state is published as well
-            for s, p in pos.items():
-                if p % K >= KC:
-                    for q in sta.incoming_of(s):
-                        pp = pos[int(q)]
-                        assert pp % K >= KC or pp % K == KC - 1
+            lay.assert_layout_invariants(sta.in_ptr, sta.in_idx, sta.n_states, info, sop, name)
 
 
 def test_layout_plan_never_refuses_what_the_reference_accepts(built_lib):

@@ -165,10 +165,10 @@ class DeviceAutomaton:
                    sta.endstate, flank_length, min_values_per_state)
 
     def info(self) -> dict:
-        buf = np.zeros(8, dtype=np.int32)
-        check(lib().wstr_automaton_info(self.handle, _ptr(buf, c_i32p), 8), 'wstr_automaton_info')
+        buf = np.zeros(9, dtype=np.int32)
+        check(lib().wstr_automaton_info(self.handle, _ptr(buf, c_i32p), 9), 'wstr_automaton_info')
         keys = ('states_per_lane', 'dir_bits_per_row', 'chain_slots', 'generic_slots', 'n_states', 'n_edges',
-                'generic_states', 'band_closed')
+                'generic_states', 'band_closed', 'unrolled_in_degree')
         return dict(zip(keys, (int(x) for x in buf)))
 
     def layout(self) -> np.ndarray:

@@ -114,7 +114,7 @@ struct Split {
     int kc, kg;
     unsigned mv_mask;   // bit mv set = instantiated for that min_values_per_state
 };
-// keep in sync with wstr_launch_fill in dtw.cu
+// the same splits as the WSTR_CASE lines of wstr_launch_fill in dtw.cu (tests/test_fill_dispatch.py checks it)
 const Split kSplits[] = {{7, 1, 0x10}, {6, 2, 0x1fc}, {8, 1, 0x10}, {4, 4, 0x10}, {7, 2, 0x10}, {8, 2, 0x10},
                          {6, 4, 0x1fc}, {7, 4, 0x10}, {8, 4, 0x10}, {12, 4, 0x10}};
 
@@ -522,9 +522,9 @@ extern "C" int wstr_automaton_destroy(wstr_automaton *a) {
 
 extern "C" int wstr_automaton_info(const wstr_automaton *a, int32_t *info, int32_t n_info) {
     if (!a || !info) return WSTR_ERR_INVALID_ARGUMENT;
-    const int32_t vals[8] = {a->dev.K,  a->dev.NB,  a->dev.KC,     a->dev.KG,
-                             a->dev.S,  a->n_edges, a->n_generic,  a->dev.band_closed};
-    for (int i = 0; i < n_info && i < 8; ++i) info[i] = vals[i];
+    const int32_t vals[9] = {a->dev.K,  a->dev.NB,  a->dev.KC,    a->dev.KG,          a->dev.S,
+                             a->n_edges, a->n_generic, a->dev.band_closed, a->dev.DEG};
+    for (int i = 0; i < n_info && i < 9; ++i) info[i] = vals[i];
     return WSTR_OK;
 }
 

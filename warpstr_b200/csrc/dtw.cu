@@ -758,7 +758,8 @@ int launch_fill_deg(int deg, const FillParams &p, cudaStream_t s) {
 
 }  // namespace
 
-// The (chain, generic) slot splits the library is built with; keep in sync with kSplits in api.cu.
+// The (chain, generic) slot splits the library is built with: the same as kSplits in api.cu
+// (tests/test_fill_dispatch.py checks both lists and that every instantiation has a test target).
 // The instantiations take minutes to compile, so this file is compiled several times in parallel, each
 // time with -DWSTR_FILL_PART=n for one group of them (__graft_entry__.py: FILL_PARTS); without the macro
 // everything lands in one object.
