@@ -90,8 +90,9 @@ int wstr_dequantize_batch(const int16_t *d_raw, const int64_t *raw_off, const in
 
 /* ---- (2c) VBZ-compressed raw signal --------------------------------------------------------------
  * Replaces the StreamVByte + zig-zag delta half of the VBZ HDF5 filter (nanoporetech/vbz_compression)
- * that h5py runs when the reference reads Raw/.../Signal (src/schemas/fast5.py:50-52); zstd stays on the
- * host.  Chunk c's body after zstd is d_payload[in_off[c] .. in_off[c] + in_bytes[c]); kind[c]:
+ * that h5py runs when the reference reads Raw/.../Signal (src/schemas/fast5.py:50-52); zstd is undone
+ * before, by wstr_zstd_decode_batch (2d) or on the host.  Chunk c's body after zstd is
+ * d_payload[in_off[c] .. in_off[c] + in_bytes[c]); kind[c]:
  *   WSTR_VBZ_KIND_V0   VBZ version 0: ceil(n/4) bytes of 2-bit codes (c + 1 data bytes), then the data;
  *   WSTR_VBZ_KIND_V1   VBZ version 1 (16-bit integers): ceil(n/8) bytes of 1-bit keys, then the data;
  *   WSTR_VBZ_KIND_RAW  verbatim little-endian int16 (a chunk the host decoded itself).
@@ -101,8 +102,10 @@ int wstr_dequantize_batch(const int16_t *d_raw, const int64_t *raw_off, const in
  * warpstr_b200/fast5.py:vbz_decompress including its wrap-around to 16 bits; its format errors become
  * d_status[c] (WSTR_VBZ_*), and a bad chunk leaves its own output range undefined and nothing else.
  * The payload is fetched in whole 16-byte words: d_payload and every in_off must be 16-byte aligned, and
- * the bytes up to in_off + in_bytes rounded up to 16 readable (the Python layer pads each chunk with
- * zeros); no byte outside that padded span is read.  Output ranges of the chunks must not overlap.
+ * the bytes up to in_off + in_bytes rounded up to 16 readable; no byte outside that padded span is read, and
+ * a chunk the decoder accepts never depends on the padding bytes' values (the Python layer zero-pads the
+ * chunks it uploads; the padding behind a body wstr_zstd_decode_batch wrote is left as it was).  Output
+ * ranges of the chunks must not overlap.
  * d_workspace: wstr_vbz_workspace_bytes(n_chunks) bytes; the chunk table travels through the staging
  * slot like every other call's host arrays. */
 #define WSTR_VBZ_KIND_V0 0
@@ -117,6 +120,33 @@ int wstr_vbz_decode_batch(const uint8_t *d_payload, const int64_t *in_off, const
                           const int32_t *n_samples, const int32_t *n_out, const int32_t *kind,
                           const int32_t *zigzag, const int64_t *out_off, int32_t n_chunks, int16_t *d_raw,
                           int32_t *d_status, void *d_workspace, int64_t workspace_bytes, void *stream);
+
+/* ---- (2d) zstd frames -------------------------------------------------------------------------------------
+ * The zstd half of the VBZ filter (RFC 8878, Zstandard), so that a VBZ chunk can cross PCIe as its file stores
+ * it.  Frame f is d_in[in_off[f] .. in_off[f] + in_bytes[f]) and holds exactly one zstd frame; out_bytes[f] is
+ * its Frame_Content_Size (the host reads it from the header).  Its content is written to
+ * d_out[out_off[f] .. out_off[f] + out_bytes[f]) and d_status[f] is WSTR_ZSTD_OK, or non-zero where libzstd's
+ * ZSTD_decompress would refuse the frame or return a size other than out_bytes[f] (the codes below name the
+ * section that failed); a failed frame leaves its own output range undefined and nothing else.  Every block
+ * type, literal type and sequence-table mode is decoded; frames with a content checksum or without a content
+ * size are refused (WSTR_ZSTD_UNSUPPORTED: decode those on the host), and no dictionary is ever loaded.
+ * The input is fetched in aligned words: d_in and every in_off must be 16-byte aligned, and the bytes up to
+ * in_off + in_bytes rounded up to 16 readable (zero padding); no byte outside that padded span is read and
+ * no byte outside [out_off, out_off + out_bytes) is written.  Output ranges of the frames must not overlap.
+ * d_workspace: wstr_zstd_workspace_bytes(n_frames) bytes; the frame table travels through the staging slot
+ * like every other call's host arrays.  The call does not block. */
+#define WSTR_ZSTD_OK 0
+#define WSTR_ZSTD_FRAME_HEADER 1          /* bad magic, reserved bit set, window too large, a dictionary ID, or too short */
+#define WSTR_ZSTD_UNSUPPORTED 2           /* content checksum or no Frame_Content_Size: the host decodes such frames */
+#define WSTR_ZSTD_SIZE 3                  /* Frame_Content_Size differs from out_bytes, or the blocks produce another size */
+#define WSTR_ZSTD_BLOCK 4                 /* block header: reserved type, size past the frame's end or above 128 KB */
+#define WSTR_ZSTD_CORRUPT 5               /* a compressed block fails a check of its literals or sequences section */
+#define WSTR_ZSTD_TRAILING 6              /* bytes follow the last block */
+int64_t wstr_zstd_workspace_bytes(int32_t n_frames);
+int wstr_zstd_decode_batch(const uint8_t *d_in, const int64_t *in_off, const int64_t *in_bytes,
+                           const int64_t *out_off, const int64_t *out_bytes, int32_t n_frames,
+                           uint8_t *d_out, int32_t *d_status, void *d_workspace, int64_t workspace_bytes,
+                           void *stream);
 
 /* ---- (3) DTW state automaton ----------------------------------------------------------------
  * wstr_automaton_create uploads one strand's automaton: the flat form of StateAutomata

@@ -55,6 +55,9 @@ _SIGNATURES = {
     'wstr_vbz_workspace_bytes': (ctypes.c_int64, [ctypes.c_int32]),
     'wstr_vbz_decode_batch': (ctypes.c_int, [c_vp, c_i64p, c_i64p, c_i32p, c_i32p, c_i32p, c_i32p, c_i64p,
                                              ctypes.c_int32, c_vp, c_vp, c_vp, ctypes.c_int64, c_vp]),
+    'wstr_zstd_workspace_bytes': (ctypes.c_int64, [ctypes.c_int32]),
+    'wstr_zstd_decode_batch': (ctypes.c_int, [c_vp, c_i64p, c_i64p, c_i64p, c_i64p, ctypes.c_int32, c_vp, c_vp, c_vp,
+                                              ctypes.c_int64, c_vp]),
     'wstr_automaton_create': (ctypes.c_int, [c_f64p, c_i32p, c_i32p, c_i32p, c_u8p, c_u8p, ctypes.c_int32,
                                              ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                              ctypes.POINTER(c_vp)]),
@@ -303,6 +306,25 @@ def vbz_decode_batch(d_payload, in_off, in_bytes, n_samples, n_out, kind, zigzag
         _ptr(zz, c_i32p), _ptr(oo, c_i64p), int(io.shape[0]), _dptr(d_raw), _dptr(d_status), _dptr(d_workspace),
         int(d_workspace.numel() * d_workspace.element_size()), _stream_ptr(stream))
     check(rc, 'wstr_vbz_decode_batch')
+
+
+def zstd_workspace_bytes(n_frames: int) -> int:
+    n = lib().wstr_zstd_workspace_bytes(int(n_frames))
+    if n < 0:
+        check(int(n), 'wstr_zstd_workspace_bytes')
+    return int(n)
+
+
+def zstd_decode_batch(d_in, in_off, in_bytes, out_off, out_bytes, d_out, d_status, d_workspace, stream=None) -> None:
+    io = _np(in_off, np.int64)
+    ib = _np(in_bytes, np.int64)
+    oo = _np(out_off, np.int64)
+    ob = _np(out_bytes, np.int64)
+    rc = lib().wstr_zstd_decode_batch(
+        _dptr(d_in), _ptr(io, c_i64p), _ptr(ib, c_i64p), _ptr(oo, c_i64p), _ptr(ob, c_i64p), int(io.shape[0]),
+        _dptr(d_out), _dptr(d_status), _dptr(d_workspace), int(d_workspace.numel() * d_workspace.element_size()),
+        _stream_ptr(stream))
+    check(rc, 'wstr_zstd_decode_batch')
 
 
 def measure_fp64_add_rate(stream=None) -> float:

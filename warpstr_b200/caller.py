@@ -286,10 +286,17 @@ def pack_raw(raws):
 
 def pack_vbz(reads):
     """Chunks of compressed reads (fast5.CompressedRead) -> what ``call_arrays_vbz`` takes: the pinned payload
-    buffer (every chunk's body at a 16-byte aligned offset, zero padded: the decoder reads whole 16-byte
+    buffer (every chunk's payload at a 16-byte aligned offset, zero padded: the decoders read whole 16-byte
     words), the chunk table, the first chunk of every read (int64[n + 1]) and the read offsets in the
-    decoded int16 buffer (int64[n + 1])."""
+    decoded int16 buffer (int64[n + 1]).
+
+    A chunk that is still a zstd frame (fast5.KIND_VBZ*_ZSTD) is uploaded as the frame: its table row has
+    ``zstd_off`` / ``zstd_bytes``, the frame's place in the payload, and ``in_off`` / ``in_bytes`` name where
+    wstr_zstd_decode_batch writes its body, in a region of the device buffer behind the uploaded bytes (the
+    decoded-body region, ``device_bytes`` in all).  Other rows have ``zstd_off`` -1 and are read where they
+    were uploaded, so every StreamVByte body is read from the one device buffer."""
     import torch
+    from .fast5 import KIND_RAW, KIND_VBZ0_ZSTD
     chunks = [c for r in reads for c in r.chunks]
     m = len(chunks)
     n_chunks = np.fromiter((len(r.chunks) for r in reads), dtype=np.int64, count=len(reads))
@@ -297,33 +304,83 @@ def pack_vbz(reads):
     read_chunk[1:] = np.cumsum(n_chunks)
     raw_off = np.zeros(len(reads) + 1, dtype=np.int64)
     raw_off[1:] = np.cumsum(np.fromiter((r.n_samples for r in reads), dtype=np.int64, count=len(reads)))
-    in_bytes = np.fromiter((len(c.payload) for c in chunks), dtype=np.int64, count=m)
-    in_off = np.zeros(m + 1, dtype=np.int64)
-    in_off[1:] = np.cumsum((in_bytes + 15) & ~15)
+    kind = np.fromiter((c.kind for c in chunks), dtype=np.int32, count=m)
+    frame = kind >= KIND_VBZ0_ZSTD
+    up_bytes = np.fromiter((len(c.payload) for c in chunks), dtype=np.int64, count=m)
+    up_off = np.zeros(m + 1, dtype=np.int64)
+    up_off[1:] = np.cumsum((up_bytes + 15) & ~15)
+    body = np.where(frame, np.fromiter((c.body_size for c in chunks), dtype=np.int64, count=m), 0)
+    body_off = np.zeros(m + 1, dtype=np.int64)
+    body_off[1:] = np.cumsum((body + 15) & ~15)
     chunk_read = np.repeat(np.arange(len(reads)), n_chunks)
-    table = dict(in_off=in_off[:-1], in_bytes=in_bytes,
-                 n_samples=np.fromiter((c.coded if c.kind != 2 else c.count for c in chunks), dtype=np.int32, count=m),
+    table = dict(in_off=np.where(frame, int(up_off[-1]) + body_off[:-1], up_off[:-1]),
+                 in_bytes=np.where(frame, body, up_bytes),
+                 n_samples=np.fromiter((c.coded if c.kind != KIND_RAW else c.count for c in chunks), dtype=np.int32,
+                                       count=m),
                  n_out=np.fromiter((c.count for c in chunks), dtype=np.int32, count=m),
-                 kind=np.fromiter((c.kind for c in chunks), dtype=np.int32, count=m),
+                 kind=np.where(frame, kind - KIND_VBZ0_ZSTD, kind).astype(np.int32),
                  zigzag=np.fromiter((c.zigzag for c in chunks), dtype=np.int32, count=m),
-                 out_off=raw_off[chunk_read] + np.fromiter((c.start for c in chunks), dtype=np.int64, count=m))
-    host = torch.zeros(max(int(in_off[-1]), 16), dtype=torch.uint8, pin_memory=torch.cuda.is_available())
+                 out_off=raw_off[chunk_read] + np.fromiter((c.start for c in chunks), dtype=np.int64, count=m),
+                 zstd_off=np.where(frame, up_off[:-1], -1), zstd_bytes=np.where(frame, up_bytes, 0))
+    host = torch.zeros(max(int(up_off[-1]), 16), dtype=torch.uint8, pin_memory=torch.cuda.is_available())
     hb = host.numpy()
-    for c, o in zip(chunks, in_off[:-1]):
+    for c, o in zip(chunks, up_off[:-1]):
         hb[o:o + len(c.payload)] = np.frombuffer(c.payload, dtype=np.uint8)
     return host, table, read_chunk, raw_off
 
 
+def _vbz_layout(table, host_payload):
+    """(upload offsets of the chunks and the end of the last one (int64[m + 1]), bytes the device payload buffer
+    needs) of a ``pack_vbz`` table; a table without zstd frames (built from bodies only) is uploaded as read."""
+    up = np.asarray(table['in_off'], dtype=np.int64)
+    size = np.asarray(table['in_bytes'], dtype=np.int64)
+    need = int(host_payload.numel())
+    if 'zstd_off' in table:
+        zo = np.asarray(table['zstd_off'], dtype=np.int64)
+        if (zo >= 0).any():
+            need = max(need, int((up + ((size + 15) & ~15)).max()))
+            up = np.where(zo >= 0, zo, up)
+            size = np.where(zo >= 0, np.asarray(table['zstd_bytes'], dtype=np.int64), size)
+    m = len(up)
+    return np.append(up, int(up[-1] + ((size[-1] + 15) & ~15)) if m else 0), max(need, 16)
+
+
+def _zstd_frames(table, c0, c1):
+    """Frame numbers [f0, f1) of chunks [c0, c1) (frames are numbered in chunk order) and their table rows."""
+    if 'zstd_off' not in table:
+        return 0, 0, np.zeros(0, dtype=np.int64)
+    is_frame = np.asarray(table['zstd_off'])[:c1] >= 0
+    f0 = int(is_frame[:c0].sum())
+    rows = c0 + np.flatnonzero(is_frame[c0:c1])
+    return f0, f0 + len(rows), rows
+
+
+def _zstd_decode(table, rows, d_payload, d_status, ws):
+    """wstr_zstd_decode_batch of the frames in table rows ``rows``, from and into ``d_payload``."""
+    _lib.zstd_decode_batch(d_payload, table['zstd_off'][rows], table['zstd_bytes'][rows], table['in_off'][rows],
+                           table['in_bytes'][rows], d_payload, d_status, ws)
+
+
+def _chunk_zstd_status(table, frame_status):
+    """Per-chunk WSTR_ZSTD_* status (0 for chunks that were not frames) from the per-frame one."""
+    m = len(table['in_off'])
+    out = np.zeros(m, dtype=np.int32)
+    if 'zstd_off' in table:
+        out[np.asarray(table['zstd_off']) >= 0] = frame_status
+    return out
+
+
 class _IngestVBZ(_IngestRaw):
-    """VBZ chunk bodies (after zstd) of whole reads + windows: the StreamVByte / delta decode
-    (wstr_vbz_decode_batch) writes the int16 reads on the device, which then go on as in _IngestRaw."""
+    """VBZ chunks of whole reads + windows, as ``pack_vbz`` lays them out: zstd frames are decoded on the device
+    (wstr_zstd_decode_batch), then the StreamVByte / delta decode (wstr_vbz_decode_batch) writes the int16
+    reads on the device, which then go on as in _IngestRaw."""
 
     def __init__(self, eng, host_payload, table, read_chunk, raw_off, lo, hi, lengths, spike_mode):
         super().__init__(eng, None, raw_off, lo, hi, lengths, spike_mode)
         self.payload, self.table, self.read_chunk = host_payload, table, read_chunk
-        m = len(table['in_off'])
-        self.pay_off = np.append(table['in_off'], int(table['in_off'][-1] + ((table['in_bytes'][-1] + 15) & ~15))
-                                 if m else 0)[read_chunk]                     # payload bytes of reads [a, b)
+        up, self.device_bytes = _vbz_layout(table, host_payload)
+        self.n_frames = int((np.asarray(table['zstd_off']) >= 0).sum()) if 'zstd_off' in table else 0
+        self.pay_off = up[read_chunk]                                          # uploaded bytes of reads [a, b)
         self.h2d_bytes = int(self.pay_off[-1]) if len(self.pay_off) else 0
 
     def allocate(self):
@@ -331,11 +388,13 @@ class _IngestVBZ(_IngestRaw):
         super().allocate()
         e = self.eng
         m = len(self.table['in_off'])
-        self.d_payload = e._device_buffer('vbz_payload', max(self.h2d_bytes, 16), torch.uint8)
+        self.d_payload = e._device_buffer('vbz_payload', self.device_bytes, torch.uint8)
         self.d_status = e._device_buffer('vbz_status', m, torch.int32)
+        self.d_zstatus = e._device_buffer('zstd_status', max(self.n_frames, 1), torch.int32)
+        pin = torch.cuda.is_available()
         cur = e._host_vbz_status
-        if cur is None or cur.numel() < m:
-            e._host_vbz_status = torch.empty(max(m, 1), dtype=torch.int32, pin_memory=torch.cuda.is_available())
+        if cur is None or cur.numel() < m + self.n_frames:
+            e._host_vbz_status = torch.empty(max(m + self.n_frames, 1), dtype=torch.int32, pin_memory=pin)
 
     def send(self, a, b):
         lo, hi = int(self.pay_off[a]), int(self.pay_off[b])
@@ -344,6 +403,10 @@ class _IngestVBZ(_IngestRaw):
     def prepare(self, a, b, lane):
         import torch
         c0, c1 = int(self.read_chunk[a]), int(self.read_chunk[b])
+        f0, f1, rows = _zstd_frames(self.table, c0, c1)
+        if f1 > f0:
+            ws = self.eng._device_buffer(f'zstd_ws{lane}', _lib.zstd_workspace_bytes(f1 - f0), torch.uint8)
+            _zstd_decode(self.table, rows, self.d_payload, self.d_zstatus[f0:f1], ws)
         if c1 > c0:
             t = {k: v[c0:c1] for k, v in self.table.items()}
             ws = self.eng._device_buffer(f'vbz_ws{lane}', _lib.vbz_workspace_bytes(c1 - c0), torch.uint8)
@@ -355,10 +418,16 @@ class _IngestVBZ(_IngestRaw):
         super().fetch(a, b, out)
         c0, c1 = int(self.read_chunk[a]), int(self.read_chunk[b])
         self.eng._host_vbz_status[c0:c1].copy_(self.d_status[c0:c1], non_blocking=True)
+        f0, f1, _ = _zstd_frames(self.table, c0, c1)
+        if f1 > f0:
+            m = len(self.table['in_off'])
+            self.eng._host_vbz_status[m + f0:m + f1].copy_(self.d_zstatus[f0:f1], non_blocking=True)
 
     def finish(self, res, out, n):
         super().finish(res, out, n)
-        res['chunk_status'] = self.eng._host_vbz_status[:len(self.table['in_off'])].numpy().copy()
+        m = len(self.table['in_off'])
+        res['chunk_status'] = self.eng._host_vbz_status[:m].numpy().copy()
+        res['zstd_status'] = _chunk_zstd_status(self.table, self.eng._host_vbz_status[m:m + self.n_frames].numpy())
 
 
 class CallerEngine:
@@ -675,7 +744,8 @@ class CallerEngine:
         """``call_arrays_raw`` for reads still VBZ-compressed as their fast5 file stores them (``pack_vbz`` makes
         the arguments): only the chunk bodies (after zstd, ~1.25 B per sample instead of 2) cross PCIe, and the
         StreamVByte / zig-zag delta decode (wstr_vbz_decode_batch) writes the int16 reads on the device.  Same
-        result dict, plus ``chunk_status`` (WSTR_VBZ_* per chunk; a read with a bad chunk has undefined results)."""
+        result dict, plus ``chunk_status`` (WSTR_VBZ_* per chunk) and ``zstd_status`` (WSTR_ZSTD_* per chunk, 0
+        for a chunk that was not a zstd frame); a read with a bad chunk has undefined results."""
         from .normalize import SPIKE_MODES
         raw_off = np.asarray(raw_off, dtype=np.int64)
         lo = np.asarray(win_lo, dtype=np.int32)
@@ -916,8 +986,8 @@ class CallerEngine:
             raise ValueError('empty raw read')
         host, table, read_chunk, raw_off = pack_vbz(reads)
         if windows is None:
-            d_raw, chunk_status = self._decode_vbz(host, table, raw_off)
-            _raise_bad_chunk(reads, read_chunk, chunk_status.cpu().numpy())
+            d_raw, chunk_status, zstd_status = self._decode_vbz(host, table, raw_off)
+            _raise_bad_chunk(reads, read_chunk, chunk_status.cpu().numpy(), zstd_status)
             return self._call_located(d_raw, raw_off, aut_ids, reverse, spike_removal, offset,
                                       lambda idx: [reads[r].decode() for r in idx])
         aut = _single_ids(aut_ids)
@@ -927,7 +997,7 @@ class CallerEngine:
         if (lo < 0).any():
             raise ValueError('negative window start')
         res = self.call_arrays_vbz(host, table, read_chunk, raw_off, lo, hi, aut, rev, spike_removal)
-        _raise_bad_chunk(reads, read_chunk, res['chunk_status'])
+        _raise_bad_chunk(reads, read_chunk, res['chunk_status'], res['zstd_status'])
         return self._raw_results(res, lambda idx: [reads[r].decode() for r in idx], windows, aut_ids, reverse,
                                  spike_removal)
 
@@ -988,11 +1058,13 @@ class CallerEngine:
     def locate_arrays_vbz(self, host_payload, table, read_chunk, raw_off, aut, spike_removal: str = 'Brute',
                           offset: float = 0.35) -> Dict[str, np.ndarray]:
         """``locate_arrays_raw`` for VBZ-compressed reads (``pack_vbz``): decoded on the device first.  The dict
-        also carries ``chunk_status`` (WSTR_VBZ_* per chunk; a read with a bad chunk has undefined results)."""
+        also carries ``chunk_status`` (WSTR_VBZ_* per chunk) and ``zstd_status`` (WSTR_ZSTD_* per chunk); a read
+        with a bad chunk has undefined results."""
         raw_off = np.asarray(raw_off, dtype=np.int64)
-        d_raw, chunk_status = self._decode_vbz(host_payload, table, raw_off)
+        d_raw, chunk_status, zstd_status = self._decode_vbz(host_payload, table, raw_off)
         res = self._locate_device(d_raw, raw_off, aut, spike_removal, offset)
         res['chunk_status'] = chunk_status.cpu().numpy()
+        res['zstd_status'] = zstd_status
         return res
 
     def _upload_raw(self, host_raw):
@@ -1003,19 +1075,27 @@ class CallerEngine:
         return d_raw
 
     def _decode_vbz(self, host_payload, table, raw_off):
-        """Payload -> device -> decoded whole int16 reads (device) and the per-chunk status (device)."""
+        """Payload -> device -> decoded whole int16 reads (device), the per-chunk StreamVByte status (device) and
+        the per-chunk zstd status (host)."""
         import torch
         m = len(table['in_off'])
+        _, need = _vbz_layout(table, host_payload)
         with torch.cuda.device(self.device):
-            d_pay = self._device_buffer('vbz_payload', int(host_payload.numel()), torch.uint8)
-            d_pay.copy_(host_payload, non_blocking=True)
+            d_pay = self._device_buffer('vbz_payload', need, torch.uint8)
+            d_pay[:int(host_payload.numel())].copy_(host_payload, non_blocking=True)
             d_raw = self._device_buffer('loc_raw16', int(raw_off[-1]), torch.int16)
             d_st = torch.zeros(max(m, 1), dtype=torch.int32, device=self.device)
+            _, nf, rows = _zstd_frames(table, 0, m)
+            d_zst = torch.zeros(max(nf, 1), dtype=torch.int32, device=self.device)
+            if nf:
+                ws = self._device_buffer('zstd_ws0', _lib.zstd_workspace_bytes(nf), torch.uint8)
+                _zstd_decode(table, rows, d_pay, d_zst, ws)
             if m:
                 ws = self._device_buffer('vbz_ws0', _lib.vbz_workspace_bytes(m), torch.uint8)
                 _lib.vbz_decode_batch(d_pay, table['in_off'], table['in_bytes'], table['n_samples'], table['n_out'],
                                       table['kind'], table['zigzag'], table['out_off'], d_raw, d_st, ws)
-        return d_raw, d_st[:m]
+            zstd_status = _chunk_zstd_status(table, d_zst[:nf].cpu().numpy())
+        return d_raw, d_st[:m], zstd_status
 
     def _locate_device(self, d_raw, raw_off, aut, spike_removal, offset) -> Dict[str, np.ndarray]:
         """Whole-read normalisation of int16 reads on the device, then the window search."""
@@ -1169,14 +1249,17 @@ def _single_ids(aut_ids) -> np.ndarray:
     return ids[:, 0].copy()
 
 
-def _raise_bad_chunk(reads, read_chunk, chunk_status) -> None:
-    """The Fast5FormatError of the first chunk the device decoder refused, naming the file and the read."""
+def _raise_bad_chunk(reads, read_chunk, chunk_status, zstd_status=None) -> None:
+    """The Fast5FormatError of the first chunk the device decoders refused, naming the file and the read: a
+    zstd frame they refuse raises the host decoder's own 'zstd: corrupt VBZ chunk'."""
     from .fast5 import Fast5FormatError
-    bad = np.flatnonzero(chunk_status)
+    zst = np.zeros(len(chunk_status), dtype=np.int32) if zstd_status is None else np.asarray(zstd_status)
+    bad = np.flatnonzero((np.asarray(chunk_status) != 0) | (zst != 0))
     if len(bad):
         c = int(bad[0])
         r = int(np.searchsorted(read_chunk, c, side='right')) - 1
-        msg = _lib.VBZ_STATUS_MESSAGES.get(int(chunk_status[c]), 'VBZ: corrupt chunk')
+        msg = ('zstd: corrupt VBZ chunk' if zst[c] else
+               _lib.VBZ_STATUS_MESSAGES.get(int(chunk_status[c]), 'VBZ: corrupt chunk'))
         raise Fast5FormatError(f'{reads[r].path}: read {reads[r].read_name}: {msg} '
                                f'(chunk at sample {reads[r].chunks[c - int(read_chunk[r])].start})')
 

@@ -174,27 +174,75 @@ def vbz_decompress(chunk: bytes, cd_values: Tuple[int, ...]) -> bytes:
     return vbz_decode_body(body, n, version, int_size, zigzag)
 
 
-# chunk kinds of raw_chunks (the numbering of wstr_vbz_decode_batch)
-KIND_VBZ0, KIND_VBZ1, KIND_RAW = 0, 1, 2
+def zstd_frame_size(frame: bytes, max_size: int) -> int:
+    """Frame_Content_Size of ``frame`` if the device decoder (wstr_zstd_decode_batch) can take it, else -1.
+    Decided from the bytes alone by walking the frame header and the 3-byte block headers: exactly one
+    frame, ending at the payload's end, no dictionary ID, no content checksum, a content size present and
+    at most ``max_size`` (the bound the host decoder uses).  Anything else is decoded on the host."""
+    n = len(frame)
+    if n < 9 or frame[:4] != b'\x28\xb5\x2f\xfd':
+        return -1
+    fhd = frame[4]
+    single, fcs_id = (fhd >> 5) & 1, fhd >> 6
+    if fhd & 0x0F:                                  # reserved bit, content checksum or dictionary ID
+        return -1
+    if not single and (frame[5] >> 3) + 10 > 31:
+        return -1
+    p = 5 + (not single)
+    width = (0, 2, 4, 8)[fcs_id] or (1 if single else 0)
+    if width == 0 or p + width + 3 > n:
+        return -1
+    fcs = int.from_bytes(frame[p:p + width], 'little') + (256 if width == 2 else 0)
+    if fcs > max_size:
+        return -1
+    p += width
+    while True:
+        if p + 3 > n:
+            return -1
+        h = int.from_bytes(frame[p:p + 3], 'little')
+        p += 3
+        btype, size = (h >> 1) & 3, h >> 3
+        if btype == 3 or (btype == 2 and size > 1 << 17):
+            return -1
+        p += 1 if btype == 1 else size
+        if p > n:
+            return -1
+        if h & 1:
+            return fcs if p == n else -1
+
+
+# chunk kinds of stored_chunks / raw_chunks: 0-2 are the numbering of wstr_vbz_decode_batch, and a VBZ chunk
+# whose payload is still its zstd frame (for wstr_zstd_decode_batch, then the StreamVByte decode) is 3 or 4
+KIND_VBZ0, KIND_VBZ1, KIND_RAW, KIND_VBZ0_ZSTD, KIND_VBZ1_ZSTD = 0, 1, 2, 3, 4
 
 
 class RawChunk(NamedTuple):
     """One chunk of a read's signal as the device decoder takes it: samples [start, start + count) of the
     read come from ``payload`` -- a VBZ StreamVByte body after zstd (kind KIND_VBZ0 / KIND_VBZ1, coding
-    ``coded`` >= count samples, zig-zag deltas if ``zigzag``) or ``count`` little-endian int16 (KIND_RAW)."""
+    ``coded`` >= count samples, zig-zag deltas if ``zigzag``), the zstd frame of such a body (KIND_VBZ0_ZSTD /
+    KIND_VBZ1_ZSTD, ``body_size`` its Frame_Content_Size) or ``count`` little-endian int16 (KIND_RAW)."""
     start: int
     count: int
     kind: int
     payload: bytes
     zigzag: bool = False
     coded: int = 0
+    body_size: int = 0
+
+    def unzstd(self) -> 'RawChunk':
+        """The chunk with its zstd frame (if any) undone on the host."""
+        if self.kind < KIND_VBZ0_ZSTD:
+            return self
+        body = zstd_decompress(self.payload, self.coded * 5 + 16)
+        return self._replace(kind=self.kind - KIND_VBZ0_ZSTD, payload=body, body_size=0)
 
     def decode(self) -> np.ndarray:
         """The chunk's int16 samples, decoded on the host (fast5.vbz_decompress)."""
-        if self.kind == KIND_RAW:
-            return np.frombuffer(self.payload, dtype='<i2', count=self.count)
-        raw = vbz_decode_body(self.payload, self.coded, self.kind, 2, int(self.zigzag))
-        return np.frombuffer(raw, dtype='<i2', count=self.count)
+        c = self.unzstd()
+        if c.kind == KIND_RAW:
+            return np.frombuffer(c.payload, dtype='<i2', count=c.count)
+        raw = vbz_decode_body(c.payload, c.coded, c.kind, 2, int(c.zigzag))
+        return np.frombuffer(raw, dtype='<i2', count=c.count)
 
 
 @dataclass
@@ -552,6 +600,15 @@ class H5File:
         or KIND_VBZ1); every other chunk -- other filters, other VBZ integer sizes, contiguous and compact
         layouts -- is decoded here, as ``dataset`` decodes it, and comes back verbatim (KIND_RAW), and so
         do unallocated chunks (zeros, as ``dataset`` leaves them)."""
+        return self._chunks(path, keep_frames=False)
+
+    def stored_chunks(self, path: str) -> Tuple[int, List[RawChunk]]:
+        """``raw_chunks`` with VBZ chunks as the file stores them: a chunk whose zstd frame the device decoder
+        takes (``zstd_frame_size``) comes back as that frame (KIND_VBZ0_ZSTD / KIND_VBZ1_ZSTD); any other zstd
+        frame is undone here."""
+        return self._chunks(path, keep_frames=True)
+
+    def _chunks(self, path: str, keep_frames: bool) -> Tuple[int, List[RawChunk]]:
         obj = self._object(self._resolve(path))
         vbz = None
         if (obj.layout is not None and obj.layout[0] == 'chunked' and obj.shape is not None and len(obj.shape) == 1
@@ -577,10 +634,18 @@ class H5File:
                     raise Fast5FormatError(f'{self.path}: chunk shorter than its extent')
                 found.append(RawChunk(start, take, KIND_RAW, data[:2 * take]))
                 continue
-            coded, body = _vbz_body(data, 2, zstd_level)
+            kind = KIND_VBZ0 if version == 0 else KIND_VBZ1
+            size = -1
+            if keep_frames and zstd_level and len(data) >= 4:
+                coded = struct.unpack_from('<I', data, 0)[0] // 2
+                size = zstd_frame_size(data[4:], coded * 5 + 16)
+            if size >= 0:
+                body, kind = data[4:], kind + KIND_VBZ0_ZSTD
+            else:
+                coded, body = _vbz_body(data, 2, zstd_level)
             if coded < take:
                 raise Fast5FormatError(f'{self.path}: chunk shorter than its extent')
-            found.append(RawChunk(start, take, KIND_VBZ0 if version == 0 else KIND_VBZ1, body, bool(zigzag), coded))
+            found.append(RawChunk(start, take, kind, body, bool(zigzag), coded, max(size, 0)))
         found.sort(key=lambda c: c.start)
         chunks, at = [], 0
         for c in found:
@@ -641,6 +706,16 @@ def raw_chunks(path: str, read_name: Optional[str] = None, h5: Optional[H5File] 
         with H5File(path) as f:
             return raw_chunks(path, read_name, f)
     n, chunks = h5.raw_chunks(_signal_path(h5, read_name))
+    return CompressedRead(path, read_name, n, chunks)
+
+
+def stored_chunks(path: str, read_name: Optional[str] = None, h5: Optional[H5File] = None) -> CompressedRead:
+    """``raw_chunks`` with the zstd frames the device decodes left as the file stores them (see
+    H5File.stored_chunks): the read's chunks cross PCIe as stored and zstd is undone on the GPU too."""
+    if h5 is None:
+        with H5File(path) as f:
+            return stored_chunks(path, read_name, f)
+    n, chunks = h5.stored_chunks(_signal_path(h5, read_name))
     return CompressedRead(path, read_name, n, chunks)
 
 

@@ -184,7 +184,7 @@ class CallerWrapper:
         host, table, read_chunk, raw_off = pack_vbz(reads)
         res = self.engine.locate_arrays_vbz(host, table, read_chunk, raw_off, self._aut(reverse),
                                             spike_removal or self.caller_config.spike_removal, offset)
-        _raise_bad_chunk(reads, read_chunk, res.pop('chunk_status'))
+        _raise_bad_chunk(reads, read_chunk, res.pop('chunk_status'), res.pop('zstd_status'))
         fill_given_strands(res, reverse)
         return res
 
@@ -350,9 +350,10 @@ def _read_source(row, path: str, has_src: bool):
 
 def get_compressed_workload(df_overview, path: str):
     """``get_raw_workload`` without the host's StreamVByte decode: (names, reverse flags, reads as their
-    files store them (fast5.CompressedRead: zstd undone, the rest left to the GPU), windows).  Files are
-    found as ``get_raw_workload`` finds them, and each is opened and parsed once for all its rows."""
-    from .fast5 import H5File, raw_chunks
+    files store them (fast5.CompressedRead from ``fast5.stored_chunks``: zstd frames left for the GPU too,
+    the others undone on the host), windows).  Files are found as ``get_raw_workload`` finds them, and each is
+    opened and parsed once for all its rows."""
+    from .fast5 import H5File, stored_chunks
     names, revs, reads, wins = [], [], [], []
     has_src = 'fast5_path' in df_overview.columns
     rows = [row for row in df_overview.itertuples() if row.saved]
@@ -364,7 +365,7 @@ def get_compressed_workload(df_overview, path: str):
     for fpath, ks in by_file.items():
         with H5File(fpath) as h5:
             for k in ks:
-                reads[k] = raw_chunks(fpath, sources[k][1], h5)
+                reads[k] = stored_chunks(fpath, sources[k][1], h5)
     for row in rows:
         names.append(row.Index)
         revs.append(_strand(row))
@@ -442,8 +443,8 @@ def main_wrapper(locus: Locus, threads: int = 1, config: Optional[Config] = None
     cc = config.caller_config if config is not None else CallerConfig()
     call_wrapper = CallerWrapper(locus, threads, flanks=flanks, config=config, engine=engine)
     if workload is None:
-        # the reads' VBZ chunk bodies (zstd undone on the host) -> StreamVByte decode -> normalisation kernel
-        # -> caller, all on the device
+        # the reads' VBZ chunks as stored -> zstd decode -> StreamVByte decode -> normalisation kernel -> caller,
+        # all on the device
         names, revs, reads, wins = get_compressed_workload(df_overview, locus.path)
         if all(w is not None for w in wins):
             results = call_wrapper.run_compressed(reads, wins, revs, cc.spike_removal)
