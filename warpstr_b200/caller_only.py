@@ -7,6 +7,10 @@ single-read file under ``<output>/<locus>/fast5/<run_id>/annot/`` (h5py) and wri
 overview keeps the ``fast5_path`` column (the reference keeps it too) and
 ``wrapper.get_workload`` reads the signal straight from the multi-read file.
 
+The ``fast5_path`` column keeps the reference's name but may name a POD5 file as well as a multi-read fast5:
+the reader is chosen from each file's first bytes (``fast5.open_raw``), and a POD5 read ID is the UUID that
+fast5 files name the same read by.  So a recent run's ``.pod5`` files are called without converting them.
+
 The STR window columns ``l_start_raw, r_end_raw`` may be left out, or left empty in some rows: the
 caller then finds those reads' windows itself in the whole read (``wrapper.main_wrapper``, DESIGN.md
 section 4.5).  The ``reverse`` column is required but its cells may be empty too: such a read is searched

@@ -608,6 +608,19 @@ class H5File:
         frame is undone here."""
         return self._chunks(path, keep_frames=True)
 
+    # -- reads (the interface fast5.open_raw's readers share with pod5.Pod5File) ------------------------------
+    def read_names(self) -> List[str]:
+        """Read ids of a multi-read fast5 (group names ``read_<id>``)."""
+        return [k[5:] for k in self.keys('/') if k.startswith('read_')]
+
+    def read_signal(self, read_name: Optional[str]) -> np.ndarray:
+        return _raw_signal(self, read_name)
+
+    def read_chunks(self, read_name: Optional[str], keep_frames: bool) -> 'CompressedRead':
+        """The read's signal dataset as ``stored_chunks`` (``keep_frames``) or ``raw_chunks`` returns it."""
+        n, chunks = self._chunks(_signal_path(self, read_name), keep_frames)
+        return CompressedRead(self.path, read_name, n, chunks)
+
     def _chunks(self, path: str, keep_frames: bool) -> Tuple[int, List[RawChunk]]:
         obj = self._object(self._resolve(path))
         vbz = None
@@ -661,19 +674,35 @@ class H5File:
 
 
 # ---------------------------------------------------------------------------------------------------
-# fast5
+# fast5 and POD5: one entry point per question, the container chosen from the file's first bytes
 # ---------------------------------------------------------------------------------------------------
+HDF5_SIGNATURE = b'\x89HDF\r\n\x1a\n'
+POD5_SIGNATURE = b'\x8bPOD\r\n\x1a\n'
+
+
+def open_raw(path: str):
+    """The raw-signal file at ``path``, opened with the reader its first 8 bytes name: an ``H5File`` for fast5
+    (HDF5), a ``pod5.Pod5File`` for POD5.  Both answer ``read_names()``, ``read_signal(read_name)`` and
+    ``read_chunks(read_name, keep_frames)`` and are context managers, so no caller looks at the file type."""
+    with open(path, 'rb') as fh:
+        head = fh.read(8)
+    if head == POD5_SIGNATURE:
+        from . import pod5
+        return pod5.Pod5File(path)
+    return H5File(path)                 # HDF5; anything else gets H5File's own 'not an HDF5 file' or 'empty file'
+
+
 def read_names(path: str) -> List[str]:
-    """Read ids of a multi-read fast5 (group names ``read_<id>``)."""
-    with H5File(path) as h5:
-        return [k[5:] for k in h5.keys('/') if k.startswith('read_')]
+    """Read ids of a multi-read fast5 (group names ``read_<id>``) or of a POD5 file."""
+    with open_raw(path) as f:
+        return f.read_names()
 
 
 def raw_signal(path: str, read_name: Optional[str] = None) -> np.ndarray:
     """The raw int16 DAC samples of one read.  ``read_name`` selects a read of a multi-read
-    file; a single-read file (``Raw/Reads/Read_<n>``) has only one."""
-    with H5File(path) as h5:
-        return _raw_signal(h5, read_name)
+    fast5 or a POD5 file; a single-read file (``Raw/Reads/Read_<n>``) has only one."""
+    with open_raw(path) as f:
+        return f.read_signal(read_name)
 
 
 def _raw_signal(h5: H5File, read_name: Optional[str]) -> np.ndarray:
@@ -698,25 +727,24 @@ def _signal_path(h5: H5File, read_name: Optional[str]) -> str:
     raise KeyError(f'read {read_name} not found in {h5.path}')
 
 
-def raw_chunks(path: str, read_name: Optional[str] = None, h5: Optional[H5File] = None) -> CompressedRead:
+def raw_chunks(path: str, read_name: Optional[str] = None, h5=None) -> CompressedRead:
     """One read's signal as its file stores it, for the device decoder (CallerEngine.call_vbz_batch):
     the read is chosen exactly as ``raw_signal`` chooses it, zstd is undone here and the StreamVByte
-    decode is left to the GPU (see H5File.raw_chunks).  ``h5``: the file, already open."""
+    decode is left to the GPU (see H5File.raw_chunks; a POD5 signal row is one chunk, see pod5.py).
+    ``h5``: the file, already open (``open_raw``)."""
     if h5 is None:
-        with H5File(path) as f:
-            return raw_chunks(path, read_name, f)
-    n, chunks = h5.raw_chunks(_signal_path(h5, read_name))
-    return CompressedRead(path, read_name, n, chunks)
+        with open_raw(path) as f:
+            return f.read_chunks(read_name, False)
+    return h5.read_chunks(read_name, False)
 
 
-def stored_chunks(path: str, read_name: Optional[str] = None, h5: Optional[H5File] = None) -> CompressedRead:
+def stored_chunks(path: str, read_name: Optional[str] = None, h5=None) -> CompressedRead:
     """``raw_chunks`` with the zstd frames the device decodes left as the file stores them (see
     H5File.stored_chunks): the read's chunks cross PCIe as stored and zstd is undone on the GPU too."""
     if h5 is None:
-        with H5File(path) as f:
-            return stored_chunks(path, read_name, f)
-    n, chunks = h5.stored_chunks(_signal_path(h5, read_name))
-    return CompressedRead(path, read_name, n, chunks)
+        with open_raw(path) as f:
+            return f.read_chunks(read_name, True)
+    return h5.read_chunks(read_name, True)
 
 
 class Fast5:

@@ -284,7 +284,8 @@ def get_raw_workload(df_overview, path: str):
     The raw signal of every saved read comes from its annotated single-read fast5
     (``<locus>/fast5/<run_id>/annot/<read>.fast5``, what the reference's extraction step
     writes) or, for a caller-only run prepared straight from a sequencing run's multi-read
-    files, from the file named in the row's ``fast5_path`` column (see caller_only.py)."""
+    files, from the file named in the row's ``fast5_path`` column, a multi-read fast5 or a POD5 file (see
+    caller_only.py)."""
     from .fast5 import raw_signal
     names, revs, raws, wins = [], [], [], []
     has_src = 'fast5_path' in df_overview.columns
@@ -339,7 +340,7 @@ def _window(row):
 
 def _read_source(row, path: str, has_src: bool):
     """(file, read name or None) a saved overview row's signal comes from: its annotated single-read fast5,
-    else the multi-read file of the row's ``fast5_path``."""
+    else the multi-read fast5 or POD5 file of the row's ``fast5_path``."""
     fpath = os.path.join(path, tmpl.FAST5_SUBDIR, str(row.run_id), tmpl.ANNOT_SUBDIR, row.Index + '.fast5')
     if os.path.exists(fpath):
         return fpath, None
@@ -352,8 +353,8 @@ def get_compressed_workload(df_overview, path: str):
     """``get_raw_workload`` without the host's StreamVByte decode: (names, reverse flags, reads as their
     files store them (fast5.CompressedRead from ``fast5.stored_chunks``: zstd frames left for the GPU too,
     the others undone on the host), windows).  Files are found as ``get_raw_workload`` finds them, and each is
-    opened and parsed once for all its rows."""
-    from .fast5 import H5File, stored_chunks
+    opened and parsed once for all its rows, fast5 or POD5 alike (``fast5.open_raw``)."""
+    from .fast5 import open_raw, stored_chunks
     names, revs, reads, wins = [], [], [], []
     has_src = 'fast5_path' in df_overview.columns
     rows = [row for row in df_overview.itertuples() if row.saved]
@@ -363,9 +364,9 @@ def get_compressed_workload(df_overview, path: str):
         by_file.setdefault(fpath, []).append(k)
     reads = [None] * len(rows)
     for fpath, ks in by_file.items():
-        with H5File(fpath) as h5:
+        with open_raw(fpath) as f:
             for k in ks:
-                reads[k] = stored_chunks(fpath, sources[k][1], h5)
+                reads[k] = stored_chunks(fpath, sources[k][1], f)
     for row in rows:
         names.append(row.Index)
         revs.append(_strand(row))
