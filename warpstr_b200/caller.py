@@ -108,11 +108,7 @@ def pack_signals(signals: Sequence[np.ndarray]):
     import torch
     n = len(signals)
     lengths = np.fromiter((len(s) for s in signals), dtype=np.int32, count=n)
-    padded = (lengths.astype(np.int64) + 1) & ~1
-    offsets = np.zeros(n, dtype=np.int64)
-    if n > 1:
-        offsets[1:] = np.cumsum(padded[:-1])
-    total = int(padded.sum()) + 2
+    offsets, total = even_offsets(lengths)
     host = torch.empty(total, dtype=torch.float64, pin_memory=torch.cuda.is_available())
     buf = host.numpy()
     for s, o, ln in zip(signals, offsets, lengths):
@@ -150,32 +146,46 @@ def even_offsets(lengths: np.ndarray):
     return off, int(padded.sum()) + 2
 
 
+def _span(off, lengths, a, b, size):
+    """Element range [lo, hi) of reads [a, b) (b > a) in a float64 buffer of ``size`` elements packed as
+    ``even_offsets`` packs them: up to 2 elements past the last read's even end (the kernels read that far),
+    clipped at the buffer's end."""
+    return int(off[a]), min(int(off[b - 1] + ((int(lengths[b - 1]) + 1) & ~1) + 2), size)
+
+
+def _window_bounds(raw_off, win_lo, win_hi):
+    """(lo int32[n], hi int32[n], lengths int32[n]) of the windows ``[win_lo, win_hi]`` (inclusive) of whole
+    reads at offsets ``raw_off`` (int64[n + 1]): a window is clipped at its read's end like a numpy slice; a
+    negative start raises ValueError."""
+    lo = np.asarray(win_lo, dtype=np.int32)
+    hi = np.asarray(win_hi, dtype=np.int32)
+    if (lo < 0).any():
+        raise ValueError('negative window start')
+    lengths = np.maximum(np.minimum(hi.astype(np.int64), np.diff(raw_off) - 1) - lo + 1, 0).astype(np.int32)
+    return lo, hi, lengths
+
+
+def _nothing(self, *args):
+    """The hook of an ingest form or whole-read source that has nothing to do at that step."""
+
+
 class _IngestF64:
     """Host float64 windows (the reference's ReadSignal.signal): copied as they are."""
 
     def __init__(self, eng, host_signal, off, lengths):
         self.eng, self.host, self.sig_off, self.lengths = eng, host_signal, off, lengths
-        n = len(lengths)
-        self.total = int(off[-1] + ((int(lengths[-1]) + 1) & ~1) + 2) if n else 0
-        self.h2d_bytes = min(self.total, host_signal.numel()) * 8
+        self.total = _span(off, lengths, 0, len(lengths), host_signal.numel())[1] if len(lengths) else 0
+        self.h2d_bytes = self.total * 8
 
     def allocate(self):
         import torch
-        self.d_sig = self.eng._device_buffer('sig', min(self.total, self.host.numel()), torch.float64)
+        self.d_sig = self.eng._device_buffer('sig', self.total, torch.float64)
 
     def send(self, a, b):
-        lo = int(self.sig_off[a])
-        hi = min(int(self.sig_off[b - 1] + ((int(self.lengths[b - 1]) + 1) & ~1) + 2), self.d_sig.numel())
+        lo, hi = _span(self.sig_off, self.lengths, a, b, self.d_sig.numel())
         self.d_sig[lo:hi].copy_(self.host[lo:hi], non_blocking=True)
 
-    def prepare(self, a, b, lane):
-        pass
-
-    def fetch(self, a, b, out):
-        pass
-
-    def finish(self, res, out, n):
-        pass
+    prepare = fetch = finish = _nothing
 
 
 class _IngestI16:
@@ -207,65 +217,7 @@ class _IngestI16:
         _lib.dequantize_batch(self.d_raw, self.raw_off[a:b], self.lengths[a:b], self.d_ss[2 * a:2 * b], self.d_sig,
                               self.sig_off[a:b], ws)
 
-    def fetch(self, a, b, out):
-        pass
-
-    def finish(self, res, out, n):
-        pass
-
-
-class _IngestRaw:
-    """Host int16 whole reads + windows; spike removal, MAD normalisation and slicing on the device."""
-
-    def __init__(self, eng, host_raw, raw_off, lo, hi, lengths, spike_mode):
-        self.eng, self.host, self.raw_off, self.lo, self.hi = eng, host_raw, raw_off, lo, hi
-        self.lengths, self.spike_mode = lengths, spike_mode
-        self.sig_off, self.total = even_offsets(lengths)
-        self.h2d_bytes = int(raw_off[-1]) * 2 if len(raw_off) else 0
-        self.d_raw = None
-
-    def allocate(self):
-        import torch
-        e = self.eng
-        self.d_sig = e._device_buffer('sig', self.total, torch.float64)
-        if self.d_raw is None:
-            self.d_raw = e._device_buffer('raw16', int(self.raw_off[-1]), torch.int16)
-        self.d_ss = e._device_buffer('shift_scale', 2 * len(self.lengths), torch.float64)
-        pin = torch.cuda.is_available()
-        cur = e._host_ss
-        if cur is None or cur.numel() < 2 * len(self.lengths):
-            e._host_ss = torch.empty(max(2 * len(self.lengths), 2), dtype=torch.float64, pin_memory=pin)
-
-    def send(self, a, b):
-        lo, hi = int(self.raw_off[a]), int(self.raw_off[b])
-        self.d_raw[lo:hi].copy_(self.host[lo:hi], non_blocking=True)
-
-    def prepare(self, a, b, lane):
-        import torch
-        n = b - a
-        ws = self.eng._device_buffer(f'norm_ws{lane}', _lib.normalize_workspace_bytes(n), torch.uint8)
-        _lib.normalize_batch(self.d_raw, self.raw_off[a:b + 1], self.lo[a:b], self.hi[a:b], self.spike_mode,
-                             self.d_sig, self.sig_off[a:b], self.d_ss[2 * a:2 * b], ws)
-
-    def fetch(self, a, b, out):
-        self.eng._host_ss[2 * a:2 * b].copy_(self.d_ss[2 * a:2 * b], non_blocking=True)
-
-    def finish(self, res, out, n):
-        res['shift_scale'] = self.eng._host_ss[:2 * n].numpy().reshape(n, 2).copy()
-        res['lengths'] = self.lengths
-
-
-class _IngestDeviceRaw(_IngestRaw):
-    """Whole int16 reads that are already on the device (the located-then-called chain): nothing crosses
-    PCIe, the windows are normalised and called as in _IngestRaw."""
-
-    def __init__(self, eng, d_raw, raw_off, lo, hi, lengths, spike_mode):
-        super().__init__(eng, None, raw_off, lo, hi, lengths, spike_mode)
-        self.d_raw = d_raw
-        self.h2d_bytes = 0
-
-    def send(self, a, b):
-        pass
+    fetch = finish = _nothing
 
 
 def pack_raw(raws):
@@ -329,105 +281,149 @@ def pack_vbz(reads):
     return host, table, read_chunk, raw_off
 
 
-def _vbz_layout(table, host_payload):
-    """(upload offsets of the chunks and the end of the last one (int64[m + 1]), bytes the device payload buffer
-    needs) of a ``pack_vbz`` table; a table without zstd frames (built from bodies only) is uploaded as read."""
-    up = np.asarray(table['in_off'], dtype=np.int64)
-    size = np.asarray(table['in_bytes'], dtype=np.int64)
-    need = int(host_payload.numel())
-    if 'zstd_off' in table:
-        zo = np.asarray(table['zstd_off'], dtype=np.int64)
-        if (zo >= 0).any():
-            need = max(need, int((up + ((size + 15) & ~15)).max()))
-            up = np.where(zo >= 0, zo, up)
-            size = np.where(zo >= 0, np.asarray(table['zstd_bytes'], dtype=np.int64), size)
-    m = len(up)
-    return np.append(up, int(up[-1] + ((size[-1] + 15) & ~15)) if m else 0), max(need, 16)
+class _WholeReads:
+    """Whole int16 reads in a pinned host buffer as ``pack_raw`` lays them out, or already on the device (``d_raw``,
+    nothing to send).  ``samples(idx)``: the host samples of reads ``idx``, for the host redo.  ``_VBZReads`` is the
+    other form; both allocate, send and decode reads [a, b) on the current stream, fetch the decode statuses, put
+    them into a result (``finish``) and raise the first bad chunk's error from it (``raise_bad``)."""
 
+    def __init__(self, host, raw_off, d_raw=None, samples=None):
+        self.host, self.d_raw, self.samples = host, d_raw, samples
+        self.raw_off = np.asarray(raw_off, dtype=np.int64)
+        self.h2d_bytes = int(self.raw_off[-1]) * 2 if host is not None else 0
 
-def _zstd_frames(table, c0, c1):
-    """Frame numbers [f0, f1) of chunks [c0, c1) (frames are numbered in chunk order) and their table rows."""
-    if 'zstd_off' not in table:
-        return 0, 0, np.zeros(0, dtype=np.int64)
-    is_frame = np.asarray(table['zstd_off'])[:c1] >= 0
-    f0 = int(is_frame[:c0].sum())
-    rows = c0 + np.flatnonzero(is_frame[c0:c1])
-    return f0, f0 + len(rows), rows
-
-
-def _zstd_decode(table, rows, d_payload, d_status, ws):
-    """wstr_zstd_decode_batch of the frames in table rows ``rows``, from and into ``d_payload``."""
-    _lib.zstd_decode_batch(d_payload, table['zstd_off'][rows], table['zstd_bytes'][rows], table['in_off'][rows],
-                           table['in_bytes'][rows], d_payload, d_status, ws)
-
-
-def _chunk_zstd_status(table, frame_status):
-    """Per-chunk WSTR_ZSTD_* status (0 for chunks that were not frames) from the per-frame one."""
-    m = len(table['in_off'])
-    out = np.zeros(m, dtype=np.int32)
-    if 'zstd_off' in table:
-        out[np.asarray(table['zstd_off']) >= 0] = frame_status
-    return out
-
-
-class _IngestVBZ(_IngestRaw):
-    """VBZ chunks of whole reads + windows, as ``pack_vbz`` lays them out: zstd frames are decoded on the device
-    (wstr_zstd_decode_batch), then the StreamVByte / delta decode (wstr_vbz_decode_batch) writes the int16
-    reads on the device, which then go on as in _IngestRaw."""
-
-    def __init__(self, eng, host_payload, table, read_chunk, raw_off, lo, hi, lengths, spike_mode):
-        super().__init__(eng, None, raw_off, lo, hi, lengths, spike_mode)
-        self.payload, self.table, self.read_chunk = host_payload, table, read_chunk
-        up, self.device_bytes = _vbz_layout(table, host_payload)
-        self.n_frames = int((np.asarray(table['zstd_off']) >= 0).sum()) if 'zstd_off' in table else 0
-        self.pay_off = up[read_chunk]                                          # uploaded bytes of reads [a, b)
-        self.h2d_bytes = int(self.pay_off[-1]) if len(self.pay_off) else 0
-
-    def allocate(self):
+    def allocate(self, eng, name):
         import torch
-        super().allocate()
-        e = self.eng
-        m = len(self.table['in_off'])
-        self.d_payload = e._device_buffer('vbz_payload', self.device_bytes, torch.uint8)
-        self.d_status = e._device_buffer('vbz_status', m, torch.int32)
-        self.d_zstatus = e._device_buffer('zstd_status', max(self.n_frames, 1), torch.int32)
-        pin = torch.cuda.is_available()
-        cur = e._host_vbz_status
-        if cur is None or cur.numel() < m + self.n_frames:
-            e._host_vbz_status = torch.empty(max(m + self.n_frames, 1), dtype=torch.int32, pin_memory=pin)
+        if self.host is not None:
+            self.d_raw = eng._device_buffer(name, int(self.raw_off[-1]), torch.int16)
+
+    def send(self, a, b):
+        if self.host is not None:
+            lo, hi = int(self.raw_off[a]), int(self.raw_off[b])
+            self.d_raw[lo:hi].copy_(self.host[lo:hi], non_blocking=True)
+
+    decode = fetch = finish = raise_bad = _nothing     # int16 reads need no decode and have no statuses
+
+
+class _VBZReads(_WholeReads):
+    """Whole reads as VBZ chunks, as ``pack_vbz`` lays them out: the payload crosses the host link as stored,
+    zstd frames are decoded on the device (wstr_zstd_decode_batch), then the StreamVByte / delta decode
+    (wstr_vbz_decode_batch) writes the int16 reads.  The statuses: WSTR_VBZ_* per chunk and WSTR_ZSTD_* per
+    frame, frames numbered in chunk order, in one pinned buffer laid out [chunks | frames]."""
+
+    def __init__(self, host_payload, table, read_chunk, raw_off, reads=None):
+        super().__init__(None, raw_off, samples=lambda idx: [reads[r].decode() for r in idx])
+        self.payload, self.table, self.reads = host_payload, table, reads
+        self.read_chunk = np.asarray(read_chunk, dtype=np.int64)
+        frame = np.asarray(table['zstd_off']) >= 0
+        self.frame_rows = np.flatnonzero(frame)                  # table rows of the zstd frames
+        self.frame_of = np.zeros(len(frame) + 1, dtype=np.int64)  # frames before chunk c
+        self.frame_of[1:] = np.cumsum(frame)
+        # the chunks are uploaded one after the other at 16-byte aligned offsets: a frame at zstd_off (its body is
+        # decoded to in_off, behind the uploaded bytes), any other chunk at in_off
+        in_end = table['in_off'] + ((table['in_bytes'] + 15) & ~15)
+        up_end = np.where(frame, table['zstd_off'] + ((table['zstd_bytes'] + 15) & ~15), in_end)
+        self.pay_off = np.append(0, up_end)[self.read_chunk]   # uploaded bytes of reads [a, b)
+        self.h2d_bytes = int(self.pay_off[-1])
+        self.device_bytes = max(int(host_payload.numel()), int(in_end.max()) if len(in_end) else 0, 16)
+
+    def allocate(self, eng, name):
+        import torch
+        m, nf = len(self.frame_of) - 1, len(self.frame_rows)
+        self.d_raw = eng._device_buffer(name, int(self.raw_off[-1]), torch.int16)
+        self.d_payload = eng._device_buffer('vbz_payload', self.device_bytes, torch.uint8)
+        self.d_status = eng._device_buffer('vbz_status', m, torch.int32)
+        self.d_zstatus = eng._device_buffer('zstd_status', max(nf, 1), torch.int32)
+        self.h_status = eng._host_buffer('vbz_status', m + nf, torch.int32)
 
     def send(self, a, b):
         lo, hi = int(self.pay_off[a]), int(self.pay_off[b])
         self.d_payload[lo:hi].copy_(self.payload[lo:hi], non_blocking=True)
 
-    def prepare(self, a, b, lane):
-        import torch
+    def _ranges(self, a, b):
+        """Chunks [c0, c1) and frames [f0, f1) of reads [a, b)."""
         c0, c1 = int(self.read_chunk[a]), int(self.read_chunk[b])
-        f0, f1, rows = _zstd_frames(self.table, c0, c1)
+        return c0, c1, int(self.frame_of[c0]), int(self.frame_of[c1])
+
+    def decode(self, eng, a, b, lane):
+        import torch
+        c0, c1, f0, f1 = self._ranges(a, b)
         if f1 > f0:
-            ws = self.eng._device_buffer(f'zstd_ws{lane}', _lib.zstd_workspace_bytes(f1 - f0), torch.uint8)
-            _zstd_decode(self.table, rows, self.d_payload, self.d_zstatus[f0:f1], ws)
+            rows, t = self.frame_rows[f0:f1], self.table
+            ws = eng._device_buffer(f'zstd_ws{lane}', _lib.zstd_workspace_bytes(f1 - f0), torch.uint8)
+            _lib.zstd_decode_batch(self.d_payload, t['zstd_off'][rows], t['zstd_bytes'][rows], t['in_off'][rows],
+                                   t['in_bytes'][rows], self.d_payload, self.d_zstatus[f0:f1], ws)
         if c1 > c0:
             t = {k: v[c0:c1] for k, v in self.table.items()}
-            ws = self.eng._device_buffer(f'vbz_ws{lane}', _lib.vbz_workspace_bytes(c1 - c0), torch.uint8)
+            ws = eng._device_buffer(f'vbz_ws{lane}', _lib.vbz_workspace_bytes(c1 - c0), torch.uint8)
             _lib.vbz_decode_batch(self.d_payload, t['in_off'], t['in_bytes'], t['n_samples'], t['n_out'], t['kind'],
                                   t['zigzag'], t['out_off'], self.d_raw, self.d_status[c0:c1], ws)
-        super().prepare(a, b, lane)
 
-    def fetch(self, a, b, out):
-        super().fetch(a, b, out)
-        c0, c1 = int(self.read_chunk[a]), int(self.read_chunk[b])
-        self.eng._host_vbz_status[c0:c1].copy_(self.d_status[c0:c1], non_blocking=True)
-        f0, f1, _ = _zstd_frames(self.table, c0, c1)
+    def fetch(self, a, b):
+        c0, c1, f0, f1 = self._ranges(a, b)
+        m = len(self.frame_of) - 1
+        self.h_status[c0:c1].copy_(self.d_status[c0:c1], non_blocking=True)
         if f1 > f0:
-            m = len(self.table['in_off'])
-            self.eng._host_vbz_status[m + f0:m + f1].copy_(self.d_zstatus[f0:f1], non_blocking=True)
+            self.h_status[m + f0:m + f1].copy_(self.d_zstatus[f0:f1], non_blocking=True)
 
-    def finish(self, res, out, n):
-        super().finish(res, out, n)
-        m = len(self.table['in_off'])
-        res['chunk_status'] = self.eng._host_vbz_status[:m].numpy().copy()
-        res['zstd_status'] = _chunk_zstd_status(self.table, self.eng._host_vbz_status[m:m + self.n_frames].numpy())
+    def finish(self, res):
+        """``chunk_status`` and ``zstd_status`` (per chunk, 0 for a chunk that was not a zstd frame) into ``res``;
+        the fetches must have completed."""
+        m = len(self.frame_of) - 1
+        h = self.h_status.numpy()
+        res['chunk_status'], res['zstd_status'] = h[:m].copy(), np.zeros(m, dtype=np.int32)
+        res['zstd_status'][self.frame_rows] = h[m:]
+
+    def raise_bad(self, res):
+        """Takes the statuses out of ``res`` and raises the Fast5FormatError of the first chunk the device decoders
+        refused, naming the file and the read: a zstd frame they refuse raises the host decoder's own 'zstd:
+        corrupt VBZ chunk'."""
+        from .fast5 import Fast5FormatError
+        chunk_status, zst = res.pop('chunk_status'), res.pop('zstd_status')
+        bad = np.flatnonzero((chunk_status != 0) | (zst != 0))
+        if len(bad):
+            c = int(bad[0])
+            r = int(np.searchsorted(self.read_chunk, c, side='right')) - 1
+            read = self.reads[r]
+            msg = ('zstd: corrupt VBZ chunk' if zst[c] else
+                   _lib.VBZ_STATUS_MESSAGES.get(int(chunk_status[c]), 'VBZ: corrupt chunk'))
+            raise Fast5FormatError(f'{read.path}: read {read.read_name}: {msg} '
+                                   f'(chunk at sample {read.chunks[c - int(self.read_chunk[r])].start})')
+
+
+class _IngestRaw:
+    """Whole int16 reads (a ``_WholeReads``) + windows: the source's decode, then spike removal, MAD
+    normalisation and slicing on the device."""
+
+    def __init__(self, eng, src, lo, hi, lengths, spike_mode):
+        self.eng, self.src, self.lo, self.hi = eng, src, lo, hi
+        self.lengths, self.spike_mode = lengths, spike_mode
+        self.sig_off, self.total = even_offsets(lengths)
+        self.h2d_bytes, self.send = src.h2d_bytes, src.send
+
+    def allocate(self):
+        import torch
+        e, n = self.eng, len(self.lengths)
+        self.d_sig = e._device_buffer('sig', self.total, torch.float64)
+        self.src.allocate(e, 'raw16')
+        self.d_ss = e._device_buffer('shift_scale', 2 * n, torch.float64)
+        self.h_ss = e._host_buffer('shift_scale', 2 * n, torch.float64)
+
+    def prepare(self, a, b, lane):
+        import torch
+        self.src.decode(self.eng, a, b, lane)
+        ws = self.eng._device_buffer(f'norm_ws{lane}', _lib.normalize_workspace_bytes(b - a), torch.uint8)
+        _lib.normalize_batch(self.src.d_raw, self.src.raw_off[a:b + 1], self.lo[a:b], self.hi[a:b], self.spike_mode,
+                             self.d_sig, self.sig_off[a:b], self.d_ss[2 * a:2 * b], ws)
+
+    def fetch(self, a, b):
+        self.h_ss[2 * a:2 * b].copy_(self.d_ss[2 * a:2 * b], non_blocking=True)
+        self.src.fetch(a, b)
+
+    def finish(self, res):
+        res['shift_scale'] = self.h_ss.numpy().reshape(-1, 2).copy()
+        res['lengths'] = self.lengths
+        self.src.finish(res)
 
 
 class CallerEngine:
@@ -446,17 +442,11 @@ class CallerEngine:
         self.workspace_limit = workspace_bytes
         self.automata: List[_lib.DeviceAutomaton] = []
         self.tables: List[dict] = []
-        self._ws = None
-        self._ws_at_limit = False
-        self._ws_need_seen = 0
         self._lane_ws = {}
-        self._lane_streams = None
-        self._copy_stream = None
+        self._streams = {}
         self.timeline = None      # set to a list to collect (label, CUDA event) pairs from call_arrays
-        self._host_out = None
-        self._host_ss = None
-        self._host_vbz_status = None
         self._dev_cache = {}
+        self._host_cache = {}
         self._h2d_probe = None
         self.split_small = (4096, 40000)   # batch sizes a resident call runs as two concurrent halves (None: never)
         self.ttest_guard_ulps = 0    # 0 = the library's default (16 ulp), see wstr_call_outputs.d_ttest_ties
@@ -479,44 +469,24 @@ class CallerEngine:
 
     # -- device helpers ---------------------------------------------------------------------
     def _workspace(self, need: int, lane: int = 0):
-        if lane:
-            # extra compute lanes of the pipelined call own a workspace each (sized for their chunks), under
-            # the same limits as the first: the explicit one, else 60 % of what is free when it has to grow
-            ws = self._lane_ws.get(lane)
-            if ws is None or ws.numel() < need:
-                import torch
-                have = ws.numel() if ws is not None else 0
-                limit = self.workspace_limit
-                if limit is None:
-                    free, _ = torch.cuda.mem_get_info(self.device)
-                    limit = int(free * 0.6) + have
-                size = min(need, max(limit, 1 << 20))
-                if size > have:
-                    self._lane_ws[lane] = None
-                    ws = torch.empty(size, dtype=torch.uint8, device=self.device)
-                    self._lane_ws[lane] = ws
-            return ws
-        return self._workspace0(need)
-
-    def _workspace0(self, need: int):
-        """Device workspace of ``need`` bytes, or as much as the memory limit allows (the library
-        then works in waves).  The buffer only grows; cudaMemGetInfo is asked only when it has
-        to (the call can block for tens of milliseconds while the GPU is busy)."""
+        """Device workspace of ``need`` bytes for compute lane ``lane`` (each lane of the pipelined call owns
+        one, sized for its chunks), or as much as the memory limit allows (the library then works in waves):
+        the explicit limit, else 60 % of what is free.  The buffer only grows; cudaMemGetInfo is asked only
+        when it has to (the call can block for tens of milliseconds while the GPU is busy)."""
         import torch
-        ws = self._ws
-        if ws is not None and (ws.numel() >= need or (self._ws_at_limit and need <= self._ws_need_seen)):
+        ws, at_limit, need_seen = self._lane_ws.get(lane, (None, False, 0))
+        if ws is not None and (ws.numel() >= need or (at_limit and need <= need_seen)):
             return ws
-        self._ws_need_seen = need        # a larger request re-evaluates the limit (memory may have been freed)
         limit = self.workspace_limit
         if limit is None:
             free, _ = torch.cuda.mem_get_info(self.device)
             limit = int(free * 0.6) + (ws.numel() if ws is not None else 0)
         size = min(need, max(limit, 1 << 20))
-        self._ws_at_limit = size < need
         if ws is None or ws.numel() < size:
-            self._ws = None
-            self._ws = torch.empty(size, dtype=torch.uint8, device=self.device)
-        return self._ws
+            ws = torch.empty(size, dtype=torch.uint8, device=self.device)
+        # a larger request re-evaluates the limit (memory may have been freed)
+        self._lane_ws[lane] = (ws, size < need, need)
+        return ws
 
     def warp_batch(self, signals: Sequence[np.ndarray], aut_ids: Sequence[int],
                    masks: Optional[Sequence[np.ndarray]] = None, return_end_cost: bool = False):
@@ -629,8 +599,7 @@ class CallerEngine:
                                      1 if self.rc.method == 'median' else 0, 1 if self.rc.reps_as_one else 0,
                                      int(self.ttest_guard_ulps))
             def run(a, b, wsp, stream):
-                lo = int(off[a])
-                hi = min(int(off[b - 1] + ((int(lengths[b - 1]) + 1) & ~1) + 2), d_sig.numel()) if b > a else lo
+                lo, hi = _span(off, lengths, a, b, d_sig.numel())
                 sl = slice(lo, hi)
 
                 def part(key, x0, x1):
@@ -664,12 +633,18 @@ class CallerEngine:
 
     def _halves(self, n: int, lane: int):
         """(split point, side stream) when a resident call should run as two concurrent halves."""
-        import torch
         if lane != 0 or not self.split_small or not (self.split_small[0] <= n <= self.split_small[1]):
             return None
-        if self._lane_streams is None:
-            self._lane_streams = [torch.cuda.Stream() for _ in range(3)]
-        return n // 2, self._lane_streams[0]
+        return n // 2, self._side_streams('lanes')[0]
+
+    def _side_streams(self, group: str):
+        """The engine's side streams: 'lanes', three compute lanes beside the current stream, or 'copy', the
+        pipeline's input and result streams.  Each group is taken from torch's stream pool when a call first needs
+        it (the pool index decides which hardware queue a stream shares)."""
+        import torch
+        if group not in self._streams:
+            self._streams[group] = [torch.cuda.Stream() for _ in range(3 if group == 'lanes' else 2)]
+        return self._streams[group]
 
     def _slices(self, ws_bytes: int, need: int, aut, lengths):
         """Consecutive read ranges of one call_packed: the whole batch when the workspace holds what a call
@@ -729,14 +704,8 @@ class CallerEngine:
         whole int16 reads ``host_raw[raw_off[r] : raw_off[r+1]]`` and their windows ``[win_lo, win_hi]`` go to
         the device, are spike-filtered, MAD-normalised and sliced there (wstr_normalize_batch) and called
         without the float64 windows ever visiting the host.  The result also carries ``shift_scale``."""
-        from .normalize import SPIKE_MODES
-        raw_off = np.asarray(raw_off, dtype=np.int64)
-        lo = np.asarray(win_lo, dtype=np.int32)
-        hi = np.asarray(win_hi, dtype=np.int32)
-        lens = np.diff(raw_off)
-        lengths = np.maximum(np.minimum(hi.astype(np.int64), lens - 1) - lo + 1, 0).astype(np.int32)
-        return self._pipeline(_IngestRaw(self, host_raw, raw_off, lo, hi, lengths, SPIKE_MODES[spike_removal]),
-                              lengths, aut, rev, want_seq, chunk_reads, lanes)
+        return self._call_whole(_WholeReads(host_raw, raw_off), win_lo, win_hi, aut, rev, spike_removal, want_seq,
+                                chunk_reads, lanes)
 
     def call_arrays_vbz(self, host_payload, table, read_chunk, raw_off, win_lo, win_hi, aut, rev,
                         spike_removal: str = 'Brute', want_seq: bool = True, chunk_reads: int = 25000,
@@ -746,15 +715,16 @@ class CallerEngine:
         StreamVByte / zig-zag delta decode (wstr_vbz_decode_batch) writes the int16 reads on the device.  Same
         result dict, plus ``chunk_status`` (WSTR_VBZ_* per chunk) and ``zstd_status`` (WSTR_ZSTD_* per chunk, 0
         for a chunk that was not a zstd frame); a read with a bad chunk has undefined results."""
+        return self._call_whole(_VBZReads(host_payload, table, read_chunk, raw_off), win_lo, win_hi, aut, rev,
+                                spike_removal, want_seq, chunk_reads, lanes)
+
+    def _call_whole(self, src, win_lo, win_hi, aut, rev, spike_removal, want_seq=True, chunk_reads=25000,
+                    lanes=2) -> Dict[str, np.ndarray]:
+        """``call_arrays_raw`` of whole reads in any form (a ``_WholeReads``)."""
         from .normalize import SPIKE_MODES
-        raw_off = np.asarray(raw_off, dtype=np.int64)
-        lo = np.asarray(win_lo, dtype=np.int32)
-        hi = np.asarray(win_hi, dtype=np.int32)
-        lens = np.diff(raw_off)
-        lengths = np.maximum(np.minimum(hi.astype(np.int64), lens - 1) - lo + 1, 0).astype(np.int32)
-        ingest = _IngestVBZ(self, host_payload, table, np.asarray(read_chunk, dtype=np.int64), raw_off, lo, hi,
-                            lengths, SPIKE_MODES[spike_removal])
-        return self._pipeline(ingest, lengths, aut, rev, want_seq, chunk_reads, lanes)
+        lo, hi, lengths = _window_bounds(src.raw_off, win_lo, win_hi)
+        return self._pipeline(_IngestRaw(self, src, lo, hi, lengths, SPIKE_MODES[spike_removal]), lengths, aut, rev,
+                              want_seq, chunk_reads, lanes)
 
     def _pipeline(self, ingest, lengths, aut, rev, want_seq, chunk_reads, lanes) -> Dict[str, np.ndarray]:
         import torch
@@ -766,22 +736,18 @@ class CallerEngine:
         cap = lengths.astype(np.int64) // max(self.cc.min_values_per_state - 1, 1) + 16
         seq_off = np.zeros(n + 1, dtype=np.int64)
         seq_off[1:] = np.cumsum(cap)
-        out = self._host_results(n, int(seq_off[-1]) if want_seq else 0)
         with torch.cuda.device(self.device):
             comp = torch.cuda.current_stream()
-            if self._copy_stream is None:
-                self._copy_stream = (torch.cuda.Stream(), torch.cuda.Stream())
-            cs_in, cs_out = self._copy_stream
-            # device-side signal and result buffers live on the engine and only ever grow, so the
-            # chunk loop makes no allocator calls
+            cs_in, cs_out = self._side_streams('copy')
+            # signal and result buffers (device, and pinned on the host) live on the engine and only ever grow,
+            # so the chunk loop makes no allocator calls
             ingest.allocate()
             d_sig = ingest.d_sig
-            dev = {k: self._device_buffer(k, n, dt) for k, dt in
-                   (('len1', torch.int32), ('len2', torch.int32), ('cost1', torch.float64),
-                    ('cost2', torch.float64), ('status', torch.int32), ('ties', torch.int32))}
+            buffers = [(k, n, torch.float64 if k in ('cost1', 'cost2') else torch.int32) for k in _SCALARS]
             if want_seq:
-                dev['seq1'] = self._device_buffer('seq1', int(seq_off[-1]), torch.uint8)
-                dev['seq2'] = self._device_buffer('seq2', int(seq_off[-1]), torch.uint8)
+                buffers += [(k, int(seq_off[-1]), torch.uint8) for k in ('seq1', 'seq2')]
+            dev = {k: self._device_buffer(k, size, dt) for k, size, dt in buffers}
+            out = {k: self._host_buffer(k, size, dt) for k, size, dt in buffers}
             cs_in.wait_stream(comp)
             cs_out.wait_stream(comp)
             chunks = list(zip(bounds[:-1], bounds[1:]))
@@ -818,17 +784,14 @@ class CallerEngine:
             # kernels of consecutive chunks are independent, so one chunk's kernel tails and
             # latency-bound mid-stage overlap the next chunk's DP
             n_lanes = max(1, int(lanes))
-            if n_lanes > 1 and self._lane_streams is None:
-                self._lane_streams = [torch.cuda.Stream() for _ in range(3)]
-            streams = [comp] + (self._lane_streams[:n_lanes - 1] if n_lanes > 1 else [])
+            streams = [comp] + (self._side_streams('lanes')[:n_lanes - 1] if n_lanes > 1 else [])
             for st in streams[1:]:
                 st.wait_stream(comp)
             for ci, (a, b) in enumerate(chunks):
                 ev = sent[ci]
                 lane = ci % len(streams)
                 st = streams[lane]
-                lo = int(off[a])
-                hi = min(int(off[b - 1] + ((int(lengths[b - 1]) + 1) & ~1) + 2), d_sig.numel())
+                lo, hi = _span(off, lengths, a, b, d_sig.numel())
                 with torch.cuda.stream(st):
                     st.wait_event(ev)
                     mark(f'call{a} begin', st)
@@ -850,7 +813,7 @@ class CallerEngine:
                         s0, s1 = int(seq_off[a]), int(seq_off[b])
                         out['seq1'][s0:s1].copy_(o['seq1'][:s1 - s0], non_blocking=True)
                         out['seq2'][s0:s1].copy_(o['seq2'][:s1 - s0], non_blocking=True)
-                    ingest.fetch(a, b, out)
+                    ingest.fetch(a, b)
                     mark(f'd2h{a} end', cs_out)
                 keep.append(o)
             for st in streams[1:]:
@@ -861,7 +824,7 @@ class CallerEngine:
         # per-read scalars are handed back as copies; reads the device could not finish (status != 0) carry
         # -1 / NaN instead of whatever the buffers held.  The sequence bytes are views of the engine's pinned
         # buffers (hundreds of MB per 100 000 reads): valid until the next call_arrays on this engine.
-        res = {k: out[k][:n].numpy().copy() for k in _SCALARS}
+        res = {k: out[k].numpy().copy() for k in _SCALARS}
         res['ttest_ties'] = res.pop('ties')
         bad = res['status'] != 0
         if bad.any():
@@ -870,10 +833,10 @@ class CallerEngine:
             res['cost1'][bad] = np.nan
             res['cost2'][bad] = np.nan
         if want_seq:
-            res['seq1'] = out['seq1'][:int(seq_off[-1])].numpy()
-            res['seq2'] = out['seq2'][:int(seq_off[-1])].numpy()
+            res['seq1'] = out['seq1'].numpy()
+            res['seq2'] = out['seq2'].numpy()
             res['seq_off'] = seq_off[:-1]
-        ingest.finish(res, out, n)
+        ingest.finish(res)
         return res
 
     def _chunk_bounds(self, n: int, step: int):
@@ -922,24 +885,14 @@ class CallerEngine:
             self._dev_cache[name] = cur
         return cur[:numel]
 
-    def _host_results(self, n: int, seq_bytes: int):
-        """Pinned host buffers for the per-read results, grown on demand and reused."""
+    def _host_buffer(self, name: str, numel: int, dtype):
+        """Pinned host buffer ``name`` as ``_device_buffer`` keeps device ones: grown on demand and reused."""
         import torch
-        cur = self._host_out
-        if cur is None or cur['len1'].numel() < n or cur['seq1'].numel() < seq_bytes:
-            n_cap = max(n, cur['len1'].numel() if cur else 0)
-            s_cap = max(seq_bytes, cur['seq1'].numel() if cur else 0, 1)
-            pin = torch.cuda.is_available()
-            cur = dict(len1=torch.empty(n_cap, dtype=torch.int32, pin_memory=pin),
-                       len2=torch.empty(n_cap, dtype=torch.int32, pin_memory=pin),
-                       cost1=torch.empty(n_cap, dtype=torch.float64, pin_memory=pin),
-                       cost2=torch.empty(n_cap, dtype=torch.float64, pin_memory=pin),
-                       status=torch.empty(n_cap, dtype=torch.int32, pin_memory=pin),
-                       ties=torch.empty(n_cap, dtype=torch.int32, pin_memory=pin),
-                       seq1=torch.empty(s_cap, dtype=torch.uint8, pin_memory=pin),
-                       seq2=torch.empty(s_cap, dtype=torch.uint8, pin_memory=pin))
-            self._host_out = cur
-        return cur
+        cur = self._host_cache.get(name)
+        if cur is None or cur.numel() < numel or cur.dtype != dtype:
+            cur = torch.empty(max(numel, 1), dtype=dtype, pin_memory=torch.cuda.is_available())
+            self._host_cache[name] = cur
+        return cur[:numel]
 
     def call_raw_batch(self, raws: Sequence[np.ndarray], windows, aut_ids, reverse,
                        spike_removal: str = 'Brute', offset: float = 0.35) -> list:
@@ -953,22 +906,10 @@ class CallerEngine:
         of ``aut_ids`` may be a (template id, reverse id) pair (its ``reverse`` entry is ignored, e.g. None): the
         read is searched on both strands and called with the strand ``choose_strand`` picks, whose id and
         orientation are then used; ``last_located['strand']`` has every read's strand, given or detected."""
-        n = len(raws)
-        if n == 0:
+        if len(raws) == 0:
             return []
-        host, raw_off = pack_raw(raws)
-        if windows is None:
-            d_raw = self._upload_raw(host)
-            return self._call_located(d_raw, raw_off, aut_ids, reverse, spike_removal, offset,
-                                      lambda idx: [raws[r] for r in idx])
-        aut = _single_ids(aut_ids)
-        rev = np.asarray(reverse, dtype=np.uint8)
-        lo = np.array([w[0] for w in windows], dtype=np.int32)
-        hi = np.array([w[1] for w in windows], dtype=np.int32)
-        if (lo < 0).any():
-            raise ValueError('negative window start')
-        res = self.call_arrays_raw(host, raw_off, lo, hi, aut, rev, spike_removal)
-        return self._raw_results(res, lambda idx: [raws[r] for r in idx], windows, aut_ids, reverse, spike_removal)
+        src = _WholeReads(*pack_raw(raws), samples=lambda idx: [raws[r] for r in idx])
+        return self._call_reads(src, windows, aut_ids, reverse, spike_removal, offset)
 
     def call_vbz_batch(self, reads, windows, aut_ids, reverse, spike_removal: str = 'Brute',
                        offset: float = 0.35) -> list:
@@ -979,27 +920,25 @@ class CallerEngine:
         locates the windows first (``locate_arrays_vbz``): the payload crosses PCIe once and the decoded reads
         stay on the device for the call; reads not found come back as ``NotLocated``.  Strand pairs in ``aut_ids``
         as in ``call_raw_batch``."""
-        n = len(reads)
-        if n == 0:
+        if len(reads) == 0:
             return []
         if any(r.n_samples <= 0 for r in reads):
             raise ValueError('empty raw read')
-        host, table, read_chunk, raw_off = pack_vbz(reads)
+        return self._call_reads(_VBZReads(*pack_vbz(reads), reads), windows, aut_ids, reverse, spike_removal, offset)
+
+    def _call_reads(self, src, windows, aut_ids, reverse, spike_removal, offset) -> list:
+        """``call_raw_batch`` of whole reads in any form (a ``_WholeReads``)."""
         if windows is None:
-            d_raw, chunk_status, zstd_status = self._decode_vbz(host, table, raw_off)
-            _raise_bad_chunk(reads, read_chunk, chunk_status.cpu().numpy(), zstd_status)
-            return self._call_located(d_raw, raw_off, aut_ids, reverse, spike_removal, offset,
-                                      lambda idx: [reads[r].decode() for r in idx])
-        aut = _single_ids(aut_ids)
-        rev = np.asarray(reverse, dtype=np.uint8)
-        lo = np.array([w[0] for w in windows], dtype=np.int32)
-        hi = np.array([w[1] for w in windows], dtype=np.int32)
-        if (lo < 0).any():
-            raise ValueError('negative window start')
-        res = self.call_arrays_vbz(host, table, read_chunk, raw_off, lo, hi, aut, rev, spike_removal)
-        _raise_bad_chunk(reads, read_chunk, res['chunk_status'], res['zstd_status'])
-        return self._raw_results(res, lambda idx: [reads[r].decode() for r in idx], windows, aut_ids, reverse,
-                                 spike_removal)
+            return self._call_located(src, aut_ids, reverse, spike_removal, offset)
+        res = self._call_whole(src, [w[0] for w in windows], [w[1] for w in windows], _single_ids(aut_ids),
+                               np.asarray(reverse, dtype=np.uint8), spike_removal)
+        src.raise_bad(res)
+
+        def signals_of(idx):
+            from .normalize import normalize_windows
+            return normalize_windows(src.samples(idx), [windows[r] for r in idx], spike_removal,
+                                     device=str(self.device))
+        return self._results(res, signals_of, aut_ids, reverse)
 
     # -- STR window search in whole reads (DESIGN.md section 4.5) ----------------------------------------------
     def locate_packed(self, d_sig, off, lengths, aut, offset: float = 0.35) -> Dict[str, np.ndarray]:
@@ -1052,50 +991,37 @@ class CallerEngine:
         """Whole int16 reads ``host_raw[raw_off[r] : raw_off[r+1]]`` (``pack_raw``) in, their STR windows out:
         whole-read normalisation (wstr_normalize_batch, window [0, N-1]) and the window search on the device.
         ``aut`` and the dict as in ``locate_packed``."""
-        raw_off = np.asarray(raw_off, dtype=np.int64)
-        return self._locate_device(self._upload_raw(host_raw), raw_off, aut, spike_removal, offset)
+        return self._locate_whole(_WholeReads(host_raw, raw_off), aut, spike_removal, offset)
 
     def locate_arrays_vbz(self, host_payload, table, read_chunk, raw_off, aut, spike_removal: str = 'Brute',
                           offset: float = 0.35) -> Dict[str, np.ndarray]:
         """``locate_arrays_raw`` for VBZ-compressed reads (``pack_vbz``): decoded on the device first.  The dict
         also carries ``chunk_status`` (WSTR_VBZ_* per chunk) and ``zstd_status`` (WSTR_ZSTD_* per chunk); a read
         with a bad chunk has undefined results."""
-        raw_off = np.asarray(raw_off, dtype=np.int64)
-        d_raw, chunk_status, zstd_status = self._decode_vbz(host_payload, table, raw_off)
-        res = self._locate_device(d_raw, raw_off, aut, spike_removal, offset)
-        res['chunk_status'] = chunk_status.cpu().numpy()
-        res['zstd_status'] = zstd_status
+        return self._locate_whole(_VBZReads(host_payload, table, read_chunk, raw_off), aut, spike_removal, offset)
+
+    def _locate_whole(self, src, aut, spike_removal, offset) -> Dict[str, np.ndarray]:
+        """``locate_arrays_raw`` of whole reads in any form (a ``_WholeReads``), with its decode statuses."""
+        st = self._load(src)
+        res = self._locate_device(src.d_raw, src.raw_off, aut, spike_removal, offset)
+        res.update(st)
         return res
 
-    def _upload_raw(self, host_raw):
+    def _load(self, src) -> dict:
+        """Every read of ``src`` sent and decoded on the current stream into the device buffer 'loc_raw16' (which
+        the pipelined call does not grow or write, so located reads can be called from it); returns the decode
+        statuses as ``finish`` puts them into a result."""
         import torch
+        n = len(src.raw_off) - 1
         with torch.cuda.device(self.device):
-            d_raw = self._device_buffer('loc_raw16', int(host_raw.numel()), torch.int16)
-            d_raw.copy_(host_raw, non_blocking=True)
-        return d_raw
-
-    def _decode_vbz(self, host_payload, table, raw_off):
-        """Payload -> device -> decoded whole int16 reads (device), the per-chunk StreamVByte status (device) and
-        the per-chunk zstd status (host)."""
-        import torch
-        m = len(table['in_off'])
-        _, need = _vbz_layout(table, host_payload)
-        with torch.cuda.device(self.device):
-            d_pay = self._device_buffer('vbz_payload', need, torch.uint8)
-            d_pay[:int(host_payload.numel())].copy_(host_payload, non_blocking=True)
-            d_raw = self._device_buffer('loc_raw16', int(raw_off[-1]), torch.int16)
-            d_st = torch.zeros(max(m, 1), dtype=torch.int32, device=self.device)
-            _, nf, rows = _zstd_frames(table, 0, m)
-            d_zst = torch.zeros(max(nf, 1), dtype=torch.int32, device=self.device)
-            if nf:
-                ws = self._device_buffer('zstd_ws0', _lib.zstd_workspace_bytes(nf), torch.uint8)
-                _zstd_decode(table, rows, d_pay, d_zst, ws)
-            if m:
-                ws = self._device_buffer('vbz_ws0', _lib.vbz_workspace_bytes(m), torch.uint8)
-                _lib.vbz_decode_batch(d_pay, table['in_off'], table['in_bytes'], table['n_samples'], table['n_out'],
-                                      table['kind'], table['zigzag'], table['out_off'], d_raw, d_st, ws)
-            zstd_status = _chunk_zstd_status(table, d_zst[:nf].cpu().numpy())
-        return d_raw, d_st[:m], zstd_status
+            src.allocate(self, 'loc_raw16')
+            src.send(0, n)
+            src.decode(self, 0, n, 0)
+            src.fetch(0, n)
+            torch.cuda.current_stream().synchronize()
+        st = {}
+        src.finish(st)
+        return st
 
     def _locate_device(self, d_raw, raw_off, aut, spike_removal, offset) -> Dict[str, np.ndarray]:
         """Whole-read normalisation of int16 reads on the device, then the window search."""
@@ -1116,12 +1042,13 @@ class CallerEngine:
             del d_sig
         return res
 
-    def _call_located(self, d_raw, raw_off, aut_ids, reverse, spike_removal, offset, raws_of) -> list:
-        """The located-then-called chain on whole int16 reads already on the device: locate, bring the windows
-        to the host, normalise the found windows and call them from the same device buffer, each with the
-        automaton and orientation of its strand (given, or chosen by the both-strand search)."""
+    def _call_located(self, src, aut_ids, reverse, spike_removal, offset) -> list:
+        """The located-then-called chain: send and decode the whole reads, locate, bring the windows to the
+        host, normalise the found windows and call them from the same device buffer, each with the automaton
+        and orientation of its strand (given, or chosen by the both-strand search)."""
         import torch
-        from .normalize import SPIKE_MODES
+        src.raise_bad(self._load(src))
+        d_raw, raw_off = src.d_raw, src.raw_off
         loc = self._locate_device(d_raw, raw_off, aut_ids, spike_removal, offset)
         pair, ids = split_pairs(aut_ids)
         fill_given_strands(loc, [None if p else r for p, r in zip(pair, reverse)])
@@ -1135,59 +1062,30 @@ class CallerEngine:
         if len(found) < len(out):         # the found reads, packed
             with torch.cuda.device(self.device):
                 d_raw = torch.cat([d_raw[int(raw_off[r]):int(raw_off[r + 1])] for r in found])
-            sub_off = np.zeros(len(found) + 1, dtype=np.int64)
-            sub_off[1:] = np.cumsum(np.diff(raw_off)[found])
-        else:
-            sub_off = raw_off
-        lo, hi = loc['lo'][found], loc['hi'][found]
-        lengths = (hi - lo + 1).astype(np.int32)
-        ingest = _IngestDeviceRaw(self, d_raw, sub_off, lo, hi, lengths, SPIKE_MODES[spike_removal])
-        res = self._pipeline(ingest, lengths, aut[found], rev[found], True, 25000, 2)
-        windows = list(zip(lo.tolist(), hi.tolist()))
-        calls = self._raw_results(res, lambda idx: raws_of([int(found[k]) for k in idx]), windows,
-                                  aut[found].tolist(), [bool(x) for x in rev[found]], spike_removal)
+            raw_off = np.zeros(len(found) + 1, dtype=np.int64)
+            raw_off[1:] = np.cumsum(np.diff(src.raw_off)[found])
+        located = _WholeReads(None, raw_off, d_raw, samples=lambda idx: src.samples([int(found[k]) for k in idx]))
+        windows = list(zip(loc['lo'][found].tolist(), loc['hi'][found].tolist()))
+        calls = self._call_reads(located, windows, aut[found], rev[found], spike_removal, offset)
         for k, r in enumerate(found):
             out[r] = calls[k]
-        return out
-
-    def _raw_results(self, res, raws_of, windows, aut_ids, reverse, spike_removal) -> List[CallerResult]:
-        """CallerResults of a ``call_arrays_raw``-style result dict.  Reads the device did not finish, or whose
-        t-test decision was within rounding of flipping, are redone as in results_from (the reference's
-        exception, or the host's libm for a t-test tie) from their host int16 samples, ``raws_of(indices)``."""
-        status, ties = res['status'], res['ttest_ties']
-        self.last_ttest_ties = int((ties > 0).sum())
-        out: List[Optional[CallerResult]] = []
-        redo = []
-        so = res['seq_off']
-        for r in range(len(status)):
-            if status[r] == 0 and ties[r] == 0:
-                a = int(so[r])
-                out.append(CallerResult(seq=res['seq1'][a:a + res['len1'][r]].tobytes().decode('ascii'),
-                                        cost=float(res['cost1'][r]),
-                                        resc_seq=res['seq2'][a:a + res['len2'][r]].tobytes().decode('ascii'),
-                                        resc_cost=float(res['cost2'][r])))
-            else:
-                out.append(None)
-                redo.append(r)
-        if redo:
-            from .normalize import normalize_windows
-            sigs = normalize_windows(raws_of(redo), [windows[r] for r in redo], spike_removal,
-                                     device=str(self.device))
-            fixed = self._call_batch_host(sigs, [aut_ids[r] for r in redo], [reverse[r] for r in redo])
-            for r, f in zip(redo, fixed):
-                out[r] = f
         return out
 
     def results_from(self, o, signals, aut_ids, reverse) -> List[CallerResult]:
         """Device results -> CallerResult list; reads the device could not finish (status != 0)
         are redone on the host path or raise what the reference raises."""
-        status = o['status'].cpu().numpy()
-        ties = o['ties'].cpu().numpy() if 'ties' in o else np.zeros_like(status)
+        h = {k: o[k].cpu().numpy() for k in ('status', 'ties', 'len1', 'len2', 'cost1', 'cost2', 'seq1', 'seq2')
+             if k in o}
+        h['ttest_ties'] = h.pop('ties', np.zeros_like(h['status']))
+        return self._results(dict(h, seq_off=o['seq_off']), lambda idx: [signals[r] for r in idx], aut_ids, reverse)
+
+    def _results(self, h, signals_of, aut_ids, reverse) -> List[CallerResult]:
+        """CallerResults of the host result arrays ``h`` of a call (as ``call_arrays`` returns them).  Reads the
+        device did not finish (status != 0), or whose t-test decision was within rounding of flipping (ttest_ties
+        > 0), are redone on the host path from their float64 windows, ``signals_of(indices)``."""
+        status, ties, len1, len2, cost1, cost2, seq1, seq2, off = (
+            h[k] for k in ('status', 'ttest_ties', 'len1', 'len2', 'cost1', 'cost2', 'seq1', 'seq2', 'seq_off'))
         self.last_ttest_ties = int((ties > 0).sum())
-        len1, len2 = o['len1'].cpu().numpy(), o['len2'].cpu().numpy()
-        cost1, cost2 = o['cost1'].cpu().numpy(), o['cost2'].cpu().numpy()
-        seq1, seq2 = o['seq1'].cpu().numpy(), o['seq2'].cpu().numpy()
-        off = o['seq_off']
         out: List[Optional[CallerResult]] = []
         redo = []
         for r in range(len(status)):
@@ -1204,8 +1102,7 @@ class CallerEngine:
         if redo:
             # status 5 (spline needs interior knots) is a legitimate host evaluation; every other
             # status is an exception in the reference, which the host path raises with its type
-            fixed = self._call_batch_host([signals[r] for r in redo], [aut_ids[r] for r in redo],
-                                          [reverse[r] for r in redo])
+            fixed = self._call_batch_host(signals_of(redo), [aut_ids[r] for r in redo], [reverse[r] for r in redo])
             for r, res in zip(redo, fixed):
                 out[r] = res
         return out
@@ -1247,21 +1144,6 @@ def _single_ids(aut_ids) -> np.ndarray:
         raise ValueError(f'read {int(np.flatnonzero(pair)[0])} of the batch: a given window needs a given strand '
                          '(one automaton id, not a pair)')
     return ids[:, 0].copy()
-
-
-def _raise_bad_chunk(reads, read_chunk, chunk_status, zstd_status=None) -> None:
-    """The Fast5FormatError of the first chunk the device decoders refused, naming the file and the read: a
-    zstd frame they refuse raises the host decoder's own 'zstd: corrupt VBZ chunk'."""
-    from .fast5 import Fast5FormatError
-    zst = np.zeros(len(chunk_status), dtype=np.int32) if zstd_status is None else np.asarray(zstd_status)
-    bad = np.flatnonzero((np.asarray(chunk_status) != 0) | (zst != 0))
-    if len(bad):
-        c = int(bad[0])
-        r = int(np.searchsorted(read_chunk, c, side='right')) - 1
-        msg = ('zstd: corrupt VBZ chunk' if zst[c] else
-               _lib.VBZ_STATUS_MESSAGES.get(int(chunk_status[c]), 'VBZ: corrupt chunk'))
-        raise Fast5FormatError(f'{reads[r].path}: read {reads[r].read_name}: {msg} '
-                               f'(chunk at sample {reads[r].chunks[c - int(read_chunk[r])].start})')
 
 
 _default_engine: Optional[CallerEngine] = None

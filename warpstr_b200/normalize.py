@@ -21,28 +21,17 @@ def normalize_windows(raws: Sequence[np.ndarray], windows: Sequence[Tuple[int, i
     """For every raw int16 read return the float64 normalised samples of
     ``[l_start_raw, r_end_raw]`` (inclusive, clipped at the read's end like a numpy slice)."""
     import torch
+    from .caller import _window_bounds, pack_raw
     if spike_removal not in SPIKE_MODES:
         raise AssertionError('spike_removal must be None, median3, median5 or Brute')
     n = len(raws)
     if n == 0:
         return ([], np.zeros((0, 2))) if return_shift_scale else []
     dev = torch.device(device)
-    lens = np.fromiter((len(r) for r in raws), dtype=np.int64, count=n)
-    if (lens <= 0).any():
-        raise ValueError('empty raw read')
-    raw_off = np.zeros(n + 1, dtype=np.int64)
-    raw_off[1:] = np.cumsum(lens)
-    lo = np.array([w[0] for w in windows], dtype=np.int32)
-    hi = np.array([w[1] for w in windows], dtype=np.int32)
-    if (lo < 0).any():
-        raise ValueError('negative window start')
-    out_len = np.maximum(np.minimum(hi.astype(np.int64), lens - 1) - lo + 1, 0)
+    host, raw_off = pack_raw(raws)
+    lo, hi, out_len = _window_bounds(raw_off, [w[0] for w in windows], [w[1] for w in windows])
     out_off = np.zeros(n, dtype=np.int64)
     out_off[1:] = np.cumsum(out_len[:-1])
-    host = torch.empty(int(raw_off[-1]), dtype=torch.int16, pin_memory=True)
-    hb = host.numpy()
-    for r, o in zip(raws, raw_off[:-1]):
-        hb[o:o + len(r)] = np.asarray(r, dtype=np.int16)
     with torch.cuda.device(dev):
         d_raw = host.to(dev, non_blocking=True)
         d_out = torch.empty(max(int(out_len.sum()), 1), dtype=torch.float64, device=dev)

@@ -16,7 +16,7 @@ import pandas as pd
 
 from . import templates as tmpl
 from .automata import StateAutomata
-from .caller import CallerEngine, CallerResult, fill_given_strands
+from .caller import CallerEngine, CallerResult, _VBZReads, _WholeReads, fill_given_strands, pack_raw, pack_vbz
 from .config import CallerConfig, Config, RescalerConfig
 from .pore_model import PoreModel, get_pore_model
 
@@ -131,22 +131,22 @@ class CallerWrapper:
         a strand may be None: the read is searched on both strands and called on the one found
         (``caller.choose_strand``); ``engine.last_located['strand']`` has every read's strand (0 template,
         1 reverse, -1 found on neither).  Given windows need given strands (ValueError naming the read)."""
-        reverse = _strands(reverse)
-        if windows is not None:
-            _need_strands(reverse, [f'#{k}' for k in range(len(reverse))], 'a given window')
-        return self.engine.call_raw_batch(raws, windows, self._aut(reverse), reverse,
-                                          spike_removal or self.caller_config.spike_removal, offset)
+        return self._run(self.engine.call_raw_batch, raws, windows, reverse, spike_removal, offset)
 
     def run_compressed(self, reads, windows, reverse: Sequence[Optional[bool]],
                        spike_removal: Optional[str] = None, offset: float = 0.35) -> list:
         """``run_raw`` for reads as their fast5 files store them (fast5.CompressedRead, see
         ``get_compressed_workload``): the VBZ decode happens on the device too, order preserved.  None strands
         as in ``run_raw``."""
+        return self._run(self.engine.call_vbz_batch, reads, windows, reverse, spike_removal, offset)
+
+    def _run(self, call, reads, windows, reverse, spike_removal, offset) -> list:
+        """``run_raw`` with the engine's ``call`` of the reads' form; errors name a read by its name, else '#k'."""
         reverse = _strands(reverse)
         if windows is not None:
-            _need_strands(reverse, [r.read_name for r in reads], 'a given window')
-        return self.engine.call_vbz_batch(reads, windows, self._aut(reverse), reverse,
-                                          spike_removal or self.caller_config.spike_removal, offset)
+            _need_strands(reverse, [getattr(r, 'read_name', f'#{k}') for k, r in enumerate(reads)], 'a given window')
+        return call(reads, windows, self._aut(reverse), reverse, spike_removal or self.caller_config.spike_removal,
+                    offset)
 
     def _aut(self, reverse):
         """Per read the automaton of its strand, or the (template, reverse) pair where the strand is None."""
@@ -163,28 +163,22 @@ class CallerWrapper:
         (0 template, 1 reverse, given or detected; -1 found on neither), ``strand_score`` / ``strand_status`` /
         ``strand_lo`` / ``strand_hi`` (n, 2) both searches of those reads (NaN / -1 for a read with a given
         strand)."""
-        from .caller import pack_raw
-        reverse = _strands(reverse)
-        if not raws:
-            return _no_reads()
-        host, raw_off = pack_raw(raws)
-        res = self.engine.locate_arrays_raw(host, raw_off, self._aut(reverse),
-                                            spike_removal or self.caller_config.spike_removal, offset)
-        fill_given_strands(res, reverse)
-        return res
+        return self._locate(_WholeReads(*pack_raw(raws)) if raws else None, reverse, spike_removal, offset)
 
     def locate_compressed(self, reads, reverse: Sequence[Optional[bool]], spike_removal: Optional[str] = None,
                           offset: float = 0.35) -> dict:
         """``locate_raw`` for reads as their fast5 files store them (fast5.CompressedRead): decoded on the device.
         A chunk the host decoder would refuse raises that Fast5FormatError."""
-        from .caller import _raise_bad_chunk, pack_vbz
+        return self._locate(_VBZReads(*pack_vbz(reads), reads) if reads else None, reverse, spike_removal, offset)
+
+    def _locate(self, src, reverse, spike_removal, offset) -> dict:
+        """``locate_raw`` of whole reads in any form (a ``caller._WholeReads``; None: no reads)."""
         reverse = _strands(reverse)
-        if not reads:
+        if src is None:
             return _no_reads()
-        host, table, read_chunk, raw_off = pack_vbz(reads)
-        res = self.engine.locate_arrays_vbz(host, table, read_chunk, raw_off, self._aut(reverse),
-                                            spike_removal or self.caller_config.spike_removal, offset)
-        _raise_bad_chunk(reads, read_chunk, res.pop('chunk_status'), res.pop('zstd_status'))
+        res = self.engine._locate_whole(src, self._aut(reverse), spike_removal or self.caller_config.spike_removal,
+                                        offset)
+        src.raise_bad(res)
         fill_given_strands(res, reverse)
         return res
 
