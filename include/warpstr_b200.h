@@ -240,6 +240,32 @@ int wstr_locate_batch(wstr_automaton *const *automata, int32_t n_automata, const
                       double offset, int32_t *d_lo, int32_t *d_hi, double *d_score, int32_t *d_status,
                       void *d_workspace, int64_t workspace_bytes, void *stream);
 
+/* ---- (3c) a panel's reads found in a whole run by their flanks --------------------------------------
+ * Replaces the basecall and the alignment that tell which reads belong to which locus (DESIGN.md section
+ * 4.6).  The automata come four per locus, in this order: template-strand left flank, template-strand right
+ * flank, reverse-strand left flank, reverse-strand right flank (chains, in practice; any automata
+ * wstr_locate_batch takes are accepted, all of one min_values_per_state).  Every automaton is searched in every
+ * read exactly as wstr_locate_batch searches it: per (read, automaton) the same lo / hi / score / status, bit
+ * for bit.  Then, per (read, locus), a strand passes iff both of its flanks are WSTR_LOCATE_FOUND and
+ * left.hi < right.lo; one strand passing gives that strand, both give the lower left.score + right.score, an
+ * exact tie the template.  Every (read, locus) with a strand is one wstr_assign_hit in d_hits (capacity
+ * n_reads * n_automata / 4), in no particular order; *d_n_hits is their count.
+ *   d_table  NULL, or n_reads * n_automata entries (e = read * n_automata + automaton) as a struct of arrays:
+ *            [score float64 x m][lo int32 x m][hi int32 x m][status int32 x m], m = n_reads * n_automata,
+ *            8-byte aligned.  Without it the table stays in the workspace.
+ * d_signal / sig_off / lengths as for wstr_locate_batch.  d_workspace: wstr_assign_workspace_bytes(...) bytes,
+ * 16-byte aligned.  Nothing is copied by the DMA engines and the call does not block. */
+typedef struct {
+    int32_t read, locus, strand, pad_;       /* strand: 0 template, 1 reverse */
+    int32_t left_lo, left_hi, right_lo, right_hi;   /* the chosen strand's flank windows, inclusive */
+    double left_score, right_score;
+} wstr_assign_hit;
+int64_t wstr_assign_workspace_bytes(wstr_automaton *const *automata, int32_t n_automata, int32_t n_reads);
+int wstr_assign_batch(wstr_automaton *const *automata, int32_t n_automata, const double *d_signal,
+                      const int64_t *sig_off, const int32_t *lengths, int32_t n_reads, double offset, void *d_table,
+                      wstr_assign_hit *d_hits, int32_t *d_n_hits, void *d_workspace, int64_t workspace_bytes,
+                      void *stream);
+
 /* ---- whole per-read call --------------------------------------------------------------------------
  * Replaces WarpSTR.run (src/caller/caller.py:117-149) for a batch: first pass, per-run statistics
  * and spline rescale, bad-repeat mask, second pass on the rescaled signal, state-wise costs and

@@ -84,6 +84,9 @@ _SIGNATURES = {
     'wstr_locate_batch': (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int32, c_i32p, c_vp, c_i64p, c_i32p,
                                          ctypes.c_int32, ctypes.c_double, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int64,
                                          c_vp]),
+    'wstr_assign_workspace_bytes': (ctypes.c_int64, [ctypes.POINTER(c_vp), ctypes.c_int32, ctypes.c_int32]),
+    'wstr_assign_batch': (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int32, c_vp, c_i64p, c_i32p, ctypes.c_int32,
+                                         ctypes.c_double, c_vp, c_vp, c_vp, c_vp, ctypes.c_int64, c_vp]),
     'wstr_profile_enable': (ctypes.c_int, [ctypes.c_int32]),
     'wstr_profile_read': (ctypes.c_int, [c_f64p, c_i32p, ctypes.c_int32]),
 }
@@ -393,6 +396,42 @@ def locate_batch(automata: Sequence[DeviceAutomaton], read_automaton, d_signal, 
         int(ln.shape[0]), float(offset), _dptr(d_lo), _dptr(d_hi), _dptr(d_score), _dptr(d_status),
         _dptr(d_workspace), int(d_workspace.numel() * d_workspace.element_size()), _stream_ptr(stream))
     check(rc, 'wstr_locate_batch')
+
+
+# wstr_assign_hit: one (read, locus) whose flanks were found on a strand
+ASSIGN_HIT = np.dtype([('read', np.int32), ('locus', np.int32), ('strand', np.int32), ('pad_', np.int32),
+                       ('left_lo', np.int32), ('left_hi', np.int32), ('right_lo', np.int32), ('right_hi', np.int32),
+                       ('left_score', np.float64), ('right_score', np.float64)])
+
+
+def assign_workspace_bytes(automata: Sequence[DeviceAutomaton], n_reads: int) -> int:
+    n = lib().wstr_assign_workspace_bytes(_handles(automata), len(automata), int(n_reads))
+    if n < 0:
+        check(int(n), 'wstr_assign_workspace_bytes')
+    return int(n)
+
+
+def assign_batch(automata: Sequence[DeviceAutomaton], d_signal, sig_off, lengths, offset: float, d_table, d_hits,
+                 d_n_hits, d_workspace, stream=None) -> None:
+    """wstr_assign_batch.  ``d_table``: None, or a uint8 tensor of 20 * n_reads * len(automata) bytes (the header's
+    struct of arrays, see ``split_table``); ``d_hits``: a uint8 tensor with room for n_reads * len(automata) / 4
+    ASSIGN_HIT records; ``d_n_hits``: one int32."""
+    so = _np(sig_off, np.int64)
+    ln = _np(lengths, np.int32)
+    rc = lib().wstr_assign_batch(
+        _handles(automata), len(automata), _dptr(d_signal), _ptr(so, c_i64p), _ptr(ln, c_i32p), int(ln.shape[0]),
+        float(offset), _dptr(d_table), _dptr(d_hits), _dptr(d_n_hits), _dptr(d_workspace),
+        int(d_workspace.numel() * d_workspace.element_size()), _stream_ptr(stream))
+    check(rc, 'wstr_assign_batch')
+
+
+def split_table(buf: np.ndarray, n_reads: int, n_automata: int):
+    """The bytes of wstr_assign_batch's d_table -> (lo, hi, score, status), each [n_reads, n_automata]."""
+    m = n_reads * n_automata
+    buf = np.ascontiguousarray(buf, dtype=np.uint8)
+    score = buf[:8 * m].view(np.float64)
+    lo, hi, status = (buf[8 * m + 4 * m * k:8 * m + 4 * m * (k + 1)].view(np.int32) for k in range(3))
+    return tuple(a.reshape(n_reads, n_automata) for a in (lo, hi, score, status))
 
 
 PROFILE_CATEGORIES =('dp_fill_traceback', 'midstage', 'normalize', 'pore_lookup', 'plan_upload')

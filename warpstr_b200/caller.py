@@ -67,6 +67,16 @@ def choose_strand(status, score):
     return strand, col, st, score[np.arange(len(col)), col]
 
 
+HIT_FIELDS = ('read', 'locus', 'strand', 'left_lo', 'left_hi', 'left_score', 'right_lo', 'right_hi', 'right_score')
+
+
+def hit_arrays(hits) -> Dict[str, np.ndarray]:
+    """wstr_assign_hit records (_lib.ASSIGN_HIT, any order) -> one array per field of HIT_FIELDS, sorted by
+    (read, locus)."""
+    order = np.lexsort((hits['locus'], hits['read']))
+    return {f: np.ascontiguousarray(hits[f][order]) for f in HIT_FIELDS}
+
+
 def split_pairs(aut):
     """Per read one automaton id or a (template id, reverse id) pair -> (pair bool[n], ids int32[n, 2]); a read
     given one id has it in both columns."""
@@ -585,8 +595,11 @@ class CallerEngine:
                 seq_off[1:] = np.cumsum(cap[:-1])
                 total = int(cap.sum())
                 if into is None:
-                    o['seq1'] = torch.empty(total, dtype=torch.uint8, device=self.device)
-                    o['seq2'] = torch.empty(total, dtype=torch.uint8, device=self.device)
+                    # zeroed for the parity tests (want_debug), as the buffers below: a read's sequence fills only
+                    # part of its capacity, the rest is never written, and the tests compare whole buffers
+                    alloc = torch.zeros if want_debug else torch.empty
+                    o['seq1'] = alloc(total, dtype=torch.uint8, device=self.device)
+                    o['seq2'] = alloc(total, dtype=torch.uint8, device=self.device)
                 o['seq_off'] = seq_off
             if want_debug:   # intermediate products, for the parity tests
                 # (zeroed: the padding between reads is never written, and the tests compare whole buffers; left
@@ -1023,8 +1036,9 @@ class CallerEngine:
         src.finish(st)
         return st
 
-    def _locate_device(self, d_raw, raw_off, aut, spike_removal, offset) -> Dict[str, np.ndarray]:
-        """Whole-read normalisation of int16 reads on the device, then the window search."""
+    def _normalize_whole(self, d_raw, raw_off, spike_removal):
+        """Whole-read normalisation of int16 reads on the device (window [0, N-1]) for the searches in whole reads:
+        (d_sig float64, sig_off, lengths)."""
         import torch
         from .normalize import SPIKE_MODES
         lens = np.diff(raw_off)
@@ -1038,8 +1052,64 @@ class CallerEngine:
             ws = self._device_buffer('norm_ws0', _lib.normalize_workspace_bytes(n), torch.uint8)
             _lib.normalize_batch(d_raw, raw_off, np.zeros(n, dtype=np.int32), lengths - 1, SPIKE_MODES[spike_removal],
                                  d_sig, sig_off, None, ws)
+        return d_sig, sig_off, lengths
+
+    def _locate_device(self, d_raw, raw_off, aut, spike_removal, offset) -> Dict[str, np.ndarray]:
+        """Whole-read normalisation of int16 reads on the device, then the window search."""
+        import torch
+        d_sig, sig_off, lengths = self._normalize_whole(d_raw, raw_off, spike_removal)
+        with torch.cuda.device(self.device):
             res = self.locate_packed(d_sig, sig_off, lengths, aut, offset)
             del d_sig
+        return res
+
+    # -- a panel's reads found in a whole run by their flanks (DESIGN.md section 4.6) ----------------------------
+    def assign_packed(self, d_sig, off, lengths, panel, offset: float = 0.35) -> Dict[str, np.ndarray]:
+        """wstr_assign_batch on device-resident whole normalised reads (float64, even starts ``off``) with the flank
+        chains of ``panel`` (an ``assign.Panel``; its chains are uploaded to this engine on first use).  Returns the
+        hits as host arrays sorted by (read, locus), the fields of ``assign.HIT_FIELDS``: every (read, locus) whose
+        flanks were found in order on a strand, and that strand (0 template, 1 reverse).  Only the hits leave the
+        device."""
+        import torch
+        ids = panel.register(self)
+        auts = [self.automata[i] for i in ids]
+        n = len(lengths)
+        cap = max(n * (len(auts) // 4), 1) * _lib.ASSIGN_HIT.itemsize
+        with torch.cuda.device(self.device):
+            ws = self._device_buffer('asg_ws', _lib.assign_workspace_bytes(auts, n), torch.uint8)
+            d_hits = self._device_buffer('asg_hits', cap, torch.uint8)
+            d_n = self._device_buffer('asg_n', 1, torch.int32)
+            _lib.assign_batch(auts, d_sig, off, lengths, offset, None, d_hits, d_n, ws)
+            k = int(d_n.cpu()[0])
+            hits = d_hits[:k * _lib.ASSIGN_HIT.itemsize].cpu().numpy().view(_lib.ASSIGN_HIT)
+        return hit_arrays(hits)
+
+    def assign_arrays_raw(self, host_raw, raw_off, panel, spike_removal: str = 'Brute',
+                          offset: float = 0.35) -> Dict[str, np.ndarray]:
+        """Whole int16 reads (``pack_raw``) in, the panel's hits out (``assign_packed``): upload, whole-read
+        normalisation and the flank search on the device."""
+        return self._assign_whole(_WholeReads(host_raw, raw_off), panel, spike_removal, offset)
+
+    def assign_arrays_vbz(self, host_payload, table, read_chunk, raw_off, panel, spike_removal: str = 'Brute',
+                          offset: float = 0.35, reads=None) -> Dict[str, np.ndarray]:
+        """``assign_arrays_raw`` for VBZ-compressed reads (``pack_vbz``), decoded on the device first.  With
+        ``reads`` (the fast5.CompressedRead list packed) a chunk the device decoders refuse raises its
+        Fast5FormatError, naming the file and the read; without, the dict carries ``chunk_status`` and
+        ``zstd_status`` and a read with a bad chunk has undefined hits."""
+        src = _VBZReads(host_payload, table, read_chunk, raw_off, reads)
+        res = self._assign_whole(src, panel, spike_removal, offset)
+        if reads is not None:
+            src.raise_bad(res)
+        return res
+
+    def _assign_whole(self, src, panel, spike_removal, offset) -> Dict[str, np.ndarray]:
+        import torch
+        st = self._load(src)
+        d_sig, sig_off, lengths = self._normalize_whole(src.d_raw, src.raw_off, spike_removal)
+        with torch.cuda.device(self.device):
+            res = self.assign_packed(d_sig, sig_off, lengths, panel, offset)
+            del d_sig
+        res.update(st)
         return res
 
     def _call_located(self, src, aut_ids, reverse, spike_removal, offset) -> list:

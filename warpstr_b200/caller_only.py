@@ -63,7 +63,12 @@ def prepare(output: str, csv_path: str, check_reads: bool = True) -> Dict[str, s
                     raise ValueError(f"Read {rec['read_name']} not found in fast5 file {src}")
             rows.setdefault(rec['locus'], []).append(row + [''] * len(add_win) + (['run_0'] if add_run_id else []) +
                                                      ['1'])
-    out_header = header + add_win + (['run_id'] if add_run_id else []) + ['saved']
+    return write_overviews(output, header + add_win + (['run_id'] if add_run_id else []) + ['saved'], rows)
+
+
+def write_overviews(output: str, header: List[str], rows: Dict[str, List[List[str]]]) -> Dict[str, str]:
+    """``<output>/<locus>/overview.csv`` with ``header`` and the locus's ``rows`` for every locus of ``rows``;
+    returns {locus: overview path}."""
     written = {}
     for locus, lines in rows.items():
         dest = os.path.join(output, locus)
@@ -71,7 +76,7 @@ def prepare(output: str, csv_path: str, check_reads: bool = True) -> Dict[str, s
         path = os.path.join(dest, 'overview.csv')
         with open(path, 'w') as fh:
             w = csv.writer(fh, delimiter=',', quotechar='"', quoting=csv.QUOTE_MINIMAL)
-            w.writerow(out_header)
+            w.writerow(header)
             w.writerows(lines)
         written[locus] = path
     return written
